@@ -1,7 +1,8 @@
 #!/usr/bin/env python
 """bench.py -- MRI subjects/s of the imaging-embedding hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2] [--subjects B] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c5] [--subjects B] [--impl b200|reference]
+                    [--dump-outputs DIR]
 
 The default workload is c3 = configs/openneuro_ds001907_resnet2d_mil.yaml (ResNet50, 48 slices, gated MIL attention): the
 configuration BASELINE.json's metric ("ResNet2D-MIL embed+fuse") is quoted on.
@@ -29,8 +30,21 @@ of the embedding table and of the per-scenario probabilities when N > 1].  Print
   heads        pdf_moddrop_sweep / pdf_moe_sweep at N = 10 000 and 1 000 000 subjects (SURVEY.md 8d), bytes-based roofline
   cpu_baseline the oracle port of the reference's CPU path on a bounded sample (rank 0, N = 1 only)
 
-`--impl reference` times the reference's own CPU implementation of the path (oracle port; /root/reference does
-not exist on the GPU box and the reference is Python, so there is nothing to compile into oracle/_ref).
+`--impl reference` times the reference's own CPU implementation of the path (the oracle port in oracle/oracle.py: the
+reference is Python, so there is nothing to compile).
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned in its last step as DIR/<name>.npy (float32),
+64 MB at most, so that two builds can be compared output for output on identical inputs (the same arguments give the same
+seeded inputs):
+  c2 / c3      embeddings.npy (c3: [B*N, L, D] slice embeddings, c2: [B*N, D] slice means) and scenario_probs.npy [B*N, 7]
+  c5           loss.npy, probs.npy [bags], and the updated weights: head_params.npy, backbone_params.npy (flat)
+An array larger than its share of the 64 MB is replaced by a fixed, seeded sample of its rows (the same rows for the same
+shapes), flattened to [rows, last axis] -- c3 embeddings to [k, D] rows of (subject, slice) pairs -- with the kept row indices in
+<name>_rows.npy (row = subject * L + slice for the c3 table).
+c3's last step depends only on the seeded inputs, so two runs of one build are expected to write the same files.  c5's weights
+are not expected to match bit for bit between runs: the training kernels accumulate with atomicAdd (the head's gradients, the
+loss and the gradient norm in float, BatchNorm statistics in double) in no fixed order, and Adam carries those last-bit
+differences through the steps; compare c5 dumps with a tolerance.
 """
 from __future__ import annotations
 
@@ -143,6 +157,31 @@ class ClockSampler:
     def summary(self):
         return {"sm_mhz": float(np.median(self.sm)) if self.sm else None, "sm_max_mhz": max(self.mx) if self.mx else None,
                 "reasons": sorted(self.reasons), "samples": len(self.sm), "source": "nvml" if self.nvml else "nvidia-smi"}
+
+
+DUMP_BYTES = 64 * 10**6 - 4096          # --dump-outputs budget, less room for the .npy headers
+
+
+def dump_outputs(out_dir: str, arrays: dict):
+    """Writes each array as out_dir/<name>.npy in float32.  Smallest first, each array gets an equal share of what is left of
+    DUMP_BYTES; one larger than its share is replaced by a sample of its rows drawn with a fixed seed (the same rows for the
+    same shapes in every run): the array flattened to [rows, last axis] (a 1-D array: to its elements), the kept rows in
+    ascending order, and their indices into that flattened array in out_dir/<name>_rows.npy (float64, exact)."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    arrays = sorted(((name, np.asarray(a, dtype=np.float32)) for name, a in arrays.items()), key=lambda kv: kv[1].nbytes)
+    left = DUMP_BYTES
+    for i, (name, a) in enumerate(arrays):
+        share = left // (len(arrays) - i)
+        if a.nbytes > share:
+            rows = a.reshape(-1, a.shape[-1]) if a.ndim > 1 else a.reshape(-1, 1)
+            keep = share // (rows.shape[1] * 4 + 8)                     # a row and its float64 index
+            pick = np.sort(np.random.default_rng(0).choice(rows.shape[0], keep, replace=False))
+            a = rows[pick] if a.ndim > 1 else rows[pick, 0]
+            np.save(out / f"{name}_rows.npy", pick.astype(np.float64))
+            left -= pick.size * 8
+        np.save(out / f"{name}.npy", a)
+        left -= a.nbytes
 
 
 def host_pool(n: int):
@@ -287,13 +326,14 @@ def run_c5(args, wl):
     host_bags = [rng.random((L, TARGET[0], TARGET[1])).astype(np.float32) for _ in range(bags_per_step)]
     dev_bags = [torch.from_numpy(b).to(dev) for b in host_bags]
     y = np.array([1.0, 0.0, 1.0, 0.0], dtype=np.float32)
+    last = [None]                                      # what the last timed call returned
 
     def timed(fn, steps):
         barrier(); torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last[0] = fn()
         e1.record()
         torch.cuda.synchronize(); barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
@@ -306,11 +346,16 @@ def run_c5(args, wl):
     for _ in range(max(args.warmup, 3)):
         step_dev()
     torch.cuda.synchronize()
-    steps = min(args.steps, 20)
+    steps = args.steps
     l0 = _lib.launch_count()
     with ClockSampler(local_rank) as clk:
         ms = timed(step_dev, steps)
     launches = _lib.launch_count() - l0
+    if args.dump_outputs and rank == 0:            # before the host-fed steps below train the weights further
+        loss, prob = last[0]
+        rt, ht, _ = model._trainers()
+        dump_outputs(args.dump_outputs, {"loss": loss.cpu().numpy(), "probs": prob.cpu().numpy(),
+                                         "head_params": ht.flat_param.cpu().numpy(), "backbone_params": rt.flat_param.cpu().numpy()})
     step_host()
     barrier(); torch.cuda.synchronize()
     t0 = time.perf_counter()
@@ -363,7 +408,12 @@ def main():
     ap.add_argument("--sustained-seconds", type=float, default=2.0, help="length of the sustained legs (0 = skip)")
     ap.add_argument("--no-heads", action="store_true", help="skip the fusion-head legs (ModDrop / MoE sweeps at N = 1e4, 1e6)")
     ap.add_argument("--mil-bags", type=int, default=2048, help="bags of the MIL roofline leg (c3)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the timed path returned in its last step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the b200 path; the reference arm keeps none")
     wl = WORKLOADS[args.workload]
     if args.impl == "reference":
         return run_reference(args, wl)
@@ -478,6 +528,8 @@ def main():
             all_gather_rows(outs[-1][1].to(dev), B * ws)
         return outs
 
+    last = [None]                                      # what the last timed call returned
+
     def timed(fn, steps):
         barrier(); torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
@@ -486,7 +538,7 @@ def main():
             pipe.overlap_begin()
         fuse_stream.wait_stream(torch.cuda.current_stream())
         for _ in range(steps):
-            fn()
+            last[0] = fn()
         if overlap:
             pipe.overlap_end()
         torch.cuda.current_stream().wait_stream(fuse_stream)
@@ -505,6 +557,9 @@ def main():
         ms = timed(step_device, args.steps)
     launches = _lib.launch_count() - launches0
     value = ws * B * args.steps / (ms / 1e3)
+    if args.dump_outputs and rank == 0:            # the legs below reuse these buffers
+        emb, pr = last[0]
+        dump_outputs(args.dump_outputs, {"embeddings": emb.cpu().numpy(), "scenario_probs": pr.cpu().numpy()})
 
     # --- per-kernel-family device time (same buffers, same launches): K2 conv stack and K1 preprocessing
     def enc_only():

@@ -1,5 +1,6 @@
 """Drop-in boundary on the GPU: the reference's entry points (CLI scripts, helper functions, model predict_proba,
 evaluate_model) served by the CUDA path, checked against outputs the reference itself produced (tests/golden)."""
+import hashlib
 import json
 import runpy
 import sys
@@ -47,27 +48,44 @@ def _run_script(name, argv):
 def test_cli_scripts_match_reference_outputs(golden, tmp_path, seeded_backbone, monkeypatch, precision, tol):
     g = golden("scripts")
     monkeypatch.setenv("PD_FUSION_B200_PRECISION", precision)
-    vols = Path(str(g["manifest_dir"]))
+    # The reference run kept its volumes in a temporary directory (`manifest_dir`) whose path the manifest records, and the
+    # manifest's hash names the cache files.  The same volumes are written under tmp_path instead: the manifest must differ from
+    # the reference's by that directory alone, and the file names by the manifest hash alone.  The reference's key rule (first
+    # 12 hex digits of the sha256 of the manifest bytes) is applied to both manifests here, not taken from the code under test.
+    vols = tmp_path / "vols"
     manifest = write_synthetic_manifest(vols, 3, shape=(48, 40, 36))
-    assert manifest.read_bytes() == g["manifest_bytes"].tobytes()        # identical manifest -> identical cache key
+    ref_manifest = g["manifest_bytes"].tobytes()
+    assert manifest.read_bytes() == ref_manifest.replace(str(g["manifest_dir"]).encode(), str(vols).encode())
+    ref_key, key = (hashlib.sha256(m).hexdigest()[:12] for m in (ref_manifest, manifest.read_bytes()))
+
+    def ref_files(tag):
+        assert all(f"_{ref_key}_" in str(f) for f in g[f"{tag}/files"])
+        return sorted(str(f).replace(f"_{ref_key}_", f"_{key}_") for f in g[f"{tag}/files"])
+
+    def ref_meta(tag):
+        meta = json.loads(str(g[f"{tag}/json"]))
+        assert meta["manifest"] == str(Path(str(g["manifest_dir"])) / "manifest.csv")
+        return dict(meta, manifest=str(manifest))
     # CLI 1
     out1 = tmp_path / "c2"
     _run_script("build_resnet2d_embeddings.py", ["--manifest", str(manifest), "--out-dir", str(out1)] + [str(a) for a in g["c2/argv"]])
-    assert sorted(p.name for p in out1.iterdir()) == sorted(str(f) for f in g["c2/files"])
+    assert sorted(p.name for p in out1.iterdir()) == ref_files("c2")
     df = pd.read_parquet(next(out1.glob("*.parquet")))
     assert list(df.columns) == [str(c) for c in g["c2/columns"]] and [str(t) for t in df.dtypes] == [str(t) for t in g["c2/dtypes"]]
     emb = df[[c for c in df.columns if c.startswith("mri_resnet_")]].values
     rel = np.linalg.norm(emb - g["c2/emb"], axis=1) / np.linalg.norm(g["c2/emb"], axis=1)
     assert rel.max() < tol, rel
-    assert json.loads(next(out1.glob("*.json")).read_text()) == json.loads(str(g["c2/json"]))
+    assert json.loads(next(out1.glob("*.json")).read_text()) == ref_meta("c2")
     # second call returns the cached parquet
     again = of.build_resnet2d_embeddings(manifest, out1, json.loads(str(g["c2/json"]))["config"])
     assert again.equals(df)
     # CLI 2 (multi-axis MIL bags)
     out2 = tmp_path / "mil"
     _run_script("build_resnet2d_mil_embeddings.py", ["--manifest", str(manifest), "--out-dir", str(out2)] + [str(a) for a in g["mil/argv"]])
-    assert sorted(p.name for p in out2.iterdir()) == sorted(str(f) for f in g["mil/files"])
-    cfg = json.loads(next(out2.glob("*.json")).read_text())["config"]
+    assert sorted(p.name for p in out2.iterdir()) == ref_files("mil")
+    meta = json.loads(next(out2.glob("*.json")).read_text())
+    assert meta == ref_meta("mil")
+    cfg = meta["config"]
     bags = of.load_resnet2d_mil_embeddings(manifest, out2, cfg)
     got = np.stack(bags["mri_mil"].tolist())
     assert got.shape == g["mil/emb"].shape and got.dtype == np.float32
