@@ -211,6 +211,13 @@ typedef struct {
   int32_t ho, wo;      /* output spatial size */
   int32_t relu;
   int32_t out_f32;     /* bf16 path only: store the output tile as f32 instead of bf16 */
+  /* bf16 1x1 stride-1 PDF_OP_CONV only, 0 otherwise: the projection shortcut of a ResNet Bottleneck (downsample conv1x1 + BN of the
+   * block input x, torchvision resnet.py Bottleneck.forward) computed as more K of this convolution:
+   * d_out = relu?(conv1x1([d_in | x_s], d_weight) + d_bias), x_s = x at stride 1 if (sc_h, sc_w) == (ho, wo), else at stride 2
+   * (then ho == (sc_h-1)/2+1, wo == (sc_w-1)/2+1).  With sc_c != 0, d_residual points at x [N, sc_h, sc_w, sc_c] bf16 (nothing is
+   * added), d_weight is [K][c + sc_c] bf16 (this conv's columns, then the shortcut's; both BN folded), d_bias the sum of both biases;
+   * c % 64 == 0, sc_c % 64 == 0.  sc_hw = (sc_h << 16) | sc_w. */
+  int32_t sc_c;
   const void* d_in;
   const void* d_weight;   /* f32 path: [R][S][C][K] f32 ; bf16 path: [K][R][S][C] bf16, BN folded */
   const float* d_scale;   /* f32 path: per-channel BN scale (NULL = 1) */
@@ -231,6 +238,7 @@ typedef struct {
   const float* d_bias3;
   void* d_out3;
   int32_t k3;
+  int32_t sc_hw;       /* shortcut input's spatial size (sc_h << 16) | sc_w, see sc_c */
 } pdf_op;
 
 typedef struct pdf_plan pdf_plan; /* opaque: validated ops + pre-encoded TMA descriptors */

@@ -1,6 +1,7 @@
 // K2 (bf16 path): pointwise (1x1) convolutions of the ResNet50 bottleneck, epilogue through shared memory.
 //
 //   Y[M, Cout] = relu?( X[M, Cin] * W[Cout, Cin]^T + bias (+ R[M, Cout]) )                 bf16 x bf16 -> f32 (TMEM) -> bf16
+//   optional shortcut segment:  Y = relu( [X | Xs] * [W | Ws]^T + bias )                      (instead of a residual R)
 //   optional chain:  T[M, N2] = relu( Y[M, Cout] * W3[N2, Cout]^T + bias3 )               (the NEXT block's 1x1 reduce conv)
 //
 // Why a second kernel next to conv_tc.cu: the bottleneck's expansion convs and downsamples have K = 64..512 and N = 256..2048,
@@ -14,7 +15,11 @@
 //   * one thread hands the buffer to the TMA unit (cp.async.bulk.tensor store): full-line writes, no LSU involvement;
 //   * the same buffer -- it has exactly the K-major SWIZZLE_128B layout of an MMA A operand -- feeds the chained GEMM:
 //     the next block's 1x1 reduce convolution accumulates over the N-chunks of the tile in a third TMEM accumulator, so that
-//     conv never re-reads the (4x wider) block output from HBM: its launch disappears.
+//     conv never re-reads the (4x wider) block output from HBM: its launch disappears;
+//   * a Bottleneck's projection shortcut (downsample 1x1 conv + BN of the block input x, added before the ReLU) is the same GEMM
+//     as conv3 over K: the last k-blocks of the mainloop come from a second map over x (2-D at stride 1, im2col-mode at stride 2)
+//     and multiply the shortcut's columns of the host-concatenated weights [W3 | Wds].  The downsample's 4x-wide output is then
+//     never written nor read back as a residual, and its launch disappears.
 //
 // Work unit = (128-row M tile, NC-column N chunk), N fastest: one CTA owns all chunks of its M tiles (persistent, round-robin).
 //   warp 0 (one lane)  TMA producer: residual tile of unit u | A/B k-blocks of unit u | chained-weight k-blocks of unit u-1
@@ -42,6 +47,8 @@ constexpr int kPwBiasMax = 2048;
 struct PwParams {
   int M_total, Cout, K, n_chunks, m_tiles, relu, im2col, has_res;
   int Ho, Wo, stride;           // im2col (strided 1x1) geometry
+  int kb_main;                  // k-blocks read through tmap_a; k-blocks kb_main .. K/64-1 are the shortcut segment (tmap_sc)
+  int sc_im2col, sc_stride;     // shortcut segment: 1 = im2col-mode map at sc_stride (2), 0 = 2-D map over [M, sc_c]
   int N2;                       // chained output channels
   int stages, nry;              // ring depth, staging buffers
   int bias_staged;              // 1: bias vector copied to shared memory at kernel start, 0: read from global memory (L1-resident)
@@ -133,7 +140,7 @@ template <int NC, bool CHAIN, bool MC>
 __global__ void __launch_bounds__(kPwThreads, 1)
 conv_pw_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant__ CUtensorMap tmap_b,
                const __grid_constant__ CUtensorMap tmap_out, const __grid_constant__ CUtensorMap tmap_res,
-               const __grid_constant__ CUtensorMap tmap_w3, const PwParams p) {
+               const __grid_constant__ CUtensorMap tmap_w3, const __grid_constant__ CUtensorMap tmap_sc, const PwParams p) {
   using L = PwSmem<NC>;
   constexpr int kSub = NC / 64;                   // 64-channel sub-tiles of a staging buffer
   extern __shared__ uint8_t smem_raw[];
@@ -166,6 +173,7 @@ conv_pw_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
     prefetch_tmap(&tmap_a); prefetch_tmap(&tmap_b); prefetch_tmap(&tmap_out);
     if (p.has_res) prefetch_tmap(&tmap_res);
     if (CHAIN) prefetch_tmap(&tmap_w3);
+    if (p.kb_main < p.K / kBlockK) prefetch_tmap(&tmap_sc);
     for (int s = 0; s < kPwStages; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, MC ? 2 : 1); }
     for (int a = 0; a < 2; ++a) { mbar_init(bar_accfull + 8 * a, 1); mbar_init(bar_accempty + 8 * a, kPwEpiWarps); }
     for (int b = 0; b < kPwRy; ++b) {
@@ -226,7 +234,7 @@ conv_pw_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
           // the NEXT row tile's A k-blocks into L2 while this tile's n_chunks units run: its first ring fills then hit L2 instead of
           // paying the HBM latency inside the ring (pdf_debug_set_pw_prefetch)
           const int m1 = tile_of(ti + 1) * kBlockM;
-          for (int kb = 0; kb < num_kb; ++kb)
+          for (int kb = 0; kb < p.kb_main; ++kb)
             asm volatile("cp.async.bulk.prefetch.tensor.2d.L2.global.tile [%0, {%1, %2}];"
                          ::"l"(reinterpret_cast<uint64_t>(&tmap_a)), "r"(kb * kBlockK), "r"(m1) : "memory");
         }
@@ -236,21 +244,27 @@ conv_pw_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_constant
           mbar_expect_tx(bar_resfull + 8 * b, (uint32_t)L::kRyBytes);
           for (int s = 0; s < kSub; ++s) tma_load_2d(s_ry + b * L::kRyBytes + s * kABytes, &tmap_res, bar_resfull + 8 * b, n0 + s * 64, m0);
         }
-        int n_img = 0, w0 = 0, h0 = 0;
-        if (p.im2col) {
+        int n_img = 0, pp = 0, qq = 0;             // first output pixel of the tile (im2col-mode loads)
+        if (p.im2col || p.sc_im2col) {
           const int hw = p.Ho * p.Wo;
           n_img = m0 / hw;
           const int rem = m0 - n_img * hw;
-          const int pp = rem / p.Wo, qq = rem - pp * p.Wo;
-          w0 = qq * p.stride; h0 = pp * p.stride;
+          pp = rem / p.Wo; qq = rem - pp * p.Wo;
         }
         for (int kb = 0; kb < num_kb; ++kb) {
           uint32_t stage;
           ring_wait(stage);
           mbar_expect_tx(bar_full + 8 * stage, (uint32_t)(kABytes + NC * 128));
           const uint32_t sa = s_ring + stage * L::kStageBytes;
-          if (p.im2col) tma_load_im2col_4d(sa, &tmap_a, bar_full + 8 * stage, kb * kBlockK, w0, h0, n_img, 0, 0);
-          else tma_load_2d(sa, &tmap_a, bar_full + 8 * stage, kb * kBlockK, m0);
+          const int kc = (kb - p.kb_main) * kBlockK;    // channel of the shortcut segment (kb >= kb_main)
+          if (kb < p.kb_main) {
+            if (p.im2col) tma_load_im2col_4d(sa, &tmap_a, bar_full + 8 * stage, kb * kBlockK, qq * p.stride, pp * p.stride, n_img, 0, 0);
+            else tma_load_2d(sa, &tmap_a, bar_full + 8 * stage, kb * kBlockK, m0);
+          } else if (p.sc_im2col) {
+            tma_load_im2col_4d(sa, &tmap_sc, bar_full + 8 * stage, kc, qq * p.sc_stride, pp * p.sc_stride, n_img, 0, 0);
+          } else {
+            tma_load_2d(sa, &tmap_sc, bar_full + 8 * stage, kc, m0);
+          }
           if (MC)      // this CTA's half of the [NC x 64] weight tile (tmap_b's box is NC/2 rows), into both rings
             tma_load_2d_mc(sa + kABytes + rank * (uint32_t)(NC * 64), &tmap_b, bar_full + 8 * stage, kb * kBlockK, n0 + (int)rank * (NC / 2), (uint16_t)3);
           else tma_load_2d(sa + kABytes, &tmap_b, bar_full + 8 * stage, kb * kBlockK, n0);
@@ -407,8 +421,8 @@ bool pw_eligible(const pdf_op& op) {
   if (g_pw_mode == 0) return false;
   if (!(op.kind == PDF_OP_CONV && op.precision == PDF_PREC_BF16 && op.r == 1 && op.s == 1 && op.pad == 0 && !op.out_f32 && !op.d_weight2))
     return false;
-  if (op.c % 64 != 0 || op.k % 64 != 0 || op.k > kPwBiasMax) return false;
-  if (op.d_weight3) return true;
+  if (op.c % 64 != 0 || op.k % 64 != 0 || op.k > kPwBiasMax || op.sc_c % 64 != 0) return false;
+  if (op.d_weight3 || op.sc_c) return true;
   if (g_pw_mode == 2) return true;
   // default policy (profiles/r02_op_times_resnet50_pw*.txt): every N chunk of a tile re-streams the A tile, so long-K reduce
   // convs and downsamples stay on conv_tc_kernel's 256-wide tiles; the epilogue-bound short-K launches come here
@@ -427,20 +441,36 @@ int prepare_conv_pw(const pdf_op& op, TcConv* tc) {
   tc->M_total = op.n * op.ho * op.wo;
   tc->Cout = op.k; tc->Ho = op.ho; tc->Wo = op.wo; tc->stride = op.stride; tc->pad = 0; tc->R = 1; tc->S = 1;
   tc->cchunks = op.c / kBlockK;
-  tc->relu = op.relu; tc->bias = op.d_bias; tc->residual = op.d_residual; tc->out = op.d_out; tc->out_f32 = 0;
+  tc->relu = op.relu; tc->bias = op.d_bias; tc->residual = op.sc_c ? nullptr : op.d_residual; tc->out = op.d_out; tc->out_f32 = 0;
   tc->n_images = op.n;
   tc->im2col = op.stride != 1;
   tc->k3 = 0; tc->bias3 = nullptr; tc->out3 = nullptr;
+  tc->sc_kb = op.sc_c / kBlockK; tc->sc_im2col = 0;
   if (tc->im2col) {
     if (int rc = encode_im2col(&tc->tmap_a, op)) return rc;
   } else {
     if (int rc = encode_2d(&tc->tmap_a, op.d_in, (uint64_t)tc->M_total, (uint64_t)op.c, kBlockM)) return rc;
   }
+  if (op.sc_c) {        // shortcut segment: d_residual is the block input x [N, sc_h, sc_w, sc_c], read at stride 1 or 2
+    const int sc_h = op.sc_hw >> 16, sc_w = op.sc_hw & 0xffff;
+    PDF_REQUIRE(op.stride == 1 && op.d_residual && (reinterpret_cast<uintptr_t>(op.d_residual) & 15) == 0,
+                "pointwise conv: a shortcut segment needs a stride-1 host convolution and d_residual = x, 16-byte aligned");
+    pdf_op xs = op;
+    xs.d_in = op.d_residual; xs.h = sc_h; xs.w = sc_w; xs.c = op.sc_c;
+    if (sc_h == op.ho && sc_w == op.wo) {
+      if (int rc = encode_2d(&tc->tmap_sc, op.d_residual, (uint64_t)tc->M_total, (uint64_t)op.sc_c, kBlockM)) return rc;
+    } else {
+      xs.stride = 2; xs.ho = op.ho; xs.wo = op.wo;
+      tc->sc_im2col = 1;
+      if (int rc = encode_im2col(&tc->tmap_sc, xs)) return rc;
+    }
+  }
   // weight-multicast CTA pairs (see the kernel): where the weight tiles are a large share of a unit's ring traffic
   tc->pw_mc = (g_pw_mc && NC == 128 && op.c >= 128 && (!op.d_weight3 || op.k3 % 2 == 0)) ? 1 : 0;
-  if (int rc = encode_2d(&tc->tmap_b, op.d_weight, (uint64_t)op.k, (uint64_t)op.c, (uint32_t)(tc->pw_mc ? NC / 2 : NC))) return rc;
+  const uint64_t k_total = (uint64_t)op.c + (uint64_t)op.sc_c;     // weights [K][c + sc_c]: conv3's columns, then the shortcut's
+  if (int rc = encode_2d(&tc->tmap_b, op.d_weight, (uint64_t)op.k, k_total, (uint32_t)(tc->pw_mc ? NC / 2 : NC))) return rc;
   if (int rc = encode_2d(&tc->tmap_out, op.d_out, (uint64_t)tc->M_total, (uint64_t)op.k, kBlockM)) return rc;
-  if (op.d_residual)
+  if (tc->residual)
     if (int rc = encode_2d(&tc->tmap_res, op.d_residual, (uint64_t)tc->M_total, (uint64_t)op.k, kBlockM)) return rc;
   if (op.d_weight3) {
     PDF_REQUIRE(NC == 128 && (op.k3 == 64 || op.k3 == 128 || op.k3 == 256) && op.d_out3 &&
@@ -456,8 +486,9 @@ template <int NC, bool CHAIN, bool MC>
 static int launch_pw(const TcConv& tc, cudaStream_t s) {
   using L = PwSmem<NC>;
   // measured (profiles/r02_pw_cfg.txt): launches that fetch a residual tile want the third staging buffer (the residual of unit
-  // u+1 streams in while unit u is still in its buffer), the others the fourth ring stage
-  const bool wants_staging = tc.residual != nullptr || CHAIN;
+  // u+1 streams in while unit u is still in its buffer), the others the fourth ring stage.  Launches with a shortcut segment fetch
+  // no residual and run a 2-4x longer k-loop: they want the fourth ring stage also when chained (profiles/r03_pw_cfg_shortcut.txt)
+  const bool wants_staging = tc.residual != nullptr || (CHAIN && !tc.sc_kb);
   int stages = g_pw_stages ? g_pw_stages : (wants_staging ? 3 : 4), nry = g_pw_ry ? g_pw_ry : (wants_staging ? 3 : 2);
   // the bias vector is staged in shared memory when it fits next to the requested ring; a deeper ring wins over bias staging
   // (the epilogue then reads the bias through L1), and the ring shrinks only when even that does not fit
@@ -473,9 +504,10 @@ static int launch_pw(const TcConv& tc, cudaStream_t s) {
   PwParams p;
   p.stages = stages; p.nry = nry; p.bias_staged = bias_floats > 0 || tc.bias == nullptr;
   p.l2_prefetch = g_pw_prefetch;
-  p.M_total = tc.M_total; p.Cout = tc.Cout; p.K = tc.Cin; p.n_chunks = tc.Cout / NC; p.m_tiles = ceil_div(tc.M_total, kBlockM);
+  p.M_total = tc.M_total; p.Cout = tc.Cout; p.K = tc.Cin + tc.sc_kb * kBlockK; p.n_chunks = tc.Cout / NC; p.m_tiles = ceil_div(tc.M_total, kBlockM);
   p.relu = tc.relu; p.im2col = tc.im2col; p.has_res = tc.residual != nullptr;
   p.Ho = tc.Ho; p.Wo = tc.Wo; p.stride = tc.stride;
+  p.kb_main = tc.Cin / kBlockK; p.sc_im2col = tc.sc_im2col; p.sc_stride = tc.sc_im2col ? 2 : 1;
   p.N2 = tc.k3; p.bias = tc.bias; p.bias3 = tc.bias3; p.out3 = reinterpret_cast<__nv_bfloat16*>(tc.out3);
   int grid = max(1, min(p.m_tiles, num_sms()));
   if (MC) grid = max(2, min((p.m_tiles + 1) / 2 * 2, num_sms() / 2 * 2));      // whole clusters of two CTAs
@@ -484,6 +516,7 @@ static int launch_pw(const TcConv& tc, cudaStream_t s) {
   const CUtensorMap& to = *reinterpret_cast<const CUtensorMap*>(&tc.tmap_out);
   const CUtensorMap& tr = p.has_res ? *reinterpret_cast<const CUtensorMap*>(&tc.tmap_res) : to;
   const CUtensorMap& tw = CHAIN ? *reinterpret_cast<const CUtensorMap*>(&tc.tmap_w3) : tb;
+  const CUtensorMap& tsc = tc.sc_kb ? *reinterpret_cast<const CUtensorMap*>(&tc.tmap_sc) : ta;
   if (MC) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kPwThreads); cfg.dynamicSmemBytes = (size_t)smem; cfg.stream = s;
@@ -493,9 +526,9 @@ static int launch_pw(const TcConv& tc, cudaStream_t s) {
     attr[1].id = cudaLaunchAttributeClusterDimension;
     attr[1].val.clusterDim.x = 2; attr[1].val.clusterDim.y = 1; attr[1].val.clusterDim.z = 1;
     cfg.attrs = attr; cfg.numAttrs = 2;
-    PDF_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_pw_kernel<NC, CHAIN, MC>, ta, tb, to, tr, tw, p));
+    PDF_CHECK_CUDA(cudaLaunchKernelEx(&cfg, conv_pw_kernel<NC, CHAIN, MC>, ta, tb, to, tr, tw, tsc, p));
   } else {
-    PDF_CHECK_CUDA(launch_pdl(conv_pw_kernel<NC, CHAIN, MC>, dim3(grid), dim3(kPwThreads), (size_t)smem, s, ta, tb, to, tr, tw, p));
+    PDF_CHECK_CUDA(launch_pdl(conv_pw_kernel<NC, CHAIN, MC>, dim3(grid), dim3(kPwThreads), (size_t)smem, s, ta, tb, to, tr, tw, tsc, p));
   }
   PDF_CHECK_LAUNCH();
   return PDF_OK;

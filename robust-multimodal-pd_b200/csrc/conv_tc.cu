@@ -527,6 +527,7 @@ int prepare_conv_tc(const pdf_op& op, TcConv* tc) {
   tc->pw = 0;
   if (pw_eligible(op)) return prepare_conv_pw(op, tc);   // 1x1 convs whose epilogue goes through shared memory (conv_pw.cu)
   PDF_REQUIRE(!op.d_weight3, "bf16 conv: a chained 1x1 convolution needs a 1x1 host convolution with bf16 output (conv_pw.cu)");
+  PDF_REQUIRE(!op.sc_c, "bf16 conv: a shortcut segment needs a 1x1 host convolution with bf16 output (conv_pw.cu)");
   tc->block_n = (op.k % 256 == 0) ? 256 : (op.k % 128 == 0 ? 128 : 64);
   tc->im2col = !(op.r == 1 && op.s == 1 && op.stride == 1 && op.pad == 0);
   tc->M_total = op.n * op.ho * op.wo;

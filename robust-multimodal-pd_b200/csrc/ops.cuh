@@ -39,6 +39,10 @@ struct TcConv {
   int k3;                  // chained output channels (0 = no chain)
   const float* bias3;
   void* out3;
+  // shortcut segment (Bottleneck projection shortcut computed as the last k-blocks of conv3's GEMM): Cin counts conv3's own channels
+  TensorMapBlob tmap_sc;   // block input x: 2-D [M, sc_c] map at stride 1, im2col-mode map at stride 2
+  int sc_kb;               // k-blocks of the shortcut segment (0 = none)
+  int sc_im2col;
 };
 
 int load_driver_entry_points();

@@ -26,6 +26,14 @@ static int validate_op(const pdf_op& op, int i) {
     PDF_REQUIRE(op.ho == (op.h + 2 * op.pad - op.r) / op.stride + 1 && op.wo == (op.w + 2 * op.pad - op.s) / op.stride + 1,
                 "op %d: inconsistent conv output size", i);
   }
+  if (op.sc_c || op.sc_hw) {          // shortcut segment: x at stride 1 when its size equals the output's, else at stride 2
+    const int sc_h = op.sc_hw >> 16, sc_w = op.sc_hw & 0xffff;
+    PDF_REQUIRE(op.kind == PDF_OP_CONV && op.precision == PDF_PREC_BF16 && op.r == 1 && op.s == 1 && op.stride == 1 && op.pad == 0 &&
+                !op.out_f32 && op.sc_c > 0 && op.sc_c % 64 == 0 && op.c % 64 == 0 && op.d_residual && sc_h > 0 && sc_w > 0,
+                "op %d: a shortcut segment needs a bf16 1x1 stride-1 conv with bf16 output, c and sc_c multiples of 64, d_residual = x", i);
+    PDF_REQUIRE((sc_h == op.ho && sc_w == op.wo) || (op.ho == (sc_h - 1) / 2 + 1 && op.wo == (sc_w - 1) / 2 + 1),
+                "op %d: shortcut input %dx%d is neither the output size %dx%d nor its stride-2 source", i, sc_h, sc_w, op.ho, op.wo);
+  }
   if (op.kind == PDF_OP_MAXPOOL)
     PDF_REQUIRE(op.ho == (op.h + 2 - 3) / 2 + 1 && op.wo == (op.w + 2 - 3) / 2 + 1, "op %d: maxpool is 3x3 s2 p1", i);
   if (op.kind == PDF_OP_STEM_IM2COL)
@@ -53,7 +61,7 @@ extern "C" int pdf_plan_create(pdf_plan** out, const pdf_op* ops, int n_ops) {
     if (rc == PDF_OK && op.kind == PDF_OP_STEM_FUSED) rc = prepare_stem_tc(op, &plan->tc[i]);
     if (rc == PDF_OK && op.kind == PDF_OP_STEM_FUSED) plan->flops += 2.0 * op.n * ((op.h - 1) / 2 + 1) * ((op.w - 1) / 2 + 1) * 64.0 * 49.0;
     if (rc == PDF_OK && op.kind == PDF_OP_CONV) {
-      plan->flops += 2.0 * op.n * op.ho * op.wo * (double)op.k * op.r * op.s * op.c;
+      plan->flops += 2.0 * op.n * op.ho * op.wo * (double)op.k * op.r * op.s * (op.c + op.sc_c);   // (+ the shortcut segment's K)
       if (op.d_weight2) {
         plan->flops += 2.0 * op.n * op.ho * op.wo * (double)op.k * op.c;
         if (op.precision != PDF_PREC_BF16) {

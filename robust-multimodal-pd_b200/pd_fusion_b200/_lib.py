@@ -51,11 +51,11 @@ class Op(C.Structure):
         ("k", C.c_int32), ("r", C.c_int32), ("s", C.c_int32),
         ("stride", C.c_int32), ("pad", C.c_int32),
         ("ho", C.c_int32), ("wo", C.c_int32),
-        ("relu", C.c_int32), ("out_f32", C.c_int32),
+        ("relu", C.c_int32), ("out_f32", C.c_int32), ("sc_c", C.c_int32),
         ("d_in", C.c_void_p), ("d_weight", C.c_void_p), ("d_scale", C.c_void_p), ("d_bias", C.c_void_p),
         ("d_residual", C.c_void_p), ("d_out", C.c_void_p),
         ("d_weight2", C.c_void_p), ("d_bias2", C.c_void_p), ("d_out2", C.c_void_p),
-        ("d_weight3", C.c_void_p), ("d_bias3", C.c_void_p), ("d_out3", C.c_void_p), ("k3", C.c_int32),
+        ("d_weight3", C.c_void_p), ("d_bias3", C.c_void_p), ("d_out3", C.c_void_p), ("k3", C.c_int32), ("sc_hw", C.c_int32),
     ]
 
 

@@ -168,10 +168,26 @@ DEFAULT_DUAL_STAGES = (2, 3)
 # Bottleneck networks, bf16 path: residual stages whose conv3 launch also computes the NEXT block's conv1 (conv_pw.cu) -- the
 # chained accumulator needs planes <= 256 TMEM columns, i.e. stages 1..3
 DEFAULT_CHAIN_STAGES = (1, 2, 3)
+# Bottleneck networks, bf16 path: residual stages whose block-0 conv3 launch also computes the projection shortcut (downsample) as
+# more K of the same GEMM (conv_pw.cu, shortcut segment); the downsample launch and its 4x-wide output disappear.  Measured
+# (profiles/r03_shortcut_ab.txt, 768 slices, downsample + conv3 -> fused conv3): stage 1 840 -> 516 us, stage 2 597 -> 498 us,
+# stage 3 426 -> 404 us, stage 4 290 -> 308 us (its K = 1536 k-loop re-streams the A tile for each of 16 N chunks)
+DEFAULT_SHORTCUT_STAGES = (1, 2, 3)
+
+
+def _parse_stages(env: str, default: Sequence[int]) -> Tuple[int, ...]:
+    """Stage list of a tuning hook: unset = default, "" or "none" = no stage, "1,2" = those stages."""
+    v = os.environ.get(env)
+    if v is None:
+        return tuple(default)
+    if v.strip().lower() == "none":
+        return ()
+    return tuple(int(t) for t in v.split(",") if t)
 
 
 def lower_resnet(arch: str, n: int, S: int, bf16: bool, fused_stem: bool, chunks: List[int], in_bytes: int | None = None,
-                 dual_stages: Sequence[int] = (), chain_stages: Sequence[int] = (), cross_stage_chain: bool = True):
+                 dual_stages: Sequence[int] = (), chain_stages: Sequence[int] = (), cross_stage_chain: bool = True,
+                 shortcut_stages: Sequence[int] = ()):
     """The network as a flat, ordered list of ops over symbolic buffers.
 
     Returns (ops, extents, final_hw): ops = [(name, fields, refs, weight_name)], where refs maps the pointer fields
@@ -185,6 +201,10 @@ def lower_resnet(arch: str, n: int, S: int, bf16: bool, fused_stem: bool, chunks
     carries `_weight3` and a `d_out3` reference; that conv1 is not emitted).  With cross_stage_chain the LAST conv3 of such a stage
     also computes the first conv1 of the following stage (stride 1 in torchvision's v1.5 Bottleneck; <= 256 output channels), into
     buffer x<k+1>.
+
+    shortcut_stages: residual stages (1..4) of a Bottleneck network whose first block emits no downsample op: its conv3 op reads the
+    block input as a shortcut segment (refs d_residual = the block input, fields sc_c / sc_hw, `_shortcut` = the downsample's
+    weight name; the weights are [W3 | Wds] and the bias b3 + bds) -- relu(h W3^T + x_s Wds^T + b3 + bds) is one GEMM over K.
 
     chunks[k] = images per launch of stage k (0 = stem, 1..4 = residual stages).  The op list is depth-first: a
     stage-k chunk is preceded by the stage-(k-1) chunks that produce its input, so the big early tensors are consumed
@@ -265,8 +285,11 @@ def lower_resnet(arch: str, n: int, S: int, bf16: bool, fused_stem: bool, chunks
         for bi, cvs in enumerate(blocks):
             last_block = bi == len(blocks) - 1
             idn, idn_slot = x, None
-            fuse_down = None
-            if "down" in cvs:
+            fuse_down = sc_down = None
+            if "down" in cvs and (bf16 and kind == "bottleneck" and k in shortcut_stages and cvs["down"]["k"] == 1 and x_c % 64 == 0
+                                  and not (last_block and k == 4)):
+                sc_down = cvs["down"]["name"]              # computed by conv3's launch as more K; x stays alive to the block's end
+            elif "down" in cvs:
                 cv = cvs["down"]
                 idn_slot = free.pop(0)
                 idn = ref(idn_slot, 0, out_bytes(k, count))
@@ -299,6 +322,9 @@ def lower_resnet(arch: str, n: int, S: int, bf16: bool, fused_stem: bool, chunks
                 if is_last:
                     refs["d_residual"] = idn
                 extra = {}
+                if is_last and sc_down is not None:
+                    refs["d_residual"] = x
+                    extra.update(_shortcut=sc_down, sc_c=x_c, sc_hw=(x_h << 16) | x_h)
                 if fuse_down is not None and cv["role"] == "a":
                     refs["d_out2"] = idn
                     extra["_weight2"] = fuse_down
@@ -385,10 +411,10 @@ class ResNetEncoder:
             front_chunk = vals[0] if len(vals) == 1 else vals
         self.front_chunk = front_chunk
         # residual stages whose 1x1 downsample is computed inside conv1's launch (BasicBlock networks, bf16 path)
-        env_dual = os.environ.get("PDFUSION_B200_DUAL")               # tuning hook: "" = none, "2,3,4" = those stages
-        self.dual_stages = tuple(int(v) for v in env_dual.split(",") if v) if env_dual is not None else DEFAULT_DUAL_STAGES
-        env_chain = os.environ.get("PDFUSION_B200_CHAIN")             # tuning hook: "" = none, "1,2" = those stages
-        self.chain_stages = tuple(int(v) for v in env_chain.split(",") if v) if env_chain is not None else DEFAULT_CHAIN_STAGES
+        self.dual_stages = _parse_stages("PDFUSION_B200_DUAL", DEFAULT_DUAL_STAGES)          # tuning hook: "2,3,4" = those stages
+        self.chain_stages = _parse_stages("PDFUSION_B200_CHAIN", DEFAULT_CHAIN_STAGES)       # tuning hook: "1,2" = those stages
+        # Bottleneck stages whose downsample is computed inside block 0's conv3 launch (tuning hook: "1,2,3" = those stages)
+        self.shortcut_stages = _parse_stages("PDFUSION_B200_SHORTCUT", DEFAULT_SHORTCUT_STAGES)
         sd = {k: v.detach().to("cpu") for k, v in state_dict.items()}
         self._keep: List[torch.Tensor] = []     # device tensors referenced by the plan
         self._build(sd)
@@ -455,6 +481,15 @@ class ResNetEncoder:
             return self._dev(wf.permute(0, 2, 3, 1).to(torch.bfloat16)), None, self._dev(shift.float())   # [K,R,S,C]
         return self._dev(w.permute(2, 3, 1, 0).float()), self._dev(scale.float()), self._dev(shift.float())  # [R,S,C,K]
 
+    def _shortcut_weights(self, sd, wname, wname_sc, weights):
+        """conv3 with its block's projection shortcut as more K: [W3 | Wds] ([K][c + sc_c] bf16, both BN folded), bias b3 + bds
+        (summed in float64, then rounded once to f32)."""
+        bn = {cv["name"]: cv["bn"] for cv in conv_list(self.arch)}
+        w3, wds = weights[wname][0], weights[wname_sc][0]
+        w = torch.cat([w3.reshape(w3.shape[0], -1), wds.reshape(wds.shape[0], -1)], dim=1)
+        bias = _bn_affine(sd, bn[wname])[1] + _bn_affine(sd, bn[wname_sc])[1]
+        return self._dev(w), None, self._dev(bias.float())
+
     # -- op list ---------------------------------------------------------------------------------
     def _chunk_sizes(self, h2: int, esz: int) -> List[int]:
         """Images per launch for the stem (index 0) and the four residual stages (1..4).
@@ -499,7 +534,8 @@ class ResNetEncoder:
         self.output = torch.empty((n, self.emb_dim), dtype=torch.float32, device=self.device)
         self.chunks = self._chunk_sizes(h2, esz)
         ops, extents, self.final_hw = lower_resnet(self.arch, n, S, self.bf16, self.fused_stem, self.chunks, in_bytes, self.dual_stages,
-                                                     self.chain_stages, os.environ.get("PDFUSION_B200_XCHAIN", "1") != "0")
+                                                     self.chain_stages, os.environ.get("PDFUSION_B200_XCHAIN", "1") != "0",
+                                                     self.shortcut_stages)
         weights = {cv["name"]: self._conv_weights(sd, cv) for cv in conv_list(self.arch)}
 
         self.buffers = {name: torch.empty(nbytes, dtype=torch.uint8, device=self.device) for name, nbytes in extents.items()
@@ -514,6 +550,7 @@ class ResNetEncoder:
             kw = dict(kw)
             wname2 = kw.pop("_weight2", None)
             wname3 = kw.pop("_weight3", None)
+            wname_sc = kw.pop("_shortcut", None)
             for key, v in kw.items():
                 setattr(op, key, v)
             if wname2 is not None:
@@ -525,7 +562,7 @@ class ResNetEncoder:
             for key, (buf, off) in refs.items():
                 setattr(op, key, base[buf] + off)
             if wname is not None:
-                w, sc, b = weights[wname]
+                w, sc, b = weights[wname] if wname_sc is None else self._shortcut_weights(sd, wname, wname_sc, weights)
                 op.d_weight, op.d_scale, op.d_bias = w.data_ptr(), _lib.ptr(sc), b.data_ptr()
             cops.append(op)
             self.op_names.append(name)
