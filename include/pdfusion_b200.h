@@ -175,6 +175,40 @@ int pdf_resize_slices(int batch, int L, int H, int W, int input_size, const floa
 int pdf_decode_volume(int batch, int nifti_datatype, int X, int Y, int Z, int fortran_order, double slope, double inter,
                       const void* d_src, float* d_dst, pdf_stream_t stream);
 
+/* ------------------------------------------------------------------------------------------
+ * Ragged batches: subjects of any raw shape, stored type, byte order and scaling in one batch.  Every stage after the resample
+ * works on the target grid, so only decode and resample need per-subject geometry.  The raw volumes are packed one after the
+ * other in one float32 buffer (C order [X][Y][Z] each, starting at 16-byte aligned offsets); the descriptors are a HOST array
+ * of `batch` entries and reach the kernels as a by-value kernel parameter, so batch <= PDF_RAGGED_MAX_BATCH.
+ * ------------------------------------------------------------------------------------------ */
+#define PDF_RAGGED_MAX_BATCH 64
+typedef struct {
+  int32_t shape[3];       /* X, Y, Z of the raw volume */
+  int32_t nifti_datatype; /* decode only: 2, 4, 8, 16, 64, 256, 512, 768 as pdf_decode_volume */
+  int32_t fortran_order;  /* decode only */
+  int32_t pad;
+  int64_t src_offset;     /* decode only: bytes into d_src (a multiple of the stored element size) */
+  int64_t raw_offset;     /* float32 elements into the packed raw buffer; multiple of 4 (16-byte aligned rows) */
+  double slope, inter;    /* decode only: nibabel's scaling rule, as pdf_decode_volume */
+} pdf_volume_desc;
+
+/* stored voxels of mixed type, order and scaling -> the packed float32 buffer, one launch (same arithmetic as pdf_decode_volume) */
+int pdf_decode_volumes(int batch, const pdf_volume_desc* descs, const void* d_src, float* d_dst, pdf_stream_t stream);
+/* workspace of the ragged entry points: the uniform workspace of `batch` subjects followed by one interpolation table per subject
+ * (pdf_select_bounds_indices, pdf_gather_* and pdf_normalize_volume then work on the same workspace unchanged).  cfg->in_shape is
+ * not read by the ragged entry points. */
+size_t pdf_preproc_ragged_workspace_bytes(const pdf_preproc_cfg* cfg, int batch);
+/* 1 when every subject of the batch can be resampled slice-major (see pdf_preproc_slice_major_ok); a batch with one ineligible
+ * subject runs C-order as a whole */
+int pdf_preproc_slice_major_ok_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs);
+/* pdf_resample_stats / pdf_preprocess with per-subject raw geometry: d_raw is the packed buffer, descs[b].shape / raw_offset
+ * place subject b.  Same outputs, bit for bit, as the uniform entry points on each subject. */
+int pdf_resample_stats_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs, const float* d_raw,
+                              float* d_zoomed, void* d_workspace, pdf_stream_t stream);
+int pdf_preprocess_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs, const float* d_raw, float* d_zoomed,
+                          void* d_workspace, float* d_lohi, int32_t* d_indices, int32_t* d_nslices, void* d_out, int out_mode,
+                          pdf_stream_t stream);
+
 /* normalised volume itself (parity helper for _normalize_volume_for_resnet): d_zoomed -> d_norm */
 int pdf_normalize_volume(int batch, size_t voxels, const float* d_zoomed, const float* d_lohi, float* d_norm,
                          pdf_stream_t stream);

@@ -44,6 +44,28 @@ struct ZoomTables {                  // lives at the head of the workspace
   double w1[3][kPlaneMax];
 };
 
+// Raw geometry of the subjects of one resample launch, passed by value (__grid_constant__: read from the parameter bank, no copy).
+// A uniform batch has one entry and subject b's volume at b * X*Y*Z; a ragged batch has one entry per subject of the launch, and
+// `subj` is the subject's index in the batch (the launch may cover a subset: the bulk-copy kernel takes the subjects whose rows fit
+// its ring, resample_kernel the rest).  NR = input rows a tile touches at the launch's TJ; plane_max = the largest per-subject
+// staging plane of the launch (NR * Z; resample_kernel: rounded up to even), which sizes the shared-memory layout.
+struct ResampleSubj {
+  int X, Y, Z, NR;
+  int subj, pad;
+  long long raw_off;   // float32 elements into the packed raw buffer (ragged)
+  ZoomTables* tabs;
+};
+struct ResampleGeom {
+  int uniform, n, plane_max, pad;
+  ResampleSubj s[PDF_RAGGED_MAX_BATCH];
+};
+
+__device__ __forceinline__ const ResampleSubj& geom_entry(const ResampleGeom& g) { return g.s[g.uniform ? 0 : blockIdx.y]; }
+__device__ __forceinline__ int geom_subject(const ResampleGeom& g) { return g.uniform ? (int)blockIdx.y : g.s[blockIdx.y].subj; }
+__device__ __forceinline__ const float* geom_raw(const ResampleGeom& g, const float* raw, const ResampleSubj& e) {
+  return raw + (g.uniform ? (size_t)blockIdx.y * e.X * e.Y * e.Z : (size_t)e.raw_off);
+}
+
 struct Workspace {
   ZoomTables* tabs;
   SubjState* st;
@@ -80,11 +102,11 @@ static Workspace carve(const pdf_preproc_cfg* cfg, int batch, void* ws) {
   return w;
 }
 
-static int validate(const pdf_preproc_cfg* cfg, int batch) {
+// everything but cfg->in_shape (which the ragged entry points take per subject from their descriptors)
+static int validate_target(const pdf_preproc_cfg* cfg, int batch) {
   PDF_REQUIRE(cfg != nullptr && batch > 0, "preproc: null cfg or batch <= 0");
   for (int i = 0; i < 3; ++i) {
-    PDF_REQUIRE(cfg->in_shape[i] >= 2 && cfg->out_shape[i] >= 2 && cfg->out_shape[i] <= kPlaneMax,
-                "preproc: shapes must be >=2 and target dims <= %d", kPlaneMax);
+    PDF_REQUIRE(cfg->out_shape[i] >= 2 && cfg->out_shape[i] <= kPlaneMax, "preproc: shapes must be >=2 and target dims <= %d", kPlaneMax);
   }
   PDF_REQUIRE(cfg->n_axes >= 1 && cfg->n_axes <= PDF_MAX_AXES, "preproc: n_axes must be 1..3");
   for (int a = 0; a < cfg->n_axes; ++a) {
@@ -97,20 +119,43 @@ static int validate(const pdf_preproc_cfg* cfg, int batch) {
   return PDF_OK;
 }
 
+static int validate(const pdf_preproc_cfg* cfg, int batch) {
+  if (int rc = validate_target(cfg, batch)) return rc;
+  for (int i = 0; i < 3; ++i) PDF_REQUIRE(cfg->in_shape[i] >= 2, "preproc: shapes must be >=2 and target dims <= %d", kPlaneMax);
+  return PDF_OK;
+}
+
+static int validate_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs) {
+  if (int rc = validate_target(cfg, batch)) return rc;
+  PDF_REQUIRE(batch <= PDF_RAGGED_MAX_BATCH && descs, "preproc (ragged): batch must be 1..%d with a descriptor per subject",
+              PDF_RAGGED_MAX_BATCH);
+  for (int b = 0; b < batch; ++b) {
+    const pdf_volume_desc& v = descs[b];
+    PDF_REQUIRE(v.shape[0] >= 2 && v.shape[1] >= 2 && v.shape[2] >= 2, "preproc (ragged): subject %d: raw dims must be >= 2", b);
+    PDF_REQUIRE(v.raw_offset >= 0 && v.raw_offset % 4 == 0, "preproc (ragged): subject %d: raw_offset must be a non-negative "
+                "multiple of 4", b);
+  }
+  return PDF_OK;
+}
+
 // the resample kernel writes slice-major only from its 8-row bulk-copy tiles (see resample_tma_kernel / pdf_resample_stats)
-static bool slice_major_ok(const pdf_preproc_cfg* cfg) {
+static bool slice_major_ok_shape(const pdf_preproc_cfg* cfg, int Y, int Z) {
   if (!cfg || cfg->n_axes != 1 || cfg->axes[0] != 2) return false;
-  const int Y = cfg->in_shape[1], Z = cfg->in_shape[2], T0 = cfg->out_shape[0], T1 = cfg->out_shape[1], T2 = cfg->out_shape[2];
+  const int T0 = cfg->out_shape[0], T1 = cfg->out_shape[1], T2 = cfg->out_shape[2];
   if (Z % 4 != 0 || (T2 + 31) / 32 * 32 > 160 || T1 < 8 || T1 % 8 != 0) return false;
   const double ystep = (double)(Y - 1) / (double)(T1 - 1);
   const int NR = (int)(7 * ystep) + 3;
   const size_t smem = (size_t)kResStages * 2 * NR * Z * 4 + (size_t)(kH0 + T0 + T1) * 4 + 16 + (size_t)T1 * 32 + 2 * kResStages * 8 + 128;
   return smem <= 110 * 1024;
 }
+static bool slice_major_ok(const pdf_preproc_cfg* cfg) { return cfg && slice_major_ok_shape(cfg, cfg->in_shape[1], cfg->in_shape[2]); }
 
 // ------------------------------------------------------------------------------------------------------
-__global__ void init_tables_kernel(ZoomTables* tabs, SubjState* st, int batch, int X, int Y, int Z, int T0, int T1, int T2) {
-  const int src[3] = {X, Y, Z};
+// grid (.., entries of g): one table per geometry entry
+__global__ void init_tables_kernel(const __grid_constant__ ResampleGeom g, SubjState* st, int batch, int T0, int T1, int T2) {
+  const ResampleSubj& e = geom_entry(g);
+  ZoomTables* tabs = e.tabs;
+  const int src[3] = {e.X, e.Y, e.Z};
   const int dst[3] = {T0, T1, T2};
   int t = blockIdx.x * blockDim.x + threadIdx.x;
   for (int a = 0; a < 3; ++a) {
@@ -127,7 +172,7 @@ __global__ void init_tables_kernel(ZoomTables* tabs, SubjState* st, int batch, i
       tabs->w1[a][t] = w1;
     }
   }
-  if (t < batch) st[t].gmin_key = 0xffffffffu;
+  if (blockIdx.y == 0 && t < batch) st[t].gmin_key = 0xffffffffu;
 }
 
 __device__ __forceinline__ double scrub(float v) {  // np.nan_to_num(nan=0, posinf=0, neginf=0)
@@ -140,19 +185,22 @@ __device__ __forceinline__ double scrub(float v) {  // np.nan_to_num(nan=0, posi
 // shared memory.  Blocks are persistent over tiles so the histogram / plane-maximum partials are flushed once.
 __global__ void __launch_bounds__(256)
 resample_kernel(const float* __restrict__ raw, float* __restrict__ zoomed, SubjState* __restrict__ states,
-                const ZoomTables* __restrict__ tabs, int X, int Y, int Z, int T0, int T1, int T2, int TJ, int NR) {
+                const __grid_constant__ ResampleGeom g, int T0, int T1, int T2, int TJ) {
   extern __shared__ __align__(16) unsigned char sm_raw[];
+  const ResampleSubj& ge = geom_entry(g);
+  const ZoomTables* __restrict__ tabs = ge.tabs;
+  const int Y = ge.Y, Z = ge.Z, NR = ge.NR;
   double* s_in = reinterpret_cast<double*>(sm_raw);                      // [2][NR][Z]
-  uint32_t* s_hist = reinterpret_cast<uint32_t*>(s_in + 2 * (((size_t)NR * Z + 1) & ~(size_t)1));
+  uint32_t* s_hist = reinterpret_cast<uint32_t*>(s_in + 2 * (size_t)g.plane_max);
   uint32_t* s_imax = s_hist + kH0;
   uint32_t* s_jmax = s_imax + T0;
-  const int b = blockIdx.y;
+  const int b = geom_subject(g);
   const int tid = threadIdx.x, nthr = blockDim.x;
   for (int i = tid; i < kH0 + T0 + T1; i += nthr) s_hist[i] = 0;        // hist, imax, jmax are contiguous
   __syncthreads();
 
   SubjState* st = states + b;
-  const float* rb = raw + (size_t)b * X * Y * Z;
+  const float* rb = geom_raw(g, raw, ge);
   float* zb = zoomed + (size_t)b * T0 * T1 * T2;
   const int tiles_per_i = (T1 + TJ - 1) / TJ;
   const int ntiles = T0 * tiles_per_i;
@@ -281,9 +329,12 @@ __device__ __forceinline__ uint32_t key_of(float f) { return float_to_ordered(f)
 template <bool NEED_JMAX, bool ZMAJOR>
 __global__ void __launch_bounds__(352, 2)
 resample_tma_kernel(const float* __restrict__ raw, float* __restrict__ zoomed, SubjState* __restrict__ states,
-                    const ZoomTables* __restrict__ tabs, int X, int Y, int Z, int T0, int T1, int T2, int TJ, int NR, int KT) {
+                    const __grid_constant__ ResampleGeom g, int T0, int T1, int T2, int TJ, int KT) {
   extern __shared__ __align__(16) unsigned char sm_raw[];
-  const uint32_t stage_bytes = (uint32_t)(2 * NR * Z * 4);
+  const ResampleSubj& ge = geom_entry(g);
+  const ZoomTables* __restrict__ tabs = ge.tabs;
+  const int Y = ge.Y, Z = ge.Z, NR = ge.NR;
+  const uint32_t stage_bytes = (uint32_t)(2 * g.plane_max * 4);
   float* s_stage = reinterpret_cast<float*>(sm_raw);
   uint32_t* s_hist = reinterpret_cast<uint32_t*>(sm_raw + (size_t)kResStages * stage_bytes);
   uint32_t* s_imax = s_hist + kH0;
@@ -293,7 +344,7 @@ resample_tma_kernel(const float* __restrict__ raw, float* __restrict__ zoomed, S
   off += (size_t)T1 * sizeof(JEntry);
   uint64_t* s_bar = reinterpret_cast<uint64_t*>(sm_raw + off);
   const uint32_t bar_full = smem_u32(s_bar), bar_empty = bar_full + kResStages * 8;
-  const int b = blockIdx.y;
+  const int b = geom_subject(g);
   const int tid = threadIdx.x, nthr = blockDim.x;
   const int n_cwarps = (nthr - 32) / 32;
   for (int i = tid; i < kH0 + T0 + T1; i += nthr) s_hist[i] = 0;
@@ -310,7 +361,7 @@ resample_tma_kernel(const float* __restrict__ raw, float* __restrict__ zoomed, S
   __syncthreads();
 
   SubjState* st = states + b;
-  const float* rb = raw + (size_t)b * X * Y * Z;
+  const float* rb = geom_raw(g, raw, ge);
   float* zb = zoomed + (size_t)b * T0 * T1 * T2;
   const int tiles_per_i = (T1 + TJ - 1) / TJ;
   const int ntiles = T0 * tiles_per_i;
@@ -1083,13 +1134,8 @@ __device__ __forceinline__ float decode_one(T v, bool scale, double slope, doubl
 // Fortran-order source: a 32 (x) by 32 (z) tile is transposed through shared memory so that both the reads (x fastest) and the
 // writes (z fastest) are coalesced.  grid (ceil(X/32), ceil(Z/32), Y * batch), block (32, 8).
 template <typename T>
-__global__ void __launch_bounds__(256)
-decode_fortran_kernel(const T* __restrict__ src, float* __restrict__ dst, int X, int Y, int Z, bool scale, double slope, double inter) {
-  __shared__ float tile[32][33];
-  const int b = blockIdx.z / Y, y = blockIdx.z - b * Y;
-  const int x0 = blockIdx.x * 32, z0 = blockIdx.y * 32;
-  const T* sb = src + (size_t)b * X * Y * Z;
-  float* db = dst + (size_t)b * X * Y * Z;
+__device__ __forceinline__ void decode_fortran_tile(const T* __restrict__ sb, float* __restrict__ db, int X, int Y, int Z, int x0, int y,
+                                                    int z0, bool scale, double slope, double inter, float (*tile)[33]) {
 #pragma unroll
   for (int k = 0; k < 32; k += 8) {
     const int x = x0 + threadIdx.x, z = z0 + threadIdx.y + k;
@@ -1101,6 +1147,15 @@ decode_fortran_kernel(const T* __restrict__ src, float* __restrict__ dst, int X,
     const int x = x0 + threadIdx.y + k, z = z0 + threadIdx.x;
     if (x < X && z < Z) db[((size_t)x * Y + y) * Z + z] = tile[threadIdx.x][threadIdx.y + k];
   }
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256)
+decode_fortran_kernel(const T* __restrict__ src, float* __restrict__ dst, int X, int Y, int Z, bool scale, double slope, double inter) {
+  __shared__ float tile[32][33];
+  const int b = blockIdx.z / Y, y = blockIdx.z - b * Y;
+  decode_fortran_tile<T>(src + (size_t)b * X * Y * Z, dst + (size_t)b * X * Y * Z, X, Y, Z, blockIdx.x * 32, y, blockIdx.y * 32, scale,
+                         slope, inter, tile);
 }
 
 template <typename T>
@@ -1125,16 +1180,115 @@ static int launch_decode(int batch, int X, int Y, int Z, int fortran, bool scale
   return PDF_OK;
 }
 
+// Ragged decode: one launch over subjects of mixed type, order and scaling.  Blocks are numbered through the subjects (blk_start:
+// first block of each subject); a Fortran-order subject gets one block per 32 x 32 (x, z) tile and y, as decode_fortran_kernel, a
+// C-order subject one block per kDecodeChunk voxels.  The datatype is a per-block switch: every block decodes one subject.
+constexpr int kDecodeChunk = 4096;
+struct DecodeSubj {
+  long long src_off, raw_off;   // bytes into d_src; float32 elements into d_dst
+  int X, Y, Z, code, fortran, scale;
+  double slope, inter;
+};
+struct DecodeGeom {
+  int n, pad;
+  int blk_start[PDF_RAGGED_MAX_BATCH + 1];
+  DecodeSubj s[PDF_RAGGED_MAX_BATCH];
+};
+
+template <typename T>
+__device__ __forceinline__ void decode_ragged_block(const unsigned char* __restrict__ src, float* __restrict__ dst, const DecodeSubj& d,
+                                                    int blk, float (*tile)[33]) {
+  const T* sb = reinterpret_cast<const T*>(src + d.src_off);
+  float* db = dst + d.raw_off;
+  if (d.fortran) {
+    const int gx = (d.X + 31) / 32, gxz = gx * ((d.Z + 31) / 32);
+    const int y = blk / gxz, r = blk - y * gxz, zt = r / gx, xt = r - zt * gx;
+    decode_fortran_tile<T>(sb, db, d.X, d.Y, d.Z, xt * 32, y, zt * 32, d.scale != 0, d.slope, d.inter, tile);
+  } else {
+    const size_t n = (size_t)d.X * d.Y * d.Z, end = min(n, (size_t)(blk + 1) * kDecodeChunk);
+    for (size_t i = (size_t)blk * kDecodeChunk + threadIdx.y * 32 + threadIdx.x; i < end; i += 256)
+      db[i] = decode_one(sb[i], d.scale != 0, d.slope, d.inter);
+  }
+}
+
+__global__ void __launch_bounds__(256)
+decode_ragged_kernel(const unsigned char* __restrict__ src, float* __restrict__ dst, const __grid_constant__ DecodeGeom g) {
+  __shared__ float tile[32][33];
+  int lo = 0, hi = g.n - 1;                     // last subject whose first block is <= blockIdx.x
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (g.blk_start[mid] <= (int)blockIdx.x) lo = mid;
+    else hi = mid - 1;
+  }
+  const DecodeSubj& d = g.s[lo];
+  const int blk = (int)blockIdx.x - g.blk_start[lo];
+  switch (d.code) {
+    case 2: decode_ragged_block<uint8_t>(src, dst, d, blk, tile); break;
+    case 4: decode_ragged_block<int16_t>(src, dst, d, blk, tile); break;
+    case 8: decode_ragged_block<int32_t>(src, dst, d, blk, tile); break;
+    case 16: decode_ragged_block<float>(src, dst, d, blk, tile); break;
+    case 64: decode_ragged_block<double>(src, dst, d, blk, tile); break;
+    case 256: decode_ragged_block<int8_t>(src, dst, d, blk, tile); break;
+    case 512: decode_ragged_block<uint16_t>(src, dst, d, blk, tile); break;
+    default: decode_ragged_block<uint32_t>(src, dst, d, blk, tile); break;   // 768 (the host admits no other code)
+  }
+}
+
+static int nifti_elem_bytes(int code) {
+  switch (code) {
+    case 2: case 256: return 1;
+    case 4: case 512: return 2;
+    case 8: case 16: case 768: return 4;
+    case 64: return 8;
+    default: return 0;
+  }
+}
+
+// nibabel applies the scaling only when scl_slope is finite and non-zero and (slope, inter) != (1, 0); a non-finite inter counts as 0
+static bool nifti_scales(double slope, double inter) { return slope != 0.0 && isfinite(slope) && !(slope == 1.0 && inter == 0.0); }
+
 }  // namespace pdf
 
 using namespace pdf;
+
+extern "C" int pdf_decode_volumes(int batch, const pdf_volume_desc* descs, const void* d_src, float* d_dst, pdf_stream_t stream) {
+  PDF_REQUIRE(batch > 0 && batch <= PDF_RAGGED_MAX_BATCH && descs && d_src && d_dst,
+              "pdf_decode_volumes: bad arguments (batch must be 1..%d)", PDF_RAGGED_MAX_BATCH);
+  DecodeGeom g;
+  memset(&g, 0, sizeof(g));
+  g.n = batch;
+  long long blocks = 0;
+  for (int b = 0; b < batch; ++b) {
+    const pdf_volume_desc& v = descs[b];
+    const int eb = nifti_elem_bytes(v.nifti_datatype);
+    PDF_REQUIRE(eb > 0, "pdf_decode_volumes: subject %d: unsupported NIfTI datatype %d", b, v.nifti_datatype);
+    PDF_REQUIRE(v.shape[0] > 0 && v.shape[1] > 0 && v.shape[2] > 0, "pdf_decode_volumes: subject %d: bad shape", b);
+    PDF_REQUIRE(v.src_offset >= 0 && v.src_offset % eb == 0, "pdf_decode_volumes: subject %d: src_offset must be a non-negative "
+                "multiple of the element size", b);
+    PDF_REQUIRE(v.raw_offset >= 0 && v.raw_offset % 4 == 0, "pdf_decode_volumes: subject %d: raw_offset must be a non-negative "
+                "multiple of 4", b);
+    DecodeSubj& d = g.s[b];
+    d.src_off = v.src_offset; d.raw_off = v.raw_offset;
+    d.X = v.shape[0]; d.Y = v.shape[1]; d.Z = v.shape[2];
+    d.code = v.nifti_datatype; d.fortran = v.fortran_order ? 1 : 0;
+    d.scale = nifti_scales(v.slope, v.inter) ? 1 : 0;
+    d.slope = v.slope; d.inter = isfinite(v.inter) ? v.inter : 0.0;
+    g.blk_start[b] = (int)blocks;
+    blocks += d.fortran ? (long long)ceil_div(d.X, 32) * ceil_div(d.Z, 32) * d.Y
+                        : ((long long)d.X * d.Y * d.Z + kDecodeChunk - 1) / kDecodeChunk;
+    PDF_REQUIRE(blocks < (1LL << 31), "pdf_decode_volumes: batch too large for one launch");
+  }
+  g.blk_start[batch] = (int)blocks;
+  decode_ragged_kernel<<<(unsigned)blocks, dim3(32, 8), 0, as_stream(stream)>>>(reinterpret_cast<const unsigned char*>(d_src), d_dst, g);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
 
 extern "C" int pdf_decode_volume(int batch, int nifti_datatype, int X, int Y, int Z, int fortran_order, double slope, double inter,
                                  const void* d_src, float* d_dst, pdf_stream_t stream) {
   PDF_REQUIRE(batch > 0 && X > 0 && Y > 0 && Z > 0 && d_src && d_dst, "pdf_decode_volume: bad arguments");
   PDF_REQUIRE((long long)Y * batch <= 65535, "pdf_decode_volume: Y * batch exceeds the grid limit");
-  // nibabel applies the scaling only when scl_slope is finite and non-zero and (slope, inter) != (1, 0)
-  const bool scale = slope != 0.0 && isfinite(slope) && !(slope == 1.0 && inter == 0.0);
+  const bool scale = nifti_scales(slope, inter);
   if (!isfinite(inter)) inter = 0.0;
   cudaStream_t s = as_stream(stream);
   switch (nifti_datatype) {
@@ -1158,100 +1312,177 @@ using namespace pdf;
 
 static int g_pre_chunk = 0;   // subjects per pdf_preprocess sub-batch (0 = whole batch); pdf_debug_set_pre_chunk
 
-extern "C" int pdf_preproc_slice_major_ok(const pdf_preproc_cfg* cfg) { return slice_major_ok(cfg) ? 1 : 0; }
-
-extern "C" size_t pdf_preproc_workspace_bytes(const pdf_preproc_cfg* cfg, int batch) {
-  if (!cfg || batch <= 0) return 0;
+static size_t uniform_workspace_bytes(const pdf_preproc_cfg* cfg, int batch) {
   size_t n = align_up(sizeof(ZoomTables), 256) + align_up(sizeof(SubjState) * (size_t)batch, 256);
   n += align_up((size_t)batch * count_axis2(cfg) * cfg->out_shape[0] * cfg->out_shape[1] * sizeof(float), 256);
   n += (size_t)batch * cand_capacity(cfg) * sizeof(uint32_t);
   return n + 256;
 }
 
+// per-subject interpolation tables of a ragged call: after the uniform regions, which keep their places
+static ZoomTables* ragged_tables(const pdf_preproc_cfg* cfg, int batch, void* ws) {
+  return reinterpret_cast<ZoomTables*>(reinterpret_cast<char*>(ws) + align_up(uniform_workspace_bytes(cfg, batch), 256));
+}
+
+extern "C" int pdf_preproc_slice_major_ok(const pdf_preproc_cfg* cfg) { return slice_major_ok(cfg) ? 1 : 0; }
+
+extern "C" int pdf_preproc_slice_major_ok_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs) {
+  if (!cfg || !descs || batch <= 0 || batch > PDF_RAGGED_MAX_BATCH) return 0;
+  for (int b = 0; b < batch; ++b)
+    if (!slice_major_ok_shape(cfg, descs[b].shape[1], descs[b].shape[2])) return 0;
+  return 1;
+}
+
+extern "C" size_t pdf_preproc_workspace_bytes(const pdf_preproc_cfg* cfg, int batch) {
+  if (!cfg || batch <= 0) return 0;
+  return uniform_workspace_bytes(cfg, batch);
+}
+
+extern "C" size_t pdf_preproc_ragged_workspace_bytes(const pdf_preproc_cfg* cfg, int batch) {
+  if (!cfg || batch <= 0 || batch > PDF_RAGGED_MAX_BATCH) return 0;
+  return align_up(uniform_workspace_bytes(cfg, batch), 256) + (size_t)batch * sizeof(ZoomTables);
+}
+
+// K1a for a uniform batch (descs == nullptr: geometry from cfg->in_shape, subject b at b * X*Y*Z) or a ragged one.  Every subject
+// goes through the bulk-copy kernel when its rows fit the staging ring at two rows per tile (Z % 4 == 0, <= 110 KB), the others
+// through resample_kernel in a second launch.  The tile height TJ of each launch is chosen once, for its largest subject.
+static int resample_impl(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs, const float* d_raw, float* d_zoomed,
+                         void* d_workspace, cudaStream_t s) {
+  Workspace w = carve(cfg, batch, d_workspace);
+  const int T0 = cfg->out_shape[0], T1 = cfg->out_shape[1], T2 = cfg->out_shape[2];
+  const int n = descs ? batch : 1;                      // geometry entries
+  ZoomTables* rtabs = descs ? ragged_tables(cfg, batch, d_workspace) : nullptr;
+  ResampleGeom gi;                                      // all entries: interpolation tables
+  memset(&gi, 0, sizeof(gi));
+  gi.uniform = descs ? 0 : 1;
+  gi.n = n;
+  for (int e = 0; e < n; ++e) {
+    ResampleSubj& r = gi.s[e];
+    const int32_t* sh = descs ? descs[e].shape : cfg->in_shape;
+    r.X = sh[0]; r.Y = sh[1]; r.Z = sh[2];
+    r.subj = e;
+    r.raw_off = descs ? descs[e].raw_offset : 0;
+    r.tabs = descs ? rtabs + e : w.tabs;
+  }
+  const size_t fixed = (size_t)(kH0 + T0 + T1) * sizeof(uint32_t);
+  const int KT = (T2 + 31) / 32 * 32;
+  const bool tma_batch = ((reinterpret_cast<uintptr_t>(d_raw) & 15) == 0) && KT <= 160 && T1 >= 2;
+  auto rows = [&](const ResampleSubj& r, int TJ) { return (int)((TJ - 1) * ((double)(r.Y - 1) / (double)(T1 - 1))) + 3; };
+  // bulk-copy pipeline: TJ output rows per tile, kResStages stages of 2 x NR x Z floats
+  auto tma_smem = [&](size_t plane) { return (size_t)kResStages * 2 * plane * 4 + fixed + 16 + (size_t)T1 * 32 + 2 * kResStages * 8 + 128; };
+  auto res_smem = [&](size_t plane_even) { return 2 * plane_even * sizeof(double) + fixed; };
+  bool tma[PDF_RAGGED_MAX_BATCH];
+  int n_tma = 0;
+  for (int e = 0; e < n; ++e) {
+    const ResampleSubj& r = gi.s[e];
+    tma[e] = tma_batch && r.Z % 4 == 0 && tma_smem((size_t)rows(r, 2) * r.Z) <= 110 * 1024;
+    n_tma += tma[e];
+  }
+  bool need_jmax = false;
+  for (int a = 0; a < cfg->n_axes; ++a) need_jmax |= cfg->axes[a] == 1;
+  ResampleGeom gt, gr;                                   // the two launches
+  int TJt = 8, TJr = 8;
+  size_t smem_t = 0, smem_r = 0;
+  if (n_tma) {
+    for (; TJt >= 2; TJt >>= 1) {
+      size_t plane = 0;
+      for (int e = 0; e < n; ++e) if (tma[e]) plane = max(plane, (size_t)rows(gi.s[e], TJt) * gi.s[e].Z);
+      smem_t = tma_smem(plane);
+      if (smem_t <= 110 * 1024) break;
+    }
+    memset(&gt, 0, sizeof(gt));
+    gt.uniform = gi.uniform;
+    for (int e = 0; e < n; ++e) {
+      if (!tma[e]) continue;
+      ResampleSubj r = gi.s[e];
+      r.NR = rows(r, TJt);
+      gt.plane_max = max(gt.plane_max, r.NR * r.Z);
+      gt.s[gt.n++] = r;
+    }
+    if (cfg->slice_major)
+      PDF_REQUIRE(n_tma == n && TJt == 8 && T1 % 8 == 0 && !need_jmax, "pdf_resample_stats: slice_major needs 8-row tiles (T1 %% 8 == 0, "
+                  "rows that fit the staging ring) -- check pdf_preproc_slice_major_ok first");
+  }
+  if (n_tma < n) {
+    PDF_REQUIRE(!cfg->slice_major, "pdf_resample_stats: slice_major needs the bulk-copy resample kernel (Z %% 4 == 0, T2 <= 160): check "
+                "pdf_preproc_slice_major_ok first");
+    // rows per tile: as many as fit the shared-memory staging buffer (2 planes x NR input rows x Z doubles)
+    size_t plane = 0;
+    for (; TJr >= 1; TJr >>= 1) {
+      plane = 0;
+      for (int e = 0; e < n; ++e) if (!tma[e]) plane = max(plane, ((size_t)rows(gi.s[e], TJr) * gi.s[e].Z + 1) & ~(size_t)1);
+      smem_r = res_smem(plane);
+      if (smem_r <= 72 * 1024 || TJr == 1) break;
+    }
+    PDF_REQUIRE(smem_r <= 200 * 1024, "pdf_resample_stats: volume rows too long for the shared-memory staging buffer");
+    memset(&gr, 0, sizeof(gr));
+    gr.uniform = gi.uniform;
+    gr.plane_max = (int)plane;
+    for (int e = 0; e < n; ++e) {
+      if (tma[e]) continue;
+      ResampleSubj r = gi.s[e];
+      r.NR = rows(r, TJr);
+      gr.s[gr.n++] = r;
+    }
+  }
+
+  PDF_CHECK_CUDA(cudaMemsetAsync(w.st, 0, sizeof(SubjState) * (size_t)batch, s));
+  const int tmax = max(max(T0, T1), max(T2, batch));
+  init_tables_kernel<<<dim3(ceil_div(tmax, 256), n), 256, 0, s>>>(gi, w.st, batch, T0, T1, T2);
+  PDF_CHECK_LAUNCH();
+  // subjects per launch: all of a uniform batch (one geometry entry), else the launch's entries
+  const int sub_t = descs ? gt.n : batch, sub_r = descs ? gr.n : batch;
+  if (n_tma) {
+    const int variant = cfg->slice_major ? 2 : (need_jmax ? 1 : 0);
+    static size_t configured[3] = {0, 0, 0};
+    if (smem_t > configured[variant]) {
+      if (variant == 2) PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_tma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
+      else if (need_jmax) PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_tma_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
+      else PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_tma_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_t));
+      configured[variant] = smem_t;
+    }
+    const int ntiles = T0 * ceil_div(T1, TJt);
+    const int per_sm = max(1, min(4, (int)((220 * 1024) / (smem_t + 1024))));
+    // one resident wave: never more blocks than the chip holds at once (a second partial wave would double the time)
+    const dim3 grid(max(1, min(ntiles, (num_sms() * per_sm) / sub_t)), sub_t);
+    if (variant == 2) resample_tma_kernel<false, true><<<grid, 32 + 2 * KT, smem_t, s>>>(d_raw, d_zoomed, w.st, gt, T0, T1, T2, TJt, KT);
+    else if (need_jmax) resample_tma_kernel<true, false><<<grid, 32 + 2 * KT, smem_t, s>>>(d_raw, d_zoomed, w.st, gt, T0, T1, T2, TJt, KT);
+    else resample_tma_kernel<false, false><<<grid, 32 + 2 * KT, smem_t, s>>>(d_raw, d_zoomed, w.st, gt, T0, T1, T2, TJt, KT);
+    PDF_CHECK_LAUNCH();
+  }
+  if (n_tma < n) {
+    static size_t configured = 0;
+    if (smem_r > configured) {
+      PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_r));
+      configured = smem_r;
+    }
+    const int threads = min(256, (T2 + 31) / 32 * 32);
+    const int ntiles = T0 * ceil_div(T1, TJr);
+    const int per_sm = max(1, min(8, (int)((220 * 1024) / (smem_r + 1024))));
+    const dim3 grid(max(1, min(ntiles, ceil_div(num_sms() * per_sm, sub_r))), sub_r);
+    resample_kernel<<<grid, threads, smem_r, s>>>(d_raw, d_zoomed, w.st, gr, T0, T1, T2, TJr);
+    PDF_CHECK_LAUNCH();
+  }
+  return PDF_OK;
+}
+
 extern "C" int pdf_resample_stats(const pdf_preproc_cfg* cfg, int batch, const float* d_raw, float* d_zoomed,
                                   void* d_workspace, pdf_stream_t stream) {
   if (int rc = validate(cfg, batch)) return rc;
   PDF_REQUIRE(d_raw && d_zoomed && d_workspace, "pdf_resample_stats: null device pointer");
-  cudaStream_t s = as_stream(stream);
-  Workspace w = carve(cfg, batch, d_workspace);
-  const int X = cfg->in_shape[0], Y = cfg->in_shape[1], Z = cfg->in_shape[2];
-  const int T0 = cfg->out_shape[0], T1 = cfg->out_shape[1], T2 = cfg->out_shape[2];
-  PDF_CHECK_CUDA(cudaMemsetAsync(w.st, 0, sizeof(SubjState) * (size_t)batch, s));
-  const int tmax = max(max(T0, T1), max(T2, batch));
-  init_tables_kernel<<<ceil_div(tmax, 256), 256, 0, s>>>(w.tabs, w.st, batch, X, Y, Z, T0, T1, T2);
-  PDF_CHECK_LAUNCH();
-  const double ystep = (double)(Y - 1) / (double)(T1 - 1);
-  const size_t fixed = (size_t)(kH0 + T0 + T1) * sizeof(uint32_t);
-  const int KT = (T2 + 31) / 32 * 32;
-  const bool tma_ok = (Z % 4 == 0) && ((reinterpret_cast<uintptr_t>(d_raw) & 15) == 0) && KT <= 160 && T1 >= 2;
-  if (tma_ok) {
-    // bulk-copy pipeline: 8 output rows per tile, kResStages stages of 2 x NR x Z floats
-    int TJ = 8, NR = 0;
-    size_t smem = 0;
-    for (; TJ >= 2; TJ >>= 1) {
-      NR = (int)((TJ - 1) * ystep) + 3;
-      smem = (size_t)kResStages * 2 * NR * Z * 4 + fixed + 16 + (size_t)T1 * 32 + 2 * kResStages * 8 + 128;
-      if (smem <= 110 * 1024) break;
-    }
-    if (TJ >= 2 && smem <= 200 * 1024) {
-      bool need_jmax = false;
-      for (int a = 0; a < cfg->n_axes; ++a) need_jmax |= cfg->axes[a] == 1;
-      static size_t configured[3] = {0, 0, 0};
-      const int variant = cfg->slice_major ? 2 : (need_jmax ? 1 : 0);
-      if (cfg->slice_major)
-        PDF_REQUIRE(TJ == 8 && T1 % 8 == 0 && !need_jmax, "pdf_resample_stats: slice_major needs 8-row tiles (T1 %% 8 == 0, rows that fit "
-                    "the staging ring) -- check pdf_preproc_slice_major_ok first");
-      if (smem > configured[variant]) {
-        if (variant == 2) PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_tma_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        else if (need_jmax) PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_tma_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        else PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_tma_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured[variant] = smem;
-      }
-      const int ntiles = T0 * ceil_div(T1, TJ);
-      const int per_sm = max(1, min(4, (int)((220 * 1024) / (smem + 1024))));
-      // one resident wave: never more blocks than the chip holds at once (a second partial wave would double the time)
-      const int blocks_per_subject = max(1, min(ntiles, (num_sms() * per_sm) / batch));
-      if (variant == 2)
-        resample_tma_kernel<false, true><<<dim3(blocks_per_subject, batch), 32 + 2 * KT, smem, s>>>(d_raw, d_zoomed, w.st, w.tabs, X, Y, Z,
-                                                                                                  T0, T1, T2, TJ, NR, KT);
-      else if (need_jmax)
-        resample_tma_kernel<true, false><<<dim3(blocks_per_subject, batch), 32 + 2 * KT, smem, s>>>(d_raw, d_zoomed, w.st, w.tabs, X, Y, Z,
-                                                                                                  T0, T1, T2, TJ, NR, KT);
-      else
-        resample_tma_kernel<false, false><<<dim3(blocks_per_subject, batch), 32 + 2 * KT, smem, s>>>(d_raw, d_zoomed, w.st, w.tabs, X, Y, Z,
-                                                                                                   T0, T1, T2, TJ, NR, KT);
-      PDF_CHECK_LAUNCH();
-      return PDF_OK;
-    }
-  }
-  PDF_REQUIRE(!cfg->slice_major, "pdf_resample_stats: slice_major needs the bulk-copy resample kernel (Z %% 4 == 0, T2 <= 160): check "
-              "pdf_preproc_slice_major_ok first");
-  const int threads = min(256, (T2 + 31) / 32 * 32);
-  // rows per tile: as many as fit the shared-memory staging buffer (2 planes x NR input rows x Z doubles)
-  int TJ = 8, NR = 0;
-  size_t smem = 0;
-  for (; TJ >= 1; TJ >>= 1) {
-    NR = (int)((TJ - 1) * ystep) + 3;
-    smem = 2 * (((size_t)NR * Z + 1) & ~(size_t)1) * sizeof(double) + fixed;
-    if (smem <= 72 * 1024 || TJ == 1) break;
-  }
-  PDF_REQUIRE(smem <= 200 * 1024, "pdf_resample_stats: volume rows too long for the shared-memory staging buffer (Z=%d)", Z);
-  static size_t configured = 0;
-  if (smem > configured) {
-    PDF_CHECK_CUDA(cudaFuncSetAttribute(resample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    configured = smem;
-  }
-  const int ntiles = T0 * ceil_div(T1, TJ);
-  const int per_sm = max(1, min(8, (int)((220 * 1024) / (smem + 1024))));
-  const int blocks_per_subject = max(1, min(ntiles, ceil_div(num_sms() * per_sm, batch)));
-  resample_kernel<<<dim3(blocks_per_subject, batch), threads, smem, s>>>(d_raw, d_zoomed, w.st, w.tabs, X, Y, Z, T0, T1, T2, TJ, NR);
-  PDF_CHECK_LAUNCH();
-  return PDF_OK;
+  return resample_impl(cfg, batch, nullptr, d_raw, d_zoomed, d_workspace, as_stream(stream));
+}
+
+extern "C" int pdf_resample_stats_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs, const float* d_raw,
+                                         float* d_zoomed, void* d_workspace, pdf_stream_t stream) {
+  if (int rc = validate_ragged(cfg, batch, descs)) return rc;
+  PDF_REQUIRE(d_raw && d_zoomed && d_workspace, "pdf_resample_stats_ragged: null device pointer");
+  return resample_impl(cfg, batch, descs, d_raw, d_zoomed, d_workspace, as_stream(stream));
 }
 
 extern "C" int pdf_select_bounds_indices(const pdf_preproc_cfg* cfg, int batch, const float* d_zoomed, void* d_workspace,
                                          float* d_lohi, int32_t* d_indices, int32_t* d_nslices, pdf_stream_t stream) {
-  if (int rc = validate(cfg, batch)) return rc;
+  if (int rc = validate_target(cfg, batch)) return rc;     // in_shape is not read here (ragged batches leave it unset)
   PDF_REQUIRE(d_zoomed && d_workspace && d_lohi && d_indices && d_nslices, "pdf_select_bounds_indices: null device pointer");
   cudaStream_t s = as_stream(stream);
   Workspace w = carve(cfg, batch, d_workspace);
@@ -1304,7 +1535,7 @@ static bool launch_resize_band(const ResizeArgs& ra, int out_mode, int batch, co
 extern "C" int pdf_gather_resize_normalize(const pdf_preproc_cfg* cfg, int batch, const float* d_zoomed, void* d_workspace,
                                               const float* d_lohi, const int32_t* d_indices, const int32_t* d_nslices,
                                               void* d_out, int out_mode, pdf_stream_t stream) {
-  if (int rc = validate(cfg, batch)) return rc;
+  if (int rc = validate_target(cfg, batch)) return rc;     // in_shape is not read here (ragged batches leave it unset)
   PDF_REQUIRE(d_zoomed && d_workspace && d_lohi && d_indices && d_nslices && d_out, "pdf_gather_resize_normalize: null device pointer");
   PDF_REQUIRE(out_mode == PDF_OUT_BF16_C1 || out_mode == PDF_OUT_F32_NHWC3 || out_mode == PDF_OUT_BF16_C1_PAD,
               "pdf_gather_resize_normalize: bad out_mode");
@@ -1362,10 +1593,10 @@ extern "C" int pdf_gather_resize_normalize(const pdf_preproc_cfg* cfg, int batch
   return PDF_OK;
 }
 
-extern "C" int pdf_preprocess(const pdf_preproc_cfg* cfg, int batch, const float* d_raw, float* d_zoomed, void* d_workspace,
-                              float* d_lohi, int32_t* d_indices, int32_t* d_nslices, void* d_out, int out_mode,
-                              pdf_stream_t stream) {
-  if (int rc = validate(cfg, batch)) return rc;
+// descs == nullptr: uniform batch of cfg->in_shape volumes; else the ragged batch the descriptors place in d_raw
+static int preprocess_impl(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs, const float* d_raw, float* d_zoomed,
+                           void* d_workspace, float* d_lohi, int32_t* d_indices, int32_t* d_nslices, void* d_out, int out_mode,
+                           pdf_stream_t stream) {
   // Sub-batches: the resampled volumes of one sub-batch (8.4 MB each at 128^3) stay L2-resident between the resample kernel,
   // the two refinement-histogram passes and the plane gather, instead of streaming B x 8.4 MB through HBM four times.
   const int chunk = (g_pre_chunk > 0 && g_pre_chunk < batch) ? g_pre_chunk : batch;
@@ -1382,17 +1613,32 @@ extern "C" int pdf_preprocess(const pdf_preproc_cfg* cfg, int batch, const float
   const size_t vout = (size_t)cfg->out_shape[0] * cfg->out_shape[1] * cfg->out_shape[2];
   for (int b0 = 0; b0 < batch; b0 += chunk) {
     const int nb = min(chunk, batch - b0);
-    const float* raw = d_raw + (size_t)b0 * vin;
+    const float* raw = descs ? d_raw : d_raw + (size_t)b0 * vin;
     float* zoomed = d_zoomed + (size_t)b0 * vout;
     float* lohi = d_lohi + 4 * (size_t)b0;
     int32_t* indices = d_indices + (size_t)b0 * lmax;
     int32_t* nslices = d_nslices + (size_t)b0 * cfg->n_axes;
     void* out = reinterpret_cast<char*>(d_out) + (size_t)b0 * out_bytes;
-    if (int rc = pdf_resample_stats(cfg, nb, raw, zoomed, d_workspace, stream)) return rc;
+    if (int rc = descs ? pdf_resample_stats_ragged(cfg, nb, descs + b0, raw, zoomed, d_workspace, stream)
+                       : pdf_resample_stats(cfg, nb, raw, zoomed, d_workspace, stream)) return rc;
     if (int rc = pdf_select_bounds_indices(cfg, nb, zoomed, d_workspace, lohi, indices, nslices, stream)) return rc;
     if (int rc = pdf_gather_resize_normalize(cfg, nb, zoomed, d_workspace, lohi, indices, nslices, out, out_mode, stream)) return rc;
   }
   return PDF_OK;
+}
+
+extern "C" int pdf_preprocess(const pdf_preproc_cfg* cfg, int batch, const float* d_raw, float* d_zoomed, void* d_workspace,
+                              float* d_lohi, int32_t* d_indices, int32_t* d_nslices, void* d_out, int out_mode,
+                              pdf_stream_t stream) {
+  if (int rc = validate(cfg, batch)) return rc;
+  return preprocess_impl(cfg, batch, nullptr, d_raw, d_zoomed, d_workspace, d_lohi, d_indices, d_nslices, d_out, out_mode, stream);
+}
+
+extern "C" int pdf_preprocess_ragged(const pdf_preproc_cfg* cfg, int batch, const pdf_volume_desc* descs, const float* d_raw,
+                                     float* d_zoomed, void* d_workspace, float* d_lohi, int32_t* d_indices, int32_t* d_nslices,
+                                     void* d_out, int out_mode, pdf_stream_t stream) {
+  if (int rc = validate_ragged(cfg, batch, descs)) return rc;
+  return preprocess_impl(cfg, batch, descs, d_raw, d_zoomed, d_workspace, d_lohi, d_indices, d_nslices, d_out, out_mode, stream);
 }
 
 extern "C" int pdf_debug_set_pre_chunk(int subjects) {
@@ -1411,7 +1657,7 @@ extern "C" int pdf_normalize_volume(int batch, size_t voxels, const float* d_zoo
 
 extern "C" int pdf_gather_slices(const pdf_preproc_cfg* cfg, int batch, const float* d_zoomed, const float* d_lohi,
                                  const int32_t* d_indices, const int32_t* d_nslices, float* d_slices, pdf_stream_t stream) {
-  if (int rc = validate(cfg, batch)) return rc;
+  if (int rc = validate_target(cfg, batch)) return rc;     // in_shape is not read here (ragged batches leave it unset)
   PDF_REQUIRE(d_zoomed && d_lohi && d_indices && d_nslices && d_slices, "pdf_gather_slices: null device pointer");
   PDF_REQUIRE(!cfg->slice_major, "pdf_gather_slices reads the C-order resampled volume (slice_major = 0)");
   FinalizeArgs fa;

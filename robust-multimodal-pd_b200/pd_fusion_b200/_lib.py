@@ -15,6 +15,7 @@ LIB_PATH = Path(os.environ.get("PDFUSION_B200_LIB", _HERE / "libpdfusion_b200.so
 PDF_MAX_AXES = 3
 PDF_MAX_LAYERS = 8
 PDF_MAX_MODS = 8
+PDF_RAGGED_MAX_BATCH = 64
 
 OUT_BF16_C1 = 0
 OUT_F32_NHWC3 = 1
@@ -37,6 +38,20 @@ class PreprocCfg(C.Structure):
         ("std", C.c_float * 3),
         ("extent_raw", C.c_int32),
         ("slice_major", C.c_int32),
+    ]
+
+
+class VolumeDesc(C.Structure):
+    """pdf_volume_desc: one subject of a ragged batch (raw geometry, and how its stored voxels decode)."""
+    _fields_ = [
+        ("shape", C.c_int32 * 3),
+        ("nifti_datatype", C.c_int32),
+        ("fortran_order", C.c_int32),
+        ("pad", C.c_int32),
+        ("src_offset", C.c_int64),
+        ("raw_offset", C.c_int64),
+        ("slope", C.c_double),
+        ("inter", C.c_double),
     ]
 
 
@@ -112,6 +127,11 @@ PROTOTYPES = {
     "pdf_resize_slices": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float), _P, _P, C.c_int, _P]),
     "pdf_normalize_volume": (C.c_int, [C.c_int, C.c_size_t, _P, _P, _P, _P]),
     "pdf_decode_volume": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, _P, _P, _P]),
+    "pdf_decode_volumes": (C.c_int, [C.c_int, C.POINTER(VolumeDesc), _P, _P, _P]),
+    "pdf_preproc_ragged_workspace_bytes": (C.c_size_t, [C.POINTER(PreprocCfg), C.c_int]),
+    "pdf_preproc_slice_major_ok_ragged": (C.c_int, [C.POINTER(PreprocCfg), C.c_int, C.POINTER(VolumeDesc)]),
+    "pdf_resample_stats_ragged": (C.c_int, [C.POINTER(PreprocCfg), C.c_int, C.POINTER(VolumeDesc), _P, _P, _P, _P]),
+    "pdf_preprocess_ragged": (C.c_int, [C.POINTER(PreprocCfg), C.c_int, C.POINTER(VolumeDesc), _P, _P, _P, _P, _P, _P, _P, C.c_int, _P]),
     "pdf_stem_padded_dims": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "pdf_plan_create": (C.c_int, [C.POINTER(_P), C.POINTER(Op), C.c_int]),
     "pdf_plan_run": (C.c_int, [_P, _P]),

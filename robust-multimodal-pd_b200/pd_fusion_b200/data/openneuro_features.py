@@ -26,7 +26,7 @@ from .. import _lib
 from ..backbone import RESNET_SPECS, ResNet2D
 from ..parallel import all_gather_rows, barrier, init_distributed, shard_range, world
 from ..pipeline import EmbeddingPipeline
-from ..preprocess import VolumePreprocessor
+from ..preprocess import RaggedBatch, VolumePreprocessor, ragged_offsets
 from ..utils.npz_writer import savez_compressed_parallel
 
 
@@ -54,14 +54,11 @@ _NP_TO_NIFTI = {"uint8": 2, "int16": 4, "int32": 8, "float32": 16, "float64": 64
 
 class StoredVolume:
     """Voxels as they are stored, plus what is needed to turn them into the reference's float32 array on the device
-    (`pdf_decode_volume`): NIfTI datatype code, [X, Y, Z], storage order, scl_slope / scl_inter."""
+    (`pdf_decode_volumes`): NIfTI datatype code, [X, Y, Z], storage order, scl_slope / scl_inter."""
     __slots__ = ("voxels", "code", "shape", "fortran", "slope", "inter")
 
     def __init__(self, voxels, code, shape, fortran, slope=1.0, inter=0.0):
         self.voxels, self.code, self.shape, self.fortran, self.slope, self.inter = voxels, int(code), tuple(shape), bool(fortran), float(slope), float(inter)
-
-    def key(self):
-        return (self.code, self.shape, self.fortran, self.slope, self.inter)
 
     def to_float32(self) -> np.ndarray:
         """Host restatement of `get_fdata().astype(np.float32)` (C-order [X, Y, Z]); the batched path decodes on the device."""
@@ -150,18 +147,38 @@ class _ReadAhead:
             self.pool.shutdown(wait=False)
 
 
-def _decode_on_device(batch, dev) -> torch.Tensor:
-    """Stored voxels of same-keyed volumes -> float32 [B, X, Y, Z] on `dev`: the upload carries the file's bytes (half of the
-    float32 array for the usual int16 T1 image), `pdf_decode_volume` does the float64 scaling, the cast and the transpose."""
-    v0 = batch[0]
-    host = torch.from_numpy(np.stack([b.voxels for b in batch]).view(np.uint8)).pin_memory()       # bytes as stored
-    src = host.to(dev, non_blocking=True)
-    out = torch.empty((len(batch),) + v0.shape, dtype=torch.float32, device=dev)
-    lib = _lib.load()
-    _lib.check(lib.pdf_decode_volume(len(batch), v0.code, v0.shape[0], v0.shape[1], v0.shape[2], int(v0.fortran), v0.slope, v0.inter,
-                                     src.data_ptr(), out.data_ptr(), _lib.stream_ptr()), "pdf_decode_volume")
-    src.record_stream(torch.cuda.current_stream(dev))
-    return out
+_DECODE_BUFS: Dict[torch.device, List[torch.Tensor]] = {}
+
+
+def _decode_on_device(batch, dev) -> RaggedBatch:
+    """StoredVolumes of any shapes, stored types, orders and scalings -> a RaggedBatch on `dev`.  One pinned upload carries the
+    files' bytes, each volume at a 16-byte aligned offset (half of the float32 array for the usual int16 T1 image); one
+    `pdf_decode_volumes` launch does the float64 scaling, the cast and the transpose of every subject.  The device buffers are
+    reused by the next call on the current stream and grow only when a larger batch arrives: consume a batch before decoding the
+    next one on another stream."""
+    src_offs, n_src = [], 0
+    for v in batch:
+        src_offs.append(n_src)
+        n_src += (v.voxels.nbytes + 15) // 16 * 16
+    raw_offs, n_raw = ragged_offsets([v.shape for v in batch])
+    descs = (_lib.VolumeDesc * len(batch))()
+    host = torch.empty(n_src, dtype=torch.uint8, pin_memory=True)
+    hb = host.numpy()
+    for b, v in enumerate(batch):
+        d = descs[b]
+        d.shape[:] = list(v.shape)
+        d.nifti_datatype, d.fortran_order, d.src_offset, d.raw_offset = v.code, int(v.fortran), src_offs[b], raw_offs[b]
+        d.slope, d.inter = v.slope, v.inter
+        hb[src_offs[b]:src_offs[b] + v.voxels.nbytes] = np.ascontiguousarray(v.voxels).reshape(-1).view(np.uint8)   # bytes as stored
+    bufs = _DECODE_BUFS.get(dev)
+    if bufs is None or bufs[0].numel() < n_src or bufs[1].numel() < n_raw:
+        old = (0, 0) if bufs is None else (bufs[0].numel(), bufs[1].numel())
+        bufs = _DECODE_BUFS[dev] = [torch.empty(max(old[0], n_src), dtype=torch.uint8, device=dev),
+                                    torch.empty(max(old[1], n_raw), dtype=torch.float32, device=dev)]
+    src, raw = bufs
+    src[:n_src].copy_(host, non_blocking=True)
+    _lib.check(_lib.load().pdf_decode_volumes(len(batch), descs, src.data_ptr(), raw.data_ptr(), _lib.stream_ptr()), "pdf_decode_volumes")
+    return RaggedBatch(raw, descs)
 
 
 # ---------------------------------------------------------------------------------------------------
@@ -171,7 +188,7 @@ _PRE_CACHE: Dict[tuple, VolumePreprocessor] = {}
 
 
 def _preprocessor(in_shape, target_shape, axes=(2,), counts=(1,), input_size=8, mode=_lib.OUT_F32_NHWC3, max_batch: int = 1) -> VolumePreprocessor:
-    key = (tuple(in_shape), tuple(target_shape), tuple(axes), tuple(counts), int(input_size), mode, int(max_batch), torch.cuda.current_device())
+    key = (None if in_shape is None else tuple(in_shape), tuple(target_shape), tuple(axes), tuple(counts), int(input_size), mode, int(max_batch), torch.cuda.current_device())
     if key not in _PRE_CACHE:
         _PRE_CACHE[key] = VolumePreprocessor(in_shape, target_shape, axes, counts, input_size, out_mode=mode, max_batch=int(max_batch))
     return _PRE_CACHE[key]
@@ -243,6 +260,11 @@ def _apply_affine_2d(slice_2d: np.ndarray, angle_deg: float, translate: np.ndarr
 # ---------------------------------------------------------------------------------------------------
 # batched builders
 # ---------------------------------------------------------------------------------------------------
+def _subject_batch() -> int:
+    """PD_FUSION_B200_SUBJECT_BATCH, capped at the largest ragged batch the library takes in one call"""
+    return min(max(1, int(os.environ.get("PD_FUSION_B200_SUBJECT_BATCH", "8"))), _lib.PDF_RAGGED_MAX_BATCH)
+
+
 def _mean_std(weights) -> Tuple[List[float], List[float]]:
     if hasattr(weights, "meta"):
         return list(weights.meta.get("mean", [0.5, 0.5, 0.5])), list(weights.meta.get("std", [0.5, 0.5, 0.5]))
@@ -267,7 +289,7 @@ def embed_manifest(df: pd.DataFrame, backbone: str, target_shape: Sequence[int],
     dev = torch.device("cuda", local_rank)
     torch.cuda.set_device(dev)
     precision = os.environ.get("PD_FUSION_B200_PRECISION", "bf16")
-    bsz = max(1, int(os.environ.get("PD_FUSION_B200_SUBJECT_BATCH", "8")))
+    bsz = _subject_batch()
     model, emb_dim, weights = _build_resnet_backbone(backbone)
     mean, std = _mean_std(weights)
     sd = {k: v for k, v in model.state_dict().items() if not k.startswith("fc.")}
@@ -277,32 +299,23 @@ def embed_manifest(df: pd.DataFrame, backbone: str, target_shape: Sequence[int],
     emb = torch.zeros((hi - lo, L, emb_dim), dtype=torch.float32, device=dev)
     avg = torch.zeros((hi - lo, emb_dim), dtype=torch.float32, device=dev)
     nsl = torch.zeros((hi - lo,), dtype=torch.int32, device=dev)
-    pipes: Dict[tuple, EmbeddingPipeline] = {}
+    # one pipeline (one encoder) serves every raw shape: a batch is the next bsz rows, whatever their geometry and stored type
+    pipe = EmbeddingPipeline(sd, None, target_shape, axes, counts, input_size, precision, bsz, mean, std,
+                             "resnet50" if backbone == "resnet50" else "resnet18", dev)
     paths = df["t1wbrain_path"].tolist()
     reader = _ReadAhead(paths, lo, hi, window=2 * bsz)     # files are read and gunzipped by worker threads, ahead of the GPU
-    i = lo
-    while i < hi:
-        first = reader.get(i)
-        batch, j = [first], i + 1
-        while j < hi and len(batch) < bsz:
-            nxt = reader.get(j)
-            if nxt.key() != first.key():                 # same shape, stored type and scaling: one decode launch
-                break
-            batch.append(nxt)
-            j += 1
+    for i in range(lo, hi, bsz):
+        j = min(hi, i + bsz)
+        batch = [reader.get(k) for k in range(i, j)]
         reader.release(i, j)
-        if first.shape not in pipes:
-            pipes[first.shape] = EmbeddingPipeline(sd, first.shape, target_shape, axes, counts, input_size, precision, bsz,
-                                                   mean, std, "resnet50" if backbone == "resnet50" else "resnet18", dev)
         raw = _decode_on_device(batch, dev)
         if tta > 1:
-            res = pipes[first.shape].embed_tta(raw, [tta_seeds[k] for k in range(i, j)], tta, tta_cfg)
+            res = pipe.embed_tta(raw, [tta_seeds[k] for k in range(i, j)], tta, tta_cfg)
         else:
-            res = pipes[first.shape].embed(raw)
+            res = pipe.embed(raw)
         emb[i - lo:j - lo].copy_(res.embeddings)
         avg[i - lo:j - lo].copy_(res.mean)
         nsl[i - lo:j - lo].copy_(res.nslices.sum(dim=1))
-        i = j
     if ws > 1:
         emb, avg, nsl = all_gather_rows(emb, n_rows), all_gather_rows(avg, n_rows), all_gather_rows(nsl, n_rows)
     torch.cuda.synchronize()
@@ -464,25 +477,17 @@ def load_simple_features(manifest_path: Path, cache_dir: Path, config: Dict) -> 
     target_shape = tuple(int(v) for v in config.get("target_shape", (96, 96, 96)))
     extra_stats = bool(config.get("extra_stats", False))
     dev = torch.device("cuda", torch.cuda.current_device())
-    bsz = max(1, int(os.environ.get("PD_FUSION_B200_SUBJECT_BATCH", "8")))
+    bsz = _subject_batch()
     paths = df["t1wbrain_path"].tolist()
     reader = _ReadAhead(paths, 0, len(paths), window=2 * bsz)
+    pre = _preprocessor(None, target_shape, max_batch=bsz)
     feats: List[np.ndarray] = []
-    i = 0
-    while i < len(paths):
-        first = reader.get(i)
-        batch, j = [first], i + 1
-        while j < len(paths) and len(batch) < bsz:
-            nxt = reader.get(j)
-            if nxt.key() != first.key():
-                break
-            batch.append(nxt)
-            j += 1
+    for i in range(0, len(paths), bsz):
+        j = min(len(paths), i + bsz)
+        batch = [reader.get(k) for k in range(i, j)]
         reader.release(i, j)
-        raw = _decode_on_device(batch, dev)
-        zoomed = _preprocessor(first.shape, target_shape, max_batch=bsz).resample(raw)
+        zoomed = pre.resample(_decode_on_device(batch, dev))
         feats.append(_simple_features_device(zoomed, hist_bins, grid_size, extra_stats))
-        i = j
     F = np.concatenate(feats, axis=0).astype(np.float64)          # the reference stores python floats -> float64 columns
     cols = {"subject_id": df["subject_id"].values, "session": df["session"].values, "label": df["label"].astype(int).values}
     cols.update({f"mri_feat_{k}": F[:, k] for k in range(F.shape[1])})

@@ -7,9 +7,10 @@ Bags are volume paths (str / Path) or ready slice stacks (np.ndarray [L, H, W] i
   launch, instead of the reference's per-bag, per-16-slice-chunk loop (`_forward_bags`, :135-162).
   `tta_inference > 1` re-augments each bag with `pdf_tta_augment` (unseeded Generator, as in the reference :267-272).
 * `train` -- forward/backward with train-mode BatchNorm, focal/BCE loss, gradient clipping, Adam with two learning rates
-  (:164-253) -- is host-side torch autograd on the CUDA device.  The dgrad/wgrad tensor-core kernels of BASELINE
-  config 5 are NOT built yet (DESIGN.md section 6); only the volume preparation of the training loop uses the CUDA kernels.
-  The `state_dict` layout ({"backbone": ..., "attn": ...}) is the reference's.
+  (:164-253) -- runs on the native kernels of training.py (ResNetTrainer, MilHeadTrainer, NativeAdam); the nn.Modules only
+  hold the parameters.  The `state_dict` layout ({"backbone": ..., "attn": ...}) is the reference's.
+* Path bags of one `predict_proba` / `train_step` call are prepared together on the device: one ragged decode -> resample ->
+  slice select -> slice gather over volumes of any shapes (`_device_stacks`), the same slices `_bag_slices` returns per bag.
 """
 from __future__ import annotations
 
@@ -71,6 +72,7 @@ class MilAttentionFineTuneModel(BaseModel):
         #  on first use by _trainers(); its moments persist across train() calls like the reference's self.optimizer)
         self.pos_weight = None if (p.get("class_weight") == "balanced" or p.get("pos_weight") is None) else float(p["pos_weight"])
         self._native: Dict[str, object] = {}
+        self._slicer: Optional[VolumePreprocessor] = None
         self._trainer = None
 
     # ------------------------------------------------------------------------------------------ native inference
@@ -113,6 +115,45 @@ class MilAttentionFineTuneModel(BaseModel):
             return bag.astype(np.float32, copy=False)
         vol = onf._normalize_volume_for_resnet(onf._load_volume(bag, target_shape=self.target_shape))
         return np.concatenate([onf._select_slices(vol, a, c) for a, c in zip(self.axes, self.counts)], axis=0).astype(np.float32, copy=False)
+
+    def _path_stacks(self, paths) -> List[torch.Tensor]:
+        """`_bag_slices` of volume paths, computed together: ragged batches of stored volumes are decoded, resampled, normalised,
+        sliced and gathered on the device ([n_i, H, W] f32 each, the valid slices of every axis group in order)."""
+        bsz = onf._subject_batch()
+        if not paths:
+            return []
+        if self._slicer is None:          # only resample / select / gather_slices are used: the network-input size is moot
+            self._slicer = VolumePreprocessor(None, self.target_shape, self.axes, self.counts, 8, out_mode=_lib.OUT_F32_NHWC3,
+                                              max_batch=bsz, device=self.device)
+        pre = self._slicer
+        out: List[torch.Tensor] = []
+        for i in range(0, len(paths), bsz):
+            raw = onf._decode_on_device([onf._read_volume_stored(p) for p in paths[i:i + bsz]], self.device)
+            B = len(raw)
+            pre.resample(raw)
+            _, _, nslices = pre.select(B)
+            slices = pre.gather_slices(B)
+            ns = nslices.cpu().numpy()
+            for b in range(B):
+                offs = np.cumsum([0] + self.counts[:-1])
+                out.append(torch.cat([slices[b, o:o + int(ns[b, a])] for a, o in enumerate(offs)], dim=0).clone())
+        return out
+
+    def _device_stacks(self, bags) -> List[Optional[torch.Tensor]]:
+        """Slice stacks [L, H, W] f32 on the device of every bag (None stays None): path bags through `_path_stacks` in one go,
+        tensors as they are, arrays uploaded."""
+        from_paths = iter(self._path_stacks([b for b in bags if _is_path(b)]))
+        out: List[Optional[torch.Tensor]] = []
+        for bag in bags:
+            if bag is None:
+                out.append(None)
+            elif _is_path(bag):
+                out.append(next(from_paths))
+            elif isinstance(bag, torch.Tensor):
+                out.append(bag.to(device=self.device, dtype=torch.float32))
+            else:
+                out.append(torch.from_numpy(np.ascontiguousarray(self._bag_slices(bag))).to(self.device))
+        return out
 
     def _capacity(self, longest: int) -> int:
         """Images per encoder pass: a FIXED capacity (bag_batch_size bags of the nominal length, at least 256 images), so that ONE
@@ -171,7 +212,7 @@ class MilAttentionFineTuneModel(BaseModel):
             return out
         self.backbone.eval()
         self.attn.eval()
-        stacks = [torch.from_numpy(np.ascontiguousarray(self._bag_slices(bags[i]))).to(self.device) for i in live]
+        stacks = self._device_stacks([bags[i] for i in live])
         passes = max(1, self.tta_inference)
         acc = torch.zeros(len(live), dtype=torch.float32, device=self.device)
         head = self._head()
@@ -230,14 +271,10 @@ class MilAttentionFineTuneModel(BaseModel):
         rt, ht, opt = self._trainers()
         pre = self._train_resizer()
         stacks, groups = [], [0]
-        for bag in batch_bags:
+        for bag, sl in zip(batch_bags, self._device_stacks(batch_bags)):
             if bag is None:
                 stacks.append(None)
                 continue
-            if isinstance(bag, torch.Tensor):                                       # slice stack already resident on the device
-                sl = bag.to(device=self.device, dtype=torch.float32)
-            else:
-                sl = torch.from_numpy(np.ascontiguousarray(self._bag_slices(bag))).to(self.device)
             if augment and self.train_aug and not isinstance(bag, (np.ndarray, torch.Tensor)):   # the reference augments bags it loads itself
                 sl = self._augment(sl, np.random.default_rng())
             stacks.append(sl)

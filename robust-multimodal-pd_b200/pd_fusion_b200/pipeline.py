@@ -14,7 +14,7 @@ import torch
 
 from . import _lib
 from .backbone import ResNetEncoder, detect_arch
-from .preprocess import VolumePreprocessor
+from .preprocess import RaggedBatch, VolumePreprocessor
 
 
 @dataclass
@@ -26,10 +26,12 @@ class EmbedResult:
 
 
 class EmbeddingPipeline:
-    def __init__(self, backbone_state_dict: Dict[str, torch.Tensor], in_shape: Sequence[int],
+    def __init__(self, backbone_state_dict: Dict[str, torch.Tensor], in_shape: Sequence[int] | None,
                  target_shape: Sequence[int] = (160, 160, 160), axes: Sequence[int] = (2,), counts: Sequence[int] = (24,),
                  input_size: int = 224, precision: str = "bf16", max_subjects: int = 8, mean=(0.5, 0.5, 0.5),
                  std=(0.5, 0.5, 0.5), arch: str | None = None, device=None):
+        """in_shape None: one pipeline for subjects of every raw shape -- embed() / embed_tta() then take a RaggedBatch
+        (see VolumePreprocessor); the end-to-end embed_host / embed_overlapped paths need a fixed in_shape."""
         _lib.require_cuda()
         self.lib = _lib.load()
         self.device = torch.device(device if device is not None else f"cuda:{torch.cuda.current_device()}")
@@ -58,10 +60,10 @@ class EmbeddingPipeline:
             self.mean_out = torch.empty((self.max_subjects, self.D), dtype=torch.float32, device=self.device)
             self.nvalid = torch.empty((self.max_subjects,), dtype=torch.int32, device=self.device)
 
-    def embed(self, raw: torch.Tensor) -> EmbedResult:
-        """raw [B<=max_subjects, X, Y, Z] f32 on the device. Enqueues everything on the current stream; results
-        live in reused buffers (copy them out before the next call)."""
-        B = int(raw.shape[0])
+    def embed(self, raw) -> EmbedResult:
+        """raw [B<=max_subjects, X, Y, Z] f32 on the device, or a RaggedBatch of B subjects (in_shape None). Enqueues everything
+        on the current stream; results live in reused buffers (copy them out before the next call)."""
+        B = len(raw) if isinstance(raw, RaggedBatch) else int(raw.shape[0])
         if B < self.max_subjects:   # the encoder plan is built for max_subjects*L images: clear the unused tail
             self.enc.input[B * self.L:].zero_()
         res = self.pre.run(raw, net_input=self._net_input)
@@ -149,7 +151,7 @@ class EmbeddingPipeline:
             ov["slot_free"][s].record(Cs)
         return EmbedResult(emb[:B], ov["mean"][s][:B], ov["indices"][s][:B], ov["nslices"][s][:B])
 
-    def embed_tta(self, raw: torch.Tensor, seeds, n_pass: int, tta_cfg: Dict) -> EmbedResult:
+    def embed_tta(self, raw, seeds, n_pass: int, tta_cfg: Dict) -> EmbedResult:
         """`tta > 1` path of the builders (data/openneuro_features.py:235-265): every pass re-augments the selected slices
         (affine, intensity, noise, clip), runs the backbone, and the per-slice / slice-mean embeddings are averaged over the
         passes.  seeds[b] seeds subject b's numpy Generator (the reference: abs(hash(str(subject_id))) % 2**32)."""
@@ -157,7 +159,7 @@ class EmbeddingPipeline:
 
         from .data.tta import draw_passes, params_bytes
 
-        B = int(raw.shape[0])
+        B = len(raw) if isinstance(raw, RaggedBatch) else int(raw.shape[0])
         self.pre.resample(raw)
         _, indices, nslices = self.pre.select(B)
         slices = self.pre.gather_slices(B)

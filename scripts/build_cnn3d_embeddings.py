@@ -20,12 +20,14 @@ from pd_fusion_b200.data import openneuro_features as onf
 def load_volumes(paths, target_shape, dev) -> torch.Tensor:
     """`load_volume` for every manifest row (scripts/build_cnn3d_embeddings.py:28-41) -> [S, D, H, W] f32 on the device."""
     out = []
-    reader = onf._ReadAhead(paths, 0, len(paths), window=8)
-    for i in range(len(paths)):
-        sv = reader.get(i)
-        reader.release(i, i + 1)
-        raw = onf._decode_on_device([sv], dev)
-        zoomed = onf._preprocessor(sv.shape, tuple(target_shape)).resample(raw)
+    bsz = onf._subject_batch()
+    reader = onf._ReadAhead(paths, 0, len(paths), window=2 * bsz)
+    pre = onf._preprocessor(None, tuple(target_shape), max_batch=bsz)      # ragged: one batch mixes every raw geometry
+    for i in range(0, len(paths), bsz):
+        j = min(len(paths), i + bsz)
+        batch = [reader.get(k) for k in range(i, j)]
+        reader.release(i, j)
+        zoomed = pre.resample(onf._decode_on_device(batch, dev))
         out.append(standardize_volumes(zoomed).clone())
     return torch.cat(out, dim=0)
 
