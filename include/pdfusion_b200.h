@@ -333,6 +333,22 @@ int pdf_mil_sweep(const pdf_mil_weights* w, int n_bags, int Lmax, const float* d
 int pdf_mil_forward(const pdf_mil_weights* w, int n_bags, int Lmax, const float* d_bags, const int32_t* d_len,
                     void* d_workspace, float* d_prob, pdf_stream_t stream);
 
+/* Explanations of the MIL head (csrc/explain.cu), always with the FP32 arithmetic of pdf_mil_sweep's PDF_PREC_F32 path, also for a
+ * model that predicts with PDF_PREC_TF32.  For every bag: d_logit [n_bags] = w_cls . sum_l a_l h_l + b_cls, pooled in the order of
+ * the sweep's pooling kernel (sigmoid(logit) is its probability; NaN for a bag with d_len 0); d_attn [n_bags, Lmax] = the attention
+ * weights a_l; d_contrib [n_bags, Lmax] = a_l (w_cls . h_l), so sum_l contrib + b_cls = logit (both 0 on the padding).
+ * d_dx [n_bags, Lmax, D] or NULL: the gradient of the logit (dz = 1, not of a loss) with respect to every instance, 0 on the padding
+ * and for missing bags.  Workspace: pdf_mil_explain_workspace_bytes. */
+size_t pdf_mil_explain_workspace_bytes(const pdf_mil_weights* w, int n_bags, int Lmax);
+int pdf_mil_explain(const pdf_mil_weights* w, int n_bags, int Lmax, const float* d_bags, const int32_t* d_len, void* d_workspace,
+                    float* d_logit, float* d_attn, float* d_contrib, float* d_dx /* [n_bags, Lmax, D] or NULL */, pdf_stream_t stream);
+/* Grad-CAM at a feature map whose spatial mean is the embedding: d_fmap [n, hw, hw, c] f32 (c % 4 == 0, 16-byte aligned),
+ * d_g [n, c] = the gradient of the logit with respect to the embedding.
+ *   cam_small[n, i, j] = ReLU(sum_c g[n, c] fmap[n, i, j, c] / hw^2)      (d_cam_small [n, hw, hw] or NULL)
+ *   cam[n, out_h, out_w] = bilinear upsample of cam_small, align_corners=False (ATen's source-index rule).  hw <= 64. */
+int pdf_gradcam(int n, int hw, int c, const float* d_fmap, const float* d_g, int out_h, int out_w,
+                float* d_cam_small /* [n, hw, hw] or NULL */, float* d_cam /* [n, out_h, out_w] */, pdf_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * K5 -- training (FP32, NHWC).  Replaces torch autograd under MilAttentionFineTuneModel.train / _forward_bags
  * (models/mil_attention_finetune.py:135-162,164-253: backbone in TRAIN mode, BatchNorm statistics per 16-slice chunk, MIL head,

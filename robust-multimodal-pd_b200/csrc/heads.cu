@@ -61,7 +61,7 @@ gemm_nt_f32_kernel(const float* __restrict__ A, int lda, const float* __restrict
   }
 }
 
-static int gemm_nt(const float* A, int lda, const float* B, int ldb, float* C, int ldc, const float* bias, int M, int N, int K,
+int gemm_nt(const float* A, int lda, const float* B, int ldb, float* C, int ldc, const float* bias, int M, int N, int K,
                    int relu, cudaStream_t s) {
   dim3 grid(ceil_div(M, 64), ceil_div(N, 64));
   gemm_nt_f32_kernel<<<grid, 256, 0, s>>>(A, lda, B, ldb, C, ldc, bias, M, N, K, relu);

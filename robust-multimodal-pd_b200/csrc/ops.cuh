@@ -64,6 +64,10 @@ int launch_conv3x3_halo(const TcConv& tc, cudaStream_t s);
 bool gemm_tf32_supported(int N, int K);
 int launch_gemm_tf32(const float* A, const float* B, int M, int N, int K, int mode, int gated, int A_dim, const float* bias,
                      const float* w_w, const float* b_w, float* out, cudaStream_t s);
+// FP32 FFMA GEMM C[M,N] = A[M,K] B[N,K]^T (+bias) (ReLU) of the MIL head (heads.cu: gemm_nt_f32_kernel); also used by explain.cu so
+// that explanations see the same h and attention pre-activations as pdf_mil_sweep's FP32 path
+int gemm_nt(const float* A, int lda, const float* B, int ldb, float* C, int ldc, const float* bias, int M, int N, int K, int relu,
+            cudaStream_t s);
 bool pw_eligible(const pdf_op& op);
 int prepare_conv_pw(const pdf_op& op, TcConv* tc);
 int launch_conv_pw(const TcConv& tc, cudaStream_t s);

@@ -142,6 +142,9 @@ PROTOTYPES = {
     "pdf_mil_workspace_bytes": (C.c_size_t, [C.POINTER(MilWeights), C.c_int, C.c_int]),
     "pdf_mil_forward": (C.c_int, [C.POINTER(MilWeights), C.c_int, C.c_int, _P, _P, _P, _P, _P]),
     "pdf_mil_sweep": (C.c_int, [C.POINTER(MilWeights), C.c_int, C.c_int, _P, _P, C.c_int, _P, C.c_int, _P, _P, _P]),
+    "pdf_mil_explain_workspace_bytes": (C.c_size_t, [C.POINTER(MilWeights), C.c_int, C.c_int]),
+    "pdf_mil_explain": (C.c_int, [C.POINTER(MilWeights), C.c_int, C.c_int, _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pdf_gradcam": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, _P, C.c_int, C.c_int, _P, _P, _P]),
     "pdf_moddrop_workspace_bytes": (C.c_size_t, [C.POINTER(Mlp), C.c_int]),
     "pdf_moddrop_sweep": (C.c_int, [C.POINTER(Mlp), C.c_int, C.c_int, _P, _P, _P, _P, _P]),
     "pdf_moe_sweep": (C.c_int, [C.POINTER(Moe), C.c_int, C.c_int, C.POINTER(_P), _P, _P, _P]),

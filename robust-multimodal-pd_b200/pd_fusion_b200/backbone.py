@@ -598,5 +598,11 @@ class ResNetEncoder:
         _lib.check(self.lib.pdf_plan_run(self.plan, _lib.stream_ptr()), "pdf_plan_run")
         return self.output
 
+    def feature_map(self) -> torch.Tensor:
+        """The last stage's output of the latest run, [n, hw, hw, D] f32 (the average-pool input: the embedding is its spatial
+        mean).  A read-only view of an encoder buffer that the next run overwrites."""
+        hw = self.final_hw
+        return self.buffers["o4"][: self.n * hw * hw * self.emb_dim * 4].view(torch.float32).view(self.n, hw, hw, self.emb_dim)
+
     def run_range(self, first: int, count: int) -> None:
         _lib.check(self.lib.pdf_plan_run_range(self.plan, first, count, _lib.stream_ptr()), "pdf_plan_run_range")

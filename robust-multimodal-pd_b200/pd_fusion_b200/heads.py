@@ -1,5 +1,5 @@
 """Host side of K3/K4: thin wrappers that marshal state_dict tensors into the C structs of
-pdf_mil_forward / pdf_moddrop_sweep / pdf_moe_sweep.  No arithmetic happens here.
+pdf_mil_forward / pdf_mil_explain / pdf_gradcam / pdf_moddrop_sweep / pdf_moe_sweep.  No arithmetic happens here.
 """
 from __future__ import annotations
 
@@ -91,6 +91,44 @@ class MilHead:
     def forward(self, bags: torch.Tensor, lens: torch.Tensor) -> torch.Tensor:
         """bags [n, Lmax, D] f32 cuda (zero padded), lens [n] i32 cuda (0 = missing) -> prob [n] f32."""
         return self.sweep(bags, lens)[0]
+
+    def explain(self, bags: torch.Tensor, lens: torch.Tensor, need_grad: bool = False):
+        """bags [n, Lmax, D] f32 cuda (zero padded), lens [n] i32 (0 = missing) -> device tensors (logit [n], attn [n, Lmax],
+        contrib [n, Lmax], dX [n, Lmax, D] or None) of pdf_mil_explain: attention weights, per-instance logit contributions
+        (sum + b_cls = logit), and with need_grad the gradient of the logit with respect to every instance.  Always the FP32 head
+        arithmetic, whatever `precision` says: sigmoid(logit) is the probability of the "fp32" sweep.  Missing bags: NaN logit,
+        zero attention, contributions and gradient."""
+        if bags.dtype != torch.float32 or not bags.is_cuda or not bags.is_contiguous() or bags.shape[2] != self.D:
+            raise ValueError("bags must be a contiguous float32 CUDA tensor [n, Lmax, D]")
+        n, lmax = int(bags.shape[0]), int(bags.shape[1])
+        lens = lens.to(device=bags.device, dtype=torch.int32).contiguous()
+        need = int(self.lib.pdf_mil_explain_workspace_bytes(C.byref(self.w), n, lmax))
+        ws = torch.empty(need, dtype=torch.uint8, device=bags.device)
+        logit = torch.empty(n, dtype=torch.float32, device=bags.device)
+        attn = torch.empty((n, lmax), dtype=torch.float32, device=bags.device)
+        contrib = torch.empty((n, lmax), dtype=torch.float32, device=bags.device)
+        dX = torch.empty_like(bags) if need_grad else None
+        _lib.check(self.lib.pdf_mil_explain(C.byref(self.w), n, lmax, bags.data_ptr(), lens.data_ptr(), ws.data_ptr(), logit.data_ptr(),
+                                            attn.data_ptr(), contrib.data_ptr(), _lib.ptr(dX), _lib.stream_ptr()), "pdf_mil_explain")
+        return logit, attn, contrib, dX
+
+
+def gradcam(fmap: torch.Tensor, g: torch.Tensor, out_hw, cam_small: bool = False):
+    """Grad-CAM of pdf_gradcam: fmap [n, hw, hw, C] f32 cuda (the feature map whose spatial mean is the embedding), g [n, C] f32 =
+    d logit / d embedding -> cam [n, out_h, out_w] = bilinear upsample (align_corners=False) of ReLU(sum_c g fmap / hw^2),
+    unnormalised; with cam_small also that [n, hw, hw] map: (cam, cam_small or None)."""
+    n, hw, hw2, c = (int(v) for v in fmap.shape)
+    if hw != hw2 or fmap.dtype != torch.float32 or not fmap.is_cuda or not fmap.is_contiguous():
+        raise ValueError("fmap must be a contiguous float32 CUDA tensor [n, hw, hw, C]")
+    if tuple(g.shape) != (n, c):
+        raise ValueError("g must be [n, C]")
+    g = g.to(device=fmap.device, dtype=torch.float32).contiguous()
+    oh, ow = (int(v) for v in out_hw)
+    cam = torch.empty((n, oh, ow), dtype=torch.float32, device=fmap.device)
+    small = torch.empty((n, hw, hw), dtype=torch.float32, device=fmap.device) if cam_small else None
+    _lib.check(_lib.load().pdf_gradcam(n, hw, c, fmap.data_ptr(), g.data_ptr(), oh, ow, _lib.ptr(small), cam.data_ptr(), _lib.stream_ptr()),
+               "pdf_gradcam")
+    return cam, small
 
 
 def _fill_mlp(m: "_lib.Mlp", weights: Sequence[torch.Tensor], biases: Sequence[torch.Tensor]) -> None:

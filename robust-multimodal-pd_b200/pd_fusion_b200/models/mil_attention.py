@@ -52,6 +52,19 @@ def _pad_bags(bags):
     return X, M
 
 
+def _fill_explanation(out: dict, rows: List[int], lens: np.ndarray, logit: torch.Tensor, attn: torch.Tensor, contrib: torch.Tensor):
+    """Copies a MilHead.explain result of the bags `rows` (in that order, lengths `lens`) into the per-bag lists / arrays of `out`.
+    prob = sigmoid(logit) on the device in float32, the pooling kernel's own last step."""
+    prob = torch.sigmoid(logit).cpu().numpy()
+    logit, attn, contrib = logit.cpu().numpy(), attn.cpu().numpy(), contrib.cpu().numpy()
+    for j, i in enumerate(rows):
+        L = int(lens[j])
+        out["prob"][i] = float(prob[j])
+        out["logit"][i] = float(logit[j])
+        out["attention"][i] = attn[j, :L].copy()
+        out["contribution"][i] = contrib[j, :L].copy()
+
+
 class MilAttentionModel(BaseModel):
     def __init__(self, input_dim: int, params: dict):
         self.params = params or {}
@@ -161,6 +174,24 @@ class MilAttentionModel(BaseModel):
             return out
         head, X, lens = self._upload(bags, live)
         out[live] = head.forward(X, lens).cpu().numpy().astype(np.float64)
+        return out
+
+    def explain(self, bags: List[Optional[np.ndarray]], masks=None) -> dict:
+        """Why each bag got its probability (bag and mask semantics of `predict_proba`), one pdf_mil_explain over the live bags:
+        {"prob": [N] float64 (as predict_proba; missing_prob for absent bags), "logit": [N] float64 (NaN where absent),
+         "attention": [a_l] and "contribution": [a_l * (w_cls . h_l)] per bag as np.ndarray [L_i] (None where absent)}.
+        The contributions of a bag add up to logit - classifier bias.  Explanations always use the FP32 head arithmetic: for a
+        "tf32" model, prob and logit are those of the same weights under "fp32"."""
+        mri = masks["mri"] if isinstance(masks, dict) and "mri" in masks else None
+        n = len(bags)
+        live = [i for i, b in enumerate(bags) if b is not None and not (mri is not None and mri[i] == 0)]
+        out = {"prob": np.full(n, self.missing_prob, dtype=np.float64), "logit": np.full(n, np.nan, dtype=np.float64),
+               "attention": [None] * n, "contribution": [None] * n}
+        if not live:
+            return out
+        head, X, lens = self._upload(bags, live)
+        logit, attn, contrib, _ = head.explain(X, lens)
+        _fill_explanation(out, live, lens.cpu().numpy(), logit, attn, contrib)
         return out
 
     def predict_proba_sweep(self, bags: List[Optional[np.ndarray]], mri_masks: Optional[np.ndarray]) -> np.ndarray:

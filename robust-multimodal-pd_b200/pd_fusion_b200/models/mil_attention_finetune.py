@@ -16,7 +16,7 @@ from __future__ import annotations
 
 import os
 from pathlib import Path
-from typing import Dict, List, Optional, Sequence
+from typing import Callable, Dict, List, Optional, Sequence
 
 import numpy as np
 import torch
@@ -26,15 +26,24 @@ from .. import _lib
 from ..backbone import ResNetEncoder
 from ..data import openneuro_features as onf
 from ..data.tta import TtaDraw, affine_matrix, params_bytes
-from ..heads import MilHead
+from ..heads import MilHead, gradcam
 from ..preprocess import VolumePreprocessor
 from ..utils.torch_utils import get_torch_device
 from .base import BaseModel
-from .mil_attention import MILAttentionNet
+from .mil_attention import MILAttentionNet, _fill_explanation
 
 
 def _is_path(bag) -> bool:
     return isinstance(bag, (str, os.PathLike))
+
+
+def _pad_embeddings(embs: Sequence[torch.Tensor], dim: int, device):
+    """Per-bag slice embeddings [L_i, D] -> zero-padded bags [n, Lmax, D] f32 and lengths [n] i32 on the device."""
+    lmax = max(int(e.shape[0]) for e in embs)
+    X = torch.zeros((len(embs), lmax, dim), dtype=torch.float32, device=device)
+    for j, e in enumerate(embs):
+        X[j, : e.shape[0]] = e
+    return X, torch.tensor([int(e.shape[0]) for e in embs], dtype=torch.int32, device=device)
 
 
 class MilAttentionFineTuneModel(BaseModel):
@@ -162,9 +171,11 @@ class MilAttentionFineTuneModel(BaseModel):
         cap = int(os.environ.get("PD_FUSION_B200_FT_IMAGES", "0")) or max(256, self.bag_batch_size * int(sum(self.counts)))
         return max(cap, int(longest))
 
-    def _embed_slices(self, stacks: Sequence[torch.Tensor]) -> List[torch.Tensor]:
+    def _embed_slices(self, stacks: Sequence[torch.Tensor], on_pass: Optional[Callable] = None) -> List[torch.Tensor]:
         """Per-slice embeddings of ready slice stacks ([L_i, H, W] f32 CUDA tensors in [0,1]): the bags go through ONE
-        fixed-capacity encoder in groups of whole bags, the unused tail of the input buffer zeroed (as EmbeddingPipeline.embed does)."""
+        fixed-capacity encoder in groups of whole bags, the unused tail of the input buffer zeroed (as EmbeddingPipeline.embed does).
+        on_pass(enc, first, embs), if given, runs after each encoder pass, while the pass's feature map is still in the encoder:
+        bags [first, first + len(embs)) went through it, their rows in order from 0."""
         cap = self._capacity(max(int(s.shape[0]) for s in stacks))
         enc = self._encoder(cap)
         H, W = int(stacks[0].shape[1]), int(stacks[0].shape[2])
@@ -186,6 +197,8 @@ class MilAttentionFineTuneModel(BaseModel):
             for s in stacks[i:j]:
                 out.append(emb[k:k + int(s.shape[0])])
                 k += int(s.shape[0])
+            if on_pass is not None:
+                on_pass(enc, i, out[i:j])
             i = j
         return out
 
@@ -222,14 +235,51 @@ class MilAttentionFineTuneModel(BaseModel):
             # the augmentation, mil_attention_finetune.py:114-125)
             cur = [self._augment(s, rng) if (self.tta_inference > 1 and self.train_aug and not isinstance(bags[i], np.ndarray)) else s
                    for s, i in zip(stacks, live)]
-            embs = self._embed_slices(cur)
-            lmax = max(int(e.shape[0]) for e in embs)
-            X = torch.zeros((len(embs), lmax, self.emb_dim), dtype=torch.float32, device=self.device)
-            lens = torch.tensor([int(e.shape[0]) for e in embs], dtype=torch.int32, device=self.device)
-            for j, e in enumerate(embs):
-                X[j, : e.shape[0]] = e
+            X, lens = _pad_embeddings(self._embed_slices(cur), self.emb_dim, self.device)
             acc += head.forward(X, lens)
         out[live] = (acc / passes).cpu().numpy().astype(np.float64)
+        return out
+
+    def explain(self, bags, masks=None) -> dict:
+        """Why each bag got its probability (bag and mask semantics of `predict_proba`):
+        {"prob": [N] float64 (predict_proba's with tta_inference = 1; missing_prob for absent bags), "logit": [N] float64 (NaN where
+         absent), and per bag (None where absent): "attention" / "contribution" np.ndarray [L_i] (attention weights a_l and
+         a_l * (w_cls . h_l), which add up to logit - classifier bias), "slices" [L_i, H, W] (the stack `_bag_slices` returns) and
+         "cam" [L_i, H, W]: the Grad-CAM map of the logit at the backbone's last stage, upsampled to the slice grid, unnormalised
+         (a ReLU output)}.
+        Explanations use no test-time augmentation, whatever tta_inference says, and the FP32 head arithmetic.  They run pass by
+        pass inside the encoder's whole-bag grouping: after each pass, while its last feature map is live, the head's explanation
+        (with the gradient of the logit with respect to every slice embedding) and pdf_gradcam of that pass's slices."""
+        mri = masks["mri"] if isinstance(masks, dict) and "mri" in masks else None
+        n = len(bags)
+        out = {"prob": np.full(n, self.missing_prob, dtype=np.float64), "logit": np.full(n, np.nan, dtype=np.float64),
+               "attention": [None] * n, "contribution": [None] * n, "slices": [None] * n, "cam": [None] * n}
+        live = [i for i, b in enumerate(bags) if b is not None and not (mri is not None and mri[i] == 0)]
+        if not live:
+            return out
+        self.backbone.eval()
+        self.attn.eval()
+        stacks = self._device_stacks([bags[i] for i in live])
+        head = self._head()
+        H, W = int(stacks[0].shape[1]), int(stacks[0].shape[2])
+
+        def explain_pass(enc, first, embs):
+            rows = live[first:first + len(embs)]
+            X, lens = _pad_embeddings(embs, self.emb_dim, self.device)
+            logit, attn, contrib, dX = head.explain(X, lens, need_grad=True)
+            g = torch.cat([dX[j, : e.shape[0]] for j, e in enumerate(embs)], dim=0)
+            cam, _ = gradcam(enc.feature_map()[: g.shape[0]], g, (H, W))
+            lens_h = lens.cpu().numpy()
+            _fill_explanation(out, rows, lens_h, logit, attn, contrib)
+            cam = cam.cpu().numpy()
+            k = 0
+            for j, i in enumerate(rows):
+                L = int(lens_h[j])
+                out["cam"][i] = cam[k:k + L]
+                out["slices"][i] = stacks[first + j].cpu().numpy()
+                k += L
+
+        self._embed_slices(stacks, on_pass=explain_pass)
         return out
 
     # ------------------------------------------------------------------------------------------ training (native kernels)
