@@ -482,6 +482,31 @@ typedef struct {
 int pdf_moe_sweep(const pdf_moe* net, int n_subjects, int n_scenarios, const float* const* d_x /* host array of device ptrs */,
                   const uint8_t* d_masks, float* d_prob, pdf_stream_t stream);
 
+/* Explanations of the fusion heads (csrc/fusion_explain.cu): exact modality Shapley values and integrated gradients, for every
+ * (scenario, subject) pair of the sweep's inputs.  A missing modality is a zeroed one, so the all-zero input is the baseline.  Modality
+ * (expert) m is bit m of a coalition, in the sweep's order (sorted(modality)).  The value v of a coalition is the logit (the value before
+ * net's final sigmoid) for ModDrop and the output probability for MoE; the sweep kernel evaluates all 2^M coalitions once per subject.
+ *   d_value [S,N] = v(P), P = the modalities present under scenario s: for ModDrop the logit of pdf_moddrop_sweep's probability (same
+ *     kernel, same arithmetic), for MoE pdf_moe_sweep's probability bit for bit;
+ *   d_base [1] = v(empty set), the same for every subject;
+ *   d_shap [S,N,M] = phi_m = sum over T subset P\{m} of |T|!(|P|-|T|-1)!/|P|! (v(T+m) - v(T)), summed in float64, so that
+ *     sum_m phi_m = value - base.  An absent or zero-width modality gets exactly 0;
+ *   integrated gradients from 0 with `steps` midpoints alpha_k = (k + 1/2)/steps (1..256; 0 only with d_ig NULL):
+ *     ModDrop d_ig [S,N,F] = (x (.) m_s) (.) mean_k d logit / d x at alpha_k (x (.) m_s);
+ *     MoE d_ig[e] [S,N,d_e] (host array of E device pointers) = the same for the probability: (x_e m_e) (.) w_e(m_s) (.)
+ *       mean_k d sigmoid(z_e) / d x_e at alpha_k x_e, w_e = the router weight; 0 where expert e is absent.
+ * Two calls return bit-identical results (no atomics).  The IG kernel keeps every hidden layer's activations of 64, 32 or 16 rows in
+ * shared memory; a net whose hidden widths do not fit 227 KB even at 16 rows is refused (PDF_ERR_ARG), as are bad arguments, before
+ * any device work.  Workspace: pdf_moddrop_explain_workspace_bytes / pdf_moe_explain_workspace_bytes. */
+size_t pdf_moddrop_explain_workspace_bytes(const pdf_mlp* net, int n_subjects, int n_scenarios, int steps);
+int pdf_moddrop_explain(const pdf_mlp* net, int n_subjects, int n_scenarios, const float* d_x, const uint8_t* d_masks, int steps,
+                        void* d_workspace, float* d_value /* [S,N] logit */, float* d_base /* [1] */, float* d_shap /* [S,N,M] */,
+                        float* d_ig /* [S,N,F] or NULL */, pdf_stream_t stream);
+size_t pdf_moe_explain_workspace_bytes(const pdf_moe* net, int n_subjects, int n_scenarios, int steps);
+int pdf_moe_explain(const pdf_moe* net, int n_subjects, int n_scenarios, const float* const* d_x, const uint8_t* d_masks, int steps,
+                    void* d_workspace, float* d_value /* [S,N] prob */, float* d_base /* [1] */, float* d_shap /* [S,N,E] */,
+                    float* const* d_ig /* host array of E device ptrs [S,N,d_e], or NULL */, pdf_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * Self-tests of the tensor-core building blocks (used by tests/ and smoke on the GPU box).
  * pdf_selftest_umma: C[M,N] = A[M,K] * B[N,K]^T through TMA(2D tiled) + tcgen05.mma, bf16 in / f32 out.

@@ -202,6 +202,9 @@ __device__ __forceinline__ void warp_dense(const float* __restrict__ W, const fl
 constexpr int kMaxWidth = 1024;
 
 // partials: [n_mods][N][h1] (layer-1 pre-activations per modality, no bias)
+// kCoalitions: "scenario" s is the coalition bit set (mask_m = (s >> m) & 1, S = 2^M) and `masks` is not read; kLogit: the output is
+// the last layer's value (the logit) instead of its sigmoid.  The explanations (fusion_explain.cu) evaluate every coalition this way.
+template <bool kCoalitions, bool kLogit>
 __global__ void __launch_bounds__(256)
 moddrop_sweep_kernel(pdf_mlp net, const float* __restrict__ partials, const uint8_t* __restrict__ masks, int N, int S,
                      float* __restrict__ prob) {
@@ -217,12 +220,12 @@ moddrop_sweep_kernel(pdf_mlp net, const float* __restrict__ partials, const uint
   for (long long pair = (long long)blockIdx.x * 8 + warp; pair < (long long)N * S; pair += (long long)gridDim.x * 8) {
     {
       const int s = (int)(pair / N), n = (int)(pair - (long long)s * N);
-      const uint8_t* mk = masks + ((size_t)s * N + n) * M;
+      const uint8_t* mk = kCoalitions ? nullptr : masks + ((size_t)s * N + n) * M;
       const bool last0 = net.n_layers == 1;
       for (int i = lane; i < h1; i += 32) {
         float v = 0.f;
         for (int m = 0; m < M; ++m)
-          if (mk[m] && net.mod_off[m + 1] > net.mod_off[m]) v += partials[((size_t)m * N + n) * h1 + i];
+          if ((kCoalitions ? ((s >> m) & 1) != 0 : mk[m]) && net.mod_off[m + 1] > net.mod_off[m]) v += partials[((size_t)m * N + n) * h1 + i];
         v += __ldg(net.b[0] + i);
         bufA[i] = last0 ? v : fmaxf(v, 0.f);
       }
@@ -233,7 +236,7 @@ moddrop_sweep_kernel(pdf_mlp net, const float* __restrict__ partials, const uint
         warp_dense(net.w[l], net.b[l], net.dims[l], net.dims[l + 1], in, out, l < net.n_layers - 1, lane);
         float* t = in; in = out; out = t;
       }
-      if (lane == 0) prob[(size_t)s * N + n] = sigmoidf_(in[0]);
+      if (lane == 0) prob[(size_t)s * N + n] = kLogit ? in[0] : sigmoidf_(in[0]);
       __syncwarp();
     }
   }
@@ -242,7 +245,7 @@ moddrop_sweep_kernel(pdf_mlp net, const float* __restrict__ partials, const uint
 // Large S*N: a block takes a tile of TP (scenario, subject) pairs and runs layers 2.. as shared-memory-tiled FFMA GEMMs, so every
 // weight element is fetched once per TILE instead of once per pair (the warp-per-pair kernel above re-reads 164 KB of weights per pair
 // at the C2 widths: 1.1 TB of L2 traffic at N = 1e6, S = 7).  Same arithmetic, summation over k in ascending order per output.
-template <int TP>
+template <int TP, bool kCoalitions, bool kLogit>
 __global__ void __launch_bounds__(256)
 moddrop_tile_kernel(pdf_mlp net, const float* __restrict__ partials, const uint8_t* __restrict__ masks, int N, int S, int maxw,
                     float* __restrict__ prob) {
@@ -264,9 +267,9 @@ moddrop_tile_kernel(pdf_mlp net, const float* __restrict__ partials, const uint8
       float v = 0.f;
       if (pair < total) {
         const int s = (int)(pair / N), n = (int)(pair - (long long)s * N);
-        const uint8_t* mk = masks + ((size_t)s * N + n) * M;
+        const uint8_t* mk = kCoalitions ? nullptr : masks + ((size_t)s * N + n) * M;
         for (int m = 0; m < M; ++m)
-          if (mk[m] && net.mod_off[m + 1] > net.mod_off[m]) v += partials[((size_t)m * N + n) * h1 + i];
+          if ((kCoalitions ? ((s >> m) & 1) != 0 : mk[m]) && net.mod_off[m + 1] > net.mod_off[m]) v += partials[((size_t)m * N + n) * h1 + i];
         v += __ldg(net.b[0] + i);
         if (net.n_layers > 1) v = fmaxf(v, 0.f);
       }
@@ -322,7 +325,7 @@ moddrop_tile_kernel(pdf_mlp net, const float* __restrict__ partials, const uint8
       float* t = in; in = out; out = t;
     }
     for (int r = tid; r < TP; r += 256)
-      if (p0 + r < total) prob[p0 + r] = sigmoidf_(in[r * stride]);       // prob is [S, N] = pair order
+      if (p0 + r < total) prob[p0 + r] = kLogit ? in[r * stride] : sigmoidf_(in[r * stride]);       // prob is [S, N] = pair order
     __syncthreads();
   }
 }
@@ -332,8 +335,12 @@ struct MoeArgs {
   const float* x[PDF_MAX_MODS];
 };
 
+// kCoalitions: as moddrop_sweep_kernel (S = 2^E, `masks` not read); the warps of subject 0 also write the router weights of every
+// coalition to router_w [2^E, E].  The output is the gated sum itself either way: MoE has no single logit.
+template <bool kCoalitions>
 __global__ void __launch_bounds__(256)
-moe_sweep_kernel(MoeArgs a, const uint8_t* __restrict__ masks, int N, int S, int maxw, float* __restrict__ prob) {
+moe_sweep_kernel(MoeArgs a, const uint8_t* __restrict__ masks, int N, int S, int maxw, float* __restrict__ prob,
+                 float* __restrict__ router_w) {
   extern __shared__ float sm[];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   float* bufA = sm + (size_t)warp * 2 * maxw;
@@ -371,11 +378,11 @@ moe_sweep_kernel(MoeArgs a, const uint8_t* __restrict__ masks, int N, int S, int
       __syncwarp();
     }
     for (int s = 0; s < S; ++s) {
-      const uint8_t* mk = masks + ((size_t)s * N + n) * E;
+      const uint8_t* mk = kCoalitions ? nullptr : masks + ((size_t)s * N + n) * E;
       // router: softmax(W1 relu(W0 mask + b0) + b1)
       for (int h = lane; h < R; h += 32) {
         float v = __ldg(a.net.b_r0 + h);
-        for (int m = 0; m < E; ++m) v = fmaf(__ldg(a.net.w_r0 + h * E + m), mk[m] ? 1.f : 0.f, v);
+        for (int m = 0; m < E; ++m) v = fmaf(__ldg(a.net.w_r0 + h * E + m), (kCoalitions ? ((s >> m) & 1) != 0 : mk[m]) ? 1.f : 0.f, v);
         bufA[h] = fmaxf(v, 0.f);
       }
       __syncwarp();
@@ -391,8 +398,10 @@ moe_sweep_kernel(MoeArgs a, const uint8_t* __restrict__ masks, int N, int S, int
       float se = 0.f;
       for (int m = 0; m < E; ++m) { logit[m] = expf(logit[m] - mx); se += logit[m]; }
       float o = 0.f;
-      for (int m = 0; m < E; ++m) o += (mk[m] ? e_x[m] : e_0[m]) * (logit[m] / se);
+      for (int m = 0; m < E; ++m) o += ((kCoalitions ? ((s >> m) & 1) != 0 : mk[m]) ? e_x[m] : e_0[m]) * (logit[m] / se);
       if (lane == 0) prob[(size_t)s * N + n] = o;
+      if (kCoalitions && n == 0 && lane == 0)
+        for (int m = 0; m < E; ++m) router_w[(size_t)s * E + m] = logit[m] / se;
       __syncwarp();
     }
   }
@@ -400,13 +409,106 @@ moe_sweep_kernel(MoeArgs a, const uint8_t* __restrict__ masks, int N, int S, int
 
 static bool g_moddrop_tiled = true;   // pdf_debug_set_moddrop_tiled
 
-static int check_mlp(const pdf_mlp& m, const char* what) {
+int check_mlp(const pdf_mlp& m, const char* what) {
   PDF_REQUIRE(m.n_layers >= 1 && m.n_layers <= PDF_MAX_LAYERS, "%s: n_layers out of range", what);
   PDF_REQUIRE(m.dims[m.n_layers] == 1, "%s: last layer must have one output", what);
   for (int l = 0; l < m.n_layers; ++l) {
     PDF_REQUIRE(m.w[l] && m.b[l] && m.dims[l] >= 0, "%s: null weights in layer %d", what, l);
     if (l > 0) PDF_REQUIRE(m.dims[l] >= 1 && m.dims[l] <= kMaxWidth, "%s: hidden width must be 1..%d", what, kMaxWidth);
   }
+  return PDF_OK;
+}
+
+int check_moddrop(const pdf_mlp& net, const char* what) {
+  if (int rc = check_mlp(net, what)) return rc;
+  PDF_REQUIRE(net.n_mods >= 1 && net.n_mods <= PDF_MAX_MODS && net.mod_off[0] == 0 && net.mod_off[net.n_mods] == net.dims[0],
+              "%s: modality offsets must tile [0, F)", what);
+  PDF_REQUIRE(net.dims[1] <= kMaxWidth, "%s: first hidden width must be <= %d", what, kMaxWidth);
+  return PDF_OK;
+}
+
+int check_moe(const pdf_moe& net, const float* const* d_x, const char* what) {
+  PDF_REQUIRE(net.n_experts >= 1 && net.n_experts <= PDF_MAX_MODS && net.router_hidden >= 1 && net.router_hidden <= kMaxWidth &&
+              net.w_r0 && net.b_r0 && net.w_r1 && net.b_r1, "%s: bad router", what);
+  int maxw = net.router_hidden;
+  for (int e = 0; e < net.n_experts; ++e) {
+    if (int rc = check_mlp(net.expert[e], what)) return rc;
+    PDF_REQUIRE(d_x[e] && net.expert[e].dims[0] >= 1 && net.expert[e].dims[0] <= 8192, "%s: expert input width 1..8192", what);
+    for (int l = 0; l <= net.expert[e].n_layers; ++l) maxw = max(maxw, net.expert[e].dims[l]);
+  }
+  PDF_REQUIRE((size_t)8 * 2 * maxw * sizeof(float) <= 200 * 1024, "%s: layers too wide for shared memory", what);
+  return PDF_OK;
+}
+
+int moddrop_partials(const pdf_mlp& net, int N, const float* d_x, float* partials, cudaStream_t s) {
+  const int F = net.dims[0], h1 = net.dims[1];
+  // linearity of layer 1: (x (.) mask) W1^T = sum_m mask_m * (x_m W1_m^T)  -> per-modality partials once, reused by every scenario
+  for (int m = 0; m < net.n_mods; ++m) {
+    const int d = net.mod_off[m + 1] - net.mod_off[m];
+    if (d <= 0) continue;
+    if (int rc = gemm_nt(d_x + net.mod_off[m], F, net.w[0] + net.mod_off[m], F, partials + (size_t)m * N * h1, h1, nullptr, N, h1, d, 0, s))
+      return rc;
+  }
+  return PDF_OK;
+}
+
+template <bool kCoalitions, bool kLogit>
+static int moddrop_launch(const pdf_mlp& net, int N, int S, const float* partials, const uint8_t* masks, long long sweep_pairs,
+                          float* out, cudaStream_t s) {
+  const int h1 = net.dims[1];
+  int maxw = h1;
+  for (int l = 2; l <= net.n_layers; ++l) maxw = max(maxw, net.dims[l]);
+  const size_t smem = (size_t)8 * 2 * maxw * sizeof(float);
+  if (smem > 48 * 1024)
+    PDF_CHECK_CUDA(cudaFuncSetAttribute(moddrop_sweep_kernel<kCoalitions, kLogit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const long long pairs = (long long)N * S;
+  if (g_moddrop_tiled && sweep_pairs >= 4096 && net.n_layers >= 2) {
+    // batched path: tiles of 64 (32 for wide networks) pairs, layers 2.. as in-block GEMMs
+    const int TP = maxw <= 384 ? 64 : 32;
+    const size_t tsmem = ((size_t)2 * TP * (maxw + 1) + 16 * 68) * sizeof(float);
+    if (tsmem <= 200 * 1024) {
+      const int tblocks = (int)max(1LL, min((pairs + TP - 1) / TP, (long long)num_sms() * (tsmem > 100 * 1024 ? 1 : 2)));
+      if (TP == 64) {
+        PDF_CHECK_CUDA(cudaFuncSetAttribute(moddrop_tile_kernel<64, kCoalitions, kLogit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsmem));
+        moddrop_tile_kernel<64, kCoalitions, kLogit><<<tblocks, 256, tsmem, s>>>(net, partials, masks, N, S, maxw, out);
+      } else {
+        PDF_CHECK_CUDA(cudaFuncSetAttribute(moddrop_tile_kernel<32, kCoalitions, kLogit>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsmem));
+        moddrop_tile_kernel<32, kCoalitions, kLogit><<<tblocks, 256, tsmem, s>>>(net, partials, masks, N, S, maxw, out);
+      }
+      PDF_CHECK_LAUNCH();
+      return PDF_OK;
+    }
+  }
+  const int blocks = max(1, min(ceil_div(pairs, 8), num_sms() * 8));
+  moddrop_sweep_kernel<kCoalitions, kLogit><<<blocks, 256, smem, s>>>(net, partials, masks, N, S, out);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+int moddrop_eval(const pdf_mlp& net, int N, int S, const float* partials, const uint8_t* masks, bool coalitions, long long sweep_pairs,
+                 float* out, cudaStream_t s) {
+  return coalitions ? moddrop_launch<true, true>(net, N, 1 << net.n_mods, partials, nullptr, sweep_pairs, out, s)
+                    : moddrop_launch<false, false>(net, N, S, partials, masks, sweep_pairs, out, s);
+}
+
+int moe_eval(const pdf_moe& net, const float* const* d_x, int N, int S, const uint8_t* masks, float* router_w, float* out, cudaStream_t s) {
+  MoeArgs a;
+  a.net = net;
+  int maxw = net.router_hidden;
+  for (int e = 0; e < net.n_experts; ++e) {
+    a.x[e] = d_x[e];
+    for (int l = 0; l <= net.expert[e].n_layers; ++l) maxw = max(maxw, net.expert[e].dims[l]);
+  }
+  const size_t smem = (size_t)8 * 2 * maxw * sizeof(float);
+  const int blocks = max(1, min(ceil_div(N, 8), num_sms() * 8));
+  if (router_w) {
+    if (smem > 48 * 1024) PDF_CHECK_CUDA(cudaFuncSetAttribute(moe_sweep_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    moe_sweep_kernel<true><<<blocks, 256, smem, s>>>(a, nullptr, N, 1 << net.n_experts, maxw, out, router_w);
+  } else {
+    if (smem > 48 * 1024) PDF_CHECK_CUDA(cudaFuncSetAttribute(moe_sweep_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    moe_sweep_kernel<false><<<blocks, 256, smem, s>>>(a, masks, N, S, maxw, out, nullptr);
+  }
+  PDF_CHECK_LAUNCH();
   return PDF_OK;
 }
 
@@ -476,70 +578,18 @@ extern "C" size_t pdf_moddrop_workspace_bytes(const pdf_mlp* net, int n_subjects
 extern "C" int pdf_moddrop_sweep(const pdf_mlp* net, int n_subjects, int n_scenarios, const float* d_x, const uint8_t* d_masks,
                                  void* d_workspace, float* d_prob, pdf_stream_t stream) {
   PDF_REQUIRE(net && n_subjects > 0 && n_scenarios > 0 && d_x && d_masks && d_workspace && d_prob, "pdf_moddrop_sweep: bad arguments");
-  if (int rc = check_mlp(*net, "pdf_moddrop_sweep")) return rc;
-  PDF_REQUIRE(net->n_mods >= 1 && net->n_mods <= PDF_MAX_MODS && net->mod_off[0] == 0 && net->mod_off[net->n_mods] == net->dims[0],
-              "pdf_moddrop_sweep: modality offsets must tile [0, F)");
-  PDF_REQUIRE(net->dims[1] <= kMaxWidth, "pdf_moddrop_sweep: first hidden width must be <= %d", kMaxWidth);
+  if (int rc = check_moddrop(*net, "pdf_moddrop_sweep")) return rc;
   cudaStream_t s = as_stream(stream);
-  const int F = net->dims[0], h1 = net->dims[1];
   float* partials = reinterpret_cast<float*>(d_workspace);
-  // linearity of layer 1: (x (.) mask) W1^T = sum_m mask_m * (x_m W1_m^T)  -> per-modality partials once, reused by every scenario
-  for (int m = 0; m < net->n_mods; ++m) {
-    const int d = net->mod_off[m + 1] - net->mod_off[m];
-    if (d <= 0) continue;
-    if (int rc = gemm_nt(d_x + net->mod_off[m], F, net->w[0] + net->mod_off[m], F, partials + (size_t)m * n_subjects * h1, h1,
-                         nullptr, n_subjects, h1, d, 0, s))
-      return rc;
-  }
-  int maxw = h1;
-  for (int l = 2; l <= net->n_layers; ++l) maxw = max(maxw, net->dims[l]);
-  const size_t smem = (size_t)8 * 2 * maxw * sizeof(float);
-  if (smem > 48 * 1024) PDF_CHECK_CUDA(cudaFuncSetAttribute(moddrop_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const long long pairs = (long long)n_subjects * n_scenarios;
-  if (g_moddrop_tiled && pairs >= 4096 && net->n_layers >= 2) {
-    // batched path: tiles of 64 (32 for wide networks) pairs, layers 2.. as in-block GEMMs
-    const int TP = maxw <= 384 ? 64 : 32;
-    const size_t tsmem = ((size_t)2 * TP * (maxw + 1) + 16 * 68) * sizeof(float);
-    if (tsmem <= 200 * 1024) {
-      const int tblocks = (int)max(1LL, min((pairs + TP - 1) / TP, (long long)num_sms() * (tsmem > 100 * 1024 ? 1 : 2)));
-      if (TP == 64) {
-        PDF_CHECK_CUDA(cudaFuncSetAttribute(moddrop_tile_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsmem));
-        moddrop_tile_kernel<64><<<tblocks, 256, tsmem, s>>>(*net, partials, d_masks, n_subjects, n_scenarios, maxw, d_prob);
-      } else {
-        PDF_CHECK_CUDA(cudaFuncSetAttribute(moddrop_tile_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tsmem));
-        moddrop_tile_kernel<32><<<tblocks, 256, tsmem, s>>>(*net, partials, d_masks, n_subjects, n_scenarios, maxw, d_prob);
-      }
-      PDF_CHECK_LAUNCH();
-      return PDF_OK;
-    }
-  }
-  const int blocks = max(1, min(ceil_div(pairs, 8), num_sms() * 8));
-  moddrop_sweep_kernel<<<blocks, 256, smem, s>>>(*net, partials, d_masks, n_subjects, n_scenarios, d_prob);
-  PDF_CHECK_LAUNCH();
-  return PDF_OK;
+  if (int rc = moddrop_partials(*net, n_subjects, d_x, partials, s)) return rc;
+  return moddrop_eval(*net, n_subjects, n_scenarios, partials, d_masks, false, (long long)n_subjects * n_scenarios, d_prob, s);
 }
 
 extern "C" int pdf_moe_sweep(const pdf_moe* net, int n_subjects, int n_scenarios, const float* const* d_x, const uint8_t* d_masks,
                              float* d_prob, pdf_stream_t stream) {
   PDF_REQUIRE(net && n_subjects > 0 && n_scenarios > 0 && d_x && d_masks && d_prob, "pdf_moe_sweep: bad arguments");
-  PDF_REQUIRE(net->n_experts >= 1 && net->n_experts <= PDF_MAX_MODS && net->router_hidden >= 1 && net->router_hidden <= kMaxWidth &&
-              net->w_r0 && net->b_r0 && net->w_r1 && net->b_r1, "pdf_moe_sweep: bad router");
-  MoeArgs a;
-  a.net = *net;
-  int maxw = net->router_hidden;
-  for (int e = 0; e < net->n_experts; ++e) {
-    if (int rc = check_mlp(net->expert[e], "pdf_moe_sweep expert")) return rc;
-    PDF_REQUIRE(d_x[e] && net->expert[e].dims[0] >= 1 && net->expert[e].dims[0] <= 8192, "pdf_moe_sweep: expert input width 1..8192");
-    a.x[e] = d_x[e];
-    for (int l = 0; l <= net->expert[e].n_layers; ++l) maxw = max(maxw, net->expert[e].dims[l]);
-  }
-  const size_t smem = (size_t)8 * 2 * maxw * sizeof(float);
-  PDF_REQUIRE(smem <= 200 * 1024, "pdf_moe_sweep: layers too wide for shared memory");
-  if (smem > 48 * 1024) PDF_CHECK_CUDA(cudaFuncSetAttribute(moe_sweep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int blocks = max(1, min(ceil_div(n_subjects, 8), num_sms() * 8));
-  moe_sweep_kernel<<<blocks, 256, smem, as_stream(stream)>>>(a, d_masks, n_subjects, n_scenarios, maxw, d_prob);
-  PDF_CHECK_LAUNCH();
-  return PDF_OK;
+  if (int rc = check_moe(*net, d_x, "pdf_moe_sweep")) return rc;
+  return moe_eval(*net, d_x, n_subjects, n_scenarios, d_masks, nullptr, d_prob, as_stream(stream));
 }
 
 /* A/B hook: 0 = the warp-per-pair ModDrop kernel for every size, 1 (default) = the tiled GEMM kernel from 4096 (scenario, subject) pairs up */

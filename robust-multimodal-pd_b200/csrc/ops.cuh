@@ -68,6 +68,19 @@ int launch_gemm_tf32(const float* A, const float* B, int M, int N, int K, int mo
 // that explanations see the same h and attention pre-activations as pdf_mil_sweep's FP32 path
 int gemm_nt(const float* A, int lda, const float* B, int ldb, float* C, int ldc, const float* bias, int M, int N, int K, int relu,
             cudaStream_t s);
+// Fusion heads (heads.cu), shared with their explanations (fusion_explain.cu).  check_*: the sweeps' argument checks.
+// moddrop_partials: partials[m] = x_m W1_m^T [N, h1] per modality of nonzero width (layer 1 without bias).
+// moddrop_eval: layers 2.. under S scenario masks -> prob [S, N]; coalitions = true: under all 2^M coalitions (mask_m = (c >> m) & 1,
+// masks not read) -> logit [2^M, N].  The kernel (tiled or warp per pair) is the one pdf_moddrop_sweep picks for sweep_pairs pairs.
+// moe_eval: router, experts and gated sum under S scenario masks -> [S, N]; router_w != NULL: under all 2^E coalitions instead, and
+// router_w [2^E, E] receives the router weights of every coalition.
+int check_mlp(const pdf_mlp& m, const char* what);
+int check_moddrop(const pdf_mlp& net, const char* what);
+int check_moe(const pdf_moe& net, const float* const* d_x, const char* what);
+int moddrop_partials(const pdf_mlp& net, int N, const float* d_x, float* partials, cudaStream_t s);
+int moddrop_eval(const pdf_mlp& net, int N, int S, const float* partials, const uint8_t* masks, bool coalitions, long long sweep_pairs,
+                 float* out, cudaStream_t s);
+int moe_eval(const pdf_moe& net, const float* const* d_x, int N, int S, const uint8_t* masks, float* router_w, float* out, cudaStream_t s);
 bool pw_eligible(const pdf_op& op);
 int prepare_conv_pw(const pdf_op& op, TcConv* tc);
 int launch_conv_pw(const TcConv& tc, cudaStream_t s);

@@ -6,6 +6,7 @@ reference's RNG order), uploaded once as uint8 [S, N, M], and the model is evalu
 launch; tabular preprocessing runs once instead of once per scenario (evaluate.py:58,67).
 Models that do not expose a sweep entry point (e.g. a CalibratedModel wrapper) fall back to the reference's
 per-scenario `predict_proba` calls -- each of which still runs on the device.
+`explain_model` explains a fusion head's predictions under the same scenario masks.
 """
 from __future__ import annotations
 
@@ -27,6 +28,24 @@ def _kind(prep_info) -> str:
     return "moe" if isinstance(prep_info, dict) else "matrix"
 
 
+def _fusion_inputs(df_test, mask_test, prep_info, scenarios: List[Dict]):
+    """Preprocessed features (unmasked), uint8 scenario masks [S, N, M], the per-scenario mask dicts (drawn in scenario order) and
+    the mask column order, for the "moe" and "matrix" kinds."""
+    if _kind(prep_info) == "moe":
+        mods = list(prep_info.keys())
+        if mods != sorted(mods):
+            # MoENet orders its experts by sorted(modality) while the reference's evaluate feeds the router in caller order
+            # (evaluation/evaluate.py:54-63): an unsorted prep_info would silently pair router outputs with the wrong experts
+            raise ValueError(f"MoE prep_info modalities must be in sorted order, got {mods}")
+        masks, per = scenario_mask_tensor(df_test, scenarios, mask_test, mods)
+        X = {m: preprocess_features(df_test, prep_info[m][2], prep_info[m][0], prep_info[m][1])[0] for m in mods}
+        return X, masks, per, mods
+    imputer, scaler, feature_cols = prep_info
+    X, _, _ = preprocess_features(df_test, feature_cols, imputer, scaler)
+    masks, per = scenario_mask_tensor(df_test, scenarios, mask_test, MODALITIES)
+    return X, masks, per, MODALITIES
+
+
 def _sweep_probs(model, df_test, mask_test, prep_info, scenarios: List[Dict]) -> Tuple[np.ndarray, List[Dict[str, np.ndarray]]]:
     """Probabilities [S, N] for all scenarios + the per-scenario mask dicts (drawn in scenario order)."""
     kind = _kind(prep_info)
@@ -45,13 +64,7 @@ def _sweep_probs(model, df_test, mask_test, prep_info, scenarios: List[Dict]) ->
             probs.append(model.predict_proba(b, masks=cur))
         return np.stack(probs), per
     if kind == "moe":
-        mods = list(prep_info.keys())
-        if mods != sorted(mods):
-            # MoENet orders its experts by sorted(modality) while the reference's evaluate feeds the router in caller order
-            # (evaluation/evaluate.py:54-63): an unsorted prep_info would silently pair router outputs with the wrong experts
-            raise ValueError(f"MoE prep_info modalities must be in sorted order, got {mods}")
-        masks, per = scenario_mask_tensor(df_test, scenarios, mask_test, mods)
-        X = {m: preprocess_features(df_test, prep_info[m][2], prep_info[m][0], prep_info[m][1])[0] for m in mods}
+        X, masks, per, mods = _fusion_inputs(df_test, mask_test, prep_info, scenarios)
         if hasattr(model, "predict_proba_sweep"):
             return model.predict_proba_sweep(X, masks, mods), per
         import torch
@@ -60,9 +73,8 @@ def _sweep_probs(model, df_test, mask_test, prep_info, scenarios: List[Dict]) ->
             Xd = {m: torch.FloatTensor(X[m] * cur[m].reshape(-1, 1) if m in cur else X[m]) for m in mods}
             probs.append(model.predict_proba(Xd, torch.FloatTensor(np.stack([cur[m] for m in mods], axis=1))))
         return np.stack(probs), per
-    imputer, scaler, feature_cols = prep_info
-    X, _, _ = preprocess_features(df_test, feature_cols, imputer, scaler)
-    masks, per = scenario_mask_tensor(df_test, scenarios, mask_test, MODALITIES)
+    feature_cols = prep_info[2]
+    X, masks, per, _ = _fusion_inputs(df_test, mask_test, prep_info, scenarios)
     if hasattr(model, "predict_proba_sweep") and not hasattr(model, "mask_dim"):
         return model.predict_proba_sweep(X, masks, MODALITIES), per
     probs = []
@@ -87,6 +99,23 @@ def evaluate_model(model, df_test, mask_test, prep_info, config) -> Dict[str, Di
     probs, _ = _sweep_probs(model, df_test, mask_test, prep_info, scenarios)
     return {sc["name"]: _with_groups(compute_metrics(y_true, np.asarray(probs[s])), df_test, y_true, np.asarray(probs[s]), group_col)
             for s, sc in enumerate(scenarios)}
+
+
+def explain_model(model, df_test, mask_test, prep_info, config, steps: int = 32) -> Dict[str, Dict]:
+    """{scenario name: explanation} of a fusion head (ModalityDropoutModel.explain / MoEModel.explain: probabilities, exact modality
+    Shapley values, integrated gradients with `steps` midpoints) under every scenario of `config`, in one explain call for all of
+    them.  The scenario masks are drawn as evaluate_model draws them (same helper, same RNG order), so with the same seed each
+    scenario's "prob" is evaluate_model's probability."""
+    if _kind(prep_info) == "mil":
+        raise ValueError("explain_model explains the fusion heads (ModDrop, MoE); explain a MIL model with MilAttentionModel.explain "
+                         "or MilAttentionFineTuneModel.explain")
+    if not hasattr(model, "explain_sweep") or hasattr(model, "mask_dim"):
+        raise ValueError(f"{type(model).__name__} has no fusion-head explanation: explain_model needs a ModalityDropoutModel or an "
+                         "MoEModel (MIL models: MilAttentionModel.explain)")
+    scenarios = config.get("scenarios", [{"name": "baseline", "drop_modalities": []}])
+    X, masks, _, order = _fusion_inputs(df_test, mask_test, prep_info, scenarios)
+    ex = model.explain_sweep(X, masks, order, steps)
+    return {sc["name"]: ex[s] for s, sc in enumerate(scenarios)}
 
 
 def predict_proba_for_scenario(model, df_test, mask_test, prep_info, scenario):

@@ -1,5 +1,6 @@
 """Host side of K3/K4: thin wrappers that marshal state_dict tensors into the C structs of
-pdf_mil_forward / pdf_mil_explain / pdf_gradcam / pdf_moddrop_sweep / pdf_moe_sweep.  No arithmetic happens here.
+pdf_mil_forward / pdf_mil_explain / pdf_gradcam / pdf_moddrop_sweep / pdf_moe_sweep / pdf_moddrop_explain / pdf_moe_explain.
+No arithmetic happens here.
 """
 from __future__ import annotations
 
@@ -176,6 +177,26 @@ class ModDropSweep:
                                               prob.data_ptr(), _lib.stream_ptr()), "pdf_moddrop_sweep")
         return prob
 
+    def explain(self, X: torch.Tensor, masks: torch.Tensor, steps: int = 0):
+        """X [N,F] f32 cuda (unmasked); masks [S,N,M] u8 cuda in self.mods order -> device tensors of pdf_moddrop_explain:
+        (logit [S,N], base logit [1], Shapley values [S,N,M] of the logit, integrated gradients [S,N,F] with `steps` midpoints or
+        None for steps = 0).  The Shapley values of a scenario add up to logit - base."""
+        N, S = int(X.shape[0]), int(masks.shape[0])
+        X = X.to(dtype=torch.float32).contiguous()
+        masks = masks.to(dtype=torch.uint8).contiguous()
+        if tuple(masks.shape) != (S, N, len(self.mods)) or X.shape[1] != int(self.net.dims[0]):
+            raise ValueError("X must be [N, F] and masks [S, N, M]")
+        need = int(self.lib.pdf_moddrop_explain_workspace_bytes(C.byref(self.net), N, S, steps))
+        ws = torch.empty(need, dtype=torch.uint8, device=X.device)
+        value = torch.empty((S, N), dtype=torch.float32, device=X.device)
+        base = torch.empty(1, dtype=torch.float32, device=X.device)
+        shap = torch.empty((S, N, len(self.mods)), dtype=torch.float32, device=X.device)
+        ig = torch.empty((S, N, X.shape[1]), dtype=torch.float32, device=X.device) if steps > 0 else None
+        _lib.check(self.lib.pdf_moddrop_explain(C.byref(self.net), N, S, X.data_ptr(), masks.data_ptr(), steps, ws.data_ptr(),
+                                                value.data_ptr(), base.data_ptr(), shap.data_ptr(), _lib.ptr(ig), _lib.stream_ptr()),
+                   "pdf_moddrop_explain")
+        return value, base, shap, ig
+
 
 class MoeSweep:
     """MoENet (models/moe.py:23-47) evaluated under S scenario masks at once; experts in sorted(modality) order."""
@@ -212,3 +233,25 @@ class MoeSweep:
         _lib.check(self.lib.pdf_moe_sweep(C.byref(self.net), N, S, ptrs, masks.data_ptr(), prob.data_ptr(), _lib.stream_ptr()),
                    "pdf_moe_sweep")
         return prob
+
+    def explain(self, X: Dict[str, torch.Tensor], masks: torch.Tensor, steps: int = 0):
+        """X {mod: [N,d] f32 cuda, UNMASKED}; masks [S,N,M] u8 in self.mods order -> device tensors of pdf_moe_explain:
+        (prob [S,N], base prob [1], Shapley values [S,N,M] of the probability, integrated gradients [[S,N,d_e] per expert] with
+        `steps` midpoints or None for steps = 0)."""
+        xs = [X[m].to(dtype=torch.float32).contiguous() for m in self.mods]
+        N, S = int(xs[0].shape[0]), int(masks.shape[0])
+        masks = masks.to(dtype=torch.uint8).contiguous()
+        if tuple(masks.shape) != (S, N, len(self.mods)):
+            raise ValueError("masks must be [S, N, M]")
+        dev = xs[0].device
+        ptrs = (C.c_void_p * len(xs))(*[x.data_ptr() for x in xs])
+        need = int(self.lib.pdf_moe_explain_workspace_bytes(C.byref(self.net), N, S, steps))
+        ws = torch.empty(need, dtype=torch.uint8, device=dev)
+        value = torch.empty((S, N), dtype=torch.float32, device=dev)
+        base = torch.empty(1, dtype=torch.float32, device=dev)
+        shap = torch.empty((S, N, len(self.mods)), dtype=torch.float32, device=dev)
+        ig = [torch.empty((S, N, x.shape[1]), dtype=torch.float32, device=dev) for x in xs] if steps > 0 else None
+        igp = (C.c_void_p * len(xs))(*[t.data_ptr() for t in ig]) if ig is not None else None
+        _lib.check(self.lib.pdf_moe_explain(C.byref(self.net), N, S, ptrs, masks.data_ptr(), steps, ws.data_ptr(), value.data_ptr(),
+                                            base.data_ptr(), shap.data_ptr(), igp, _lib.stream_ptr()), "pdf_moe_explain")
+        return value, base, shap, ig

@@ -2,7 +2,8 @@
 
 `ModalityDropoutNet` keeps the reference's layout (feature blocks in sorted(modality) order, `net.{0,3,6,..}`
 keys).  `predict_proba` runs on the device through pdf_moddrop_sweep; `predict_proba_sweep` evaluates every
-scenario mask of a missingness sweep in ONE launch (layer-1 partials per modality computed once).
+scenario mask of a missingness sweep in ONE launch (layer-1 partials per modality computed once).  `explain`
+returns the modalities' exact Shapley values and integrated gradients of the logit (pdf_moddrop_explain).
 """
 from __future__ import annotations
 
@@ -107,14 +108,29 @@ class ModalityDropoutModel(BaseModel):
             self._sweep = ModDropSweep(self.model.state_dict(), self.modality_dims, device=get_torch_device())
         return self._sweep
 
-    def predict_proba_sweep(self, X: np.ndarray, masks_snm: np.ndarray, order: List[str]) -> np.ndarray:
-        """X [N,F] (unmasked); masks_snm uint8 [S,N,len(order)] -> probabilities [S,N] f32, one launch."""
+    def _sweep_masks(self, masks_snm: np.ndarray, order: List[str]) -> np.ndarray:
+        """masks_snm [S,N,len(order)] -> [S,N,M] in the sweep's sorted(modality) order; modalities missing from `order` are present."""
         sw = self._get_sweep()
         cols = [order.index(m) if m in order else -1 for m in sw.mods]
         mk = np.ones(masks_snm.shape[:2] + (len(sw.mods),), dtype=np.uint8)
         for j, c in enumerate(cols):
             if c >= 0:
                 mk[:, :, j] = masks_snm[:, :, c]
+        return mk
+
+    def _single_mask(self, n: int, masks) -> np.ndarray:
+        mk = np.ones((1, n, len(self._get_sweep().mods)), dtype=np.uint8)
+        if masks is not None:
+            for j, mod in enumerate(self._get_sweep().mods):
+                if mod in masks:
+                    # the reference multiplies by the float mask value; masks are {0,1} on every call site
+                    mk[0, :, j] = np.asarray(masks[mod]) != 0
+        return mk
+
+    def predict_proba_sweep(self, X: np.ndarray, masks_snm: np.ndarray, order: List[str]) -> np.ndarray:
+        """X [N,F] (unmasked); masks_snm uint8 [S,N,len(order)] -> probabilities [S,N] f32, one launch."""
+        sw = self._get_sweep()
+        mk = self._sweep_masks(masks_snm, order)
         dev = sw.device
         prob = sw.forward(torch.as_tensor(np.asarray(X), dtype=torch.float32).to(dev), torch.from_numpy(mk).to(dev))
         return prob.cpu().numpy()
@@ -122,13 +138,30 @@ class ModalityDropoutModel(BaseModel):
     def predict_proba(self, X, masks=None):
         X = np.asarray(X)
         sw = self._get_sweep()
-        mk = np.ones((1, X.shape[0], len(sw.mods)), dtype=np.uint8)
-        if masks is not None:
-            for j, mod in enumerate(sw.mods):
-                if mod in masks:
-                    # the reference multiplies by the float mask value; masks are {0,1} on every call site
-                    mk[0, :, j] = np.asarray(masks[mod]) != 0
-        return self.predict_proba_sweep(X, mk, sw.mods)[0]
+        return self.predict_proba_sweep(X, self._single_mask(X.shape[0], masks), sw.mods)[0]
+
+    def explain_sweep(self, X: np.ndarray, masks_snm: np.ndarray, order: List[str], steps: int = 32) -> List[Dict]:
+        """`explain` under every scenario mask of masks_snm (uint8 [S,N,len(order)], as predict_proba_sweep) in one
+        pdf_moddrop_explain call -> one explanation dict per scenario."""
+        sw = self._get_sweep()
+        dev = sw.device
+        value, base, shap, ig = sw.explain(torch.as_tensor(np.asarray(X), dtype=torch.float32).to(dev),
+                                           torch.from_numpy(self._sweep_masks(masks_snm, order)).to(dev), steps)
+        prob = torch.sigmoid(value).cpu().numpy().astype(np.float64)
+        value, shap = value.cpu().numpy(), shap.cpu().numpy()
+        ig = ig.cpu().numpy() if ig is not None else None
+        b = float(base.item())
+        return [{"prob": prob[s], "logit": value[s], "base_logit": b, "shapley": {m: shap[s, :, j] for j, m in enumerate(sw.mods)},
+                 "ig": ig[s] if ig is not None else None} for s in range(value.shape[0])]
+
+    def explain(self, X, masks=None, steps: int = 32) -> Dict:
+        """Why each subject got its probability, for the arguments of `predict_proba` (X [N,F] unmasked, masks {mod: [N]} or None):
+        prob [N] (predict_proba's, as float64), logit [N] (before net's final sigmoid), base_logit (the logit of the all-zero input,
+        i.e. with every modality missing), shapley {mod: [N]} = exact Shapley values of the modalities for the logit (they add up
+        to logit - base_logit; 0 for a missing modality), and ig [N,F] = integrated gradients of the logit from the zero input
+        with `steps` midpoints (None for steps = 0; 0 on a missing modality's features)."""
+        X = np.asarray(X)
+        return self.explain_sweep(X, self._single_mask(X.shape[0], masks), self._get_sweep().mods, steps)[0]
 
     def save(self, path):
         torch.save(self.model.state_dict(), path)

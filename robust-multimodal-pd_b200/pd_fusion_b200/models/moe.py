@@ -1,6 +1,7 @@
 """Mixture-of-experts fusion head (reference: models/moe.py): one MLP expert per modality, a router MLP on the
 availability mask with softmax gating.  Inference runs through pdf_moe_sweep (router + experts + gated sum for
-every (scenario, subject) pair in one launch)."""
+every (scenario, subject) pair in one launch); `explain` returns the modalities' exact Shapley values and integrated gradients
+of the probability (pdf_moe_explain)."""
 from __future__ import annotations
 
 from typing import Dict, List, Optional
@@ -105,9 +106,7 @@ class MoEModel(BaseModel):
         Xd = {m: torch.as_tensor(np.asarray(X_dict[m]), dtype=torch.float32).to(dev) for m in sw.mods}
         return sw.forward(Xd, torch.from_numpy(np.ascontiguousarray(mk)).to(dev)).cpu().numpy()
 
-    def predict_proba(self, X_dict, mask=None):
-        """X_dict {mod: FloatTensor [N,d]} (already multiplied by the mask by the caller, evaluate.py:59-61),
-        mask FloatTensor [N,M] with columns in the X_dict key order the caller stacked them in."""
+    def _single(self, X_dict, mask):
         mods_in = list(X_dict.keys())
         if mods_in != sorted(mods_in):
             # the reference feeds the router mask columns in caller order but gates experts in sorted order
@@ -117,7 +116,36 @@ class MoEModel(BaseModel):
         m = np.ones((N, len(mods_in)), dtype=np.float32) if mask is None else np.asarray(mask, dtype=np.float32)
         mk = (m != 0).astype(np.uint8)[None]
         Xn = {k: (v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else np.asarray(v)) for k, v in X_dict.items()}
+        return Xn, mk, mods_in
+
+    def predict_proba(self, X_dict, mask=None):
+        """X_dict {mod: FloatTensor [N,d]} (already multiplied by the mask by the caller, evaluate.py:59-61),
+        mask FloatTensor [N,M] with columns in the X_dict key order the caller stacked them in."""
+        Xn, mk, mods_in = self._single(X_dict, mask)
         return self.predict_proba_sweep(Xn, mk, mods_in)[0]
+
+    def explain_sweep(self, X_dict: Dict[str, np.ndarray], masks_snm: np.ndarray, order: List[str], steps: int = 32) -> List[Dict]:
+        """`explain` under every scenario mask of masks_snm (uint8 [S,N,len(order)], as predict_proba_sweep; X_dict unmasked) in
+        one pdf_moe_explain call -> one explanation dict per scenario."""
+        sw = self._get_sweep()
+        mk = np.stack([masks_snm[:, :, order.index(m)] for m in sw.mods], axis=2).astype(np.uint8)
+        dev = sw.device
+        Xd = {m: torch.as_tensor(np.asarray(X_dict[m]), dtype=torch.float32).to(dev) for m in sw.mods}
+        value, base, shap, ig = sw.explain(Xd, torch.from_numpy(np.ascontiguousarray(mk)).to(dev), steps)
+        prob = value.cpu().numpy().astype(np.float64)
+        shap = shap.cpu().numpy()
+        ig = [t.cpu().numpy() for t in ig] if ig is not None else None
+        b = float(base.item())
+        return [{"prob": prob[s], "base_prob": b, "shapley": {m: shap[s, :, j] for j, m in enumerate(sw.mods)},
+                 "ig": {m: ig[j][s] for j, m in enumerate(sw.mods)} if ig is not None else None} for s in range(prob.shape[0])]
+
+    def explain(self, X_dict, mask=None, steps: int = 32) -> Dict:
+        """Why each subject got its probability, for the arguments of `predict_proba`: prob [N] (predict_proba's, as float64),
+        base_prob (the output for the all-zero input, every modality missing), shapley {mod: [N]} = exact Shapley values of the
+        modalities for the probability (they add up to prob - base_prob; 0 for a missing modality), and ig {mod: [N, d_m]} =
+        integrated gradients of the probability from the zero input with `steps` midpoints (None for steps = 0)."""
+        Xn, mk, mods_in = self._single(X_dict, mask)
+        return self.explain_sweep(Xn, mk, mods_in, steps)[0]
 
     def save(self, path):
         torch.save(self.model.state_dict(), path)
