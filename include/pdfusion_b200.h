@@ -507,6 +507,24 @@ int pdf_moe_explain(const pdf_moe* net, int n_subjects, int n_scenarios, const f
                     void* d_workspace, float* d_value /* [S,N] prob */, float* d_base /* [1] */, float* d_shap /* [S,N,E] */,
                     float* const* d_ig /* host array of E device ptrs [S,N,d_e], or NULL */, pdf_stream_t stream);
 
+/* Bootstrap replicates of the scenario metrics (csrc/metrics.cu), for every scenario in one call.  A Poisson(1) bootstrap: replicate b
+ * gives sampling unit u the integer weight w = Poisson1(philox4x32_10(key = seed, counter = (u, b, 0, 0)).x), Poisson1 = inversion of
+ * the 32-bit word against T_k = floor(2^32 P(X <= k)), k = 0..12 (w <= 13).  Weights are stateless in (seed, b, u): replicate b is the
+ * same whatever n_boot, n_scenarios or the unit count, and pairs across scenarios.
+ *   d_prob [S,N] float64 probabilities in [0, 1]; d_label [N], != 0 positive; d_unit [N] non-negative unit ids or NULL (unit = row);
+ *   d_out [S, 1+B, 6] float64: row 0 is the point estimate (every weight 1), row 1+b replicate b.  The six metrics are those of
+ *     utils.metrics.compute_metrics in its order (roc_auc, pr_auc, balanced_accuracy, f1, brier_score, ece), each equal to the
+ *     sklearn / numpy function with sample_weight = w: roc_auc NaN without both classes, pr_auc 0 without positives, balanced accuracy
+ *     the recall of the one class present, F1 0 on zero division; every metric NaN when the total weight is 0.
+ * AUC, balanced accuracy and F1 are exact integer rationals divided once; the float64 sums are in a fixed order, so calls are
+ * bit-identical.  n_boot = 0 computes the point estimate only.  Bad arguments (S < 1, N < 1 or N > 2^28, B < 0 or B > 2^20, NULL
+ * d_prob / d_label / d_workspace / d_out, d_prob or d_out not 8-byte, d_unit not 4-byte or d_workspace not 256-byte aligned) return
+ * PDF_ERR_ARG before any device work.  Workspace: pdf_bootstrap_metrics_workspace_bytes (0 for bad sizes). */
+size_t pdf_bootstrap_metrics_workspace_bytes(int n_scenarios, int n);
+int pdf_bootstrap_metrics(int n_scenarios, int n, int n_boot, uint64_t seed, const double* d_prob /* [S,N] */,
+                          const uint8_t* d_label /* [N], != 0 positive */, const int32_t* d_unit /* [N] or NULL = row index */,
+                          void* d_workspace, double* d_out /* [S, 1+B, 6] */, pdf_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * Self-tests of the tensor-core building blocks (used by tests/ and smoke on the GPU box).
  * pdf_selftest_umma: C[M,N] = A[M,K] * B[N,K]^T through TMA(2D tiled) + tcgen05.mma, bf16 in / f32 out.

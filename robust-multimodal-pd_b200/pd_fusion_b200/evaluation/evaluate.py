@@ -7,6 +7,8 @@ launch; tabular preprocessing runs once instead of once per scenario (evaluate.p
 Models that do not expose a sweep entry point (e.g. a CalibratedModel wrapper) fall back to the reference's
 per-scenario `predict_proba` calls -- each of which still runs on the device.
 `explain_model` explains a fusion head's predictions under the same scenario masks.
+`bootstrap_model` adds bootstrap confidence intervals, and paired intervals of each scenario's difference to a reference scenario, to
+`evaluate_model`'s metrics; the replicates are computed on the device (utils.metrics.bootstrap_metrics).
 """
 from __future__ import annotations
 
@@ -19,7 +21,7 @@ from ..data.feature_utils import apply_masks_to_matrix
 from ..data.missingness import apply_missingness_scenario, get_modality_mask_matrix, scenario_mask_tensor
 from ..data.preprocess import preprocess_features
 from ..data.schema import MODALITIES, TARGET_COL
-from ..utils.metrics import compute_metrics
+from ..utils.metrics import METRIC_NAMES, bootstrap_metrics, compute_metrics
 
 
 def _kind(prep_info) -> str:
@@ -99,6 +101,75 @@ def evaluate_model(model, df_test, mask_test, prep_info, config) -> Dict[str, Di
     probs, _ = _sweep_probs(model, df_test, mask_test, prep_info, scenarios)
     return {sc["name"]: _with_groups(compute_metrics(y_true, np.asarray(probs[s])), df_test, y_true, np.asarray(probs[s]), group_col)
             for s, sc in enumerate(scenarios)}
+
+
+def _group_units(groups: np.ndarray) -> Tuple[np.ndarray, int]:
+    """(unit id per row, G): the groups of _with_groups (groupby order, NaN keys dropped) are units 0..G-1, and each row whose key is
+    NaN is a unit of its own, numbered after them."""
+    ids = pd.DataFrame({"group": groups}).groupby("group").ngroup().to_numpy(dtype=np.float64, copy=True)
+    G = int(np.nanmax(ids)) + 1 if np.any(~np.isnan(ids)) else 0
+    lone = np.isnan(ids)
+    ids[lone] = G + np.arange(int(lone.sum()))
+    return ids.astype(np.int64), G
+
+
+def _interval(value: float, reps: np.ndarray, alpha: float) -> Dict[str, float]:
+    n = int(np.count_nonzero(~np.isnan(reps)))
+    lo, hi = np.nanpercentile(reps, [100 * alpha / 2, 100 * (1 - alpha / 2)]) if n else (np.nan, np.nan)
+    return {"value": float(value), "lo": float(lo), "hi": float(hi), "n_valid": n}
+
+
+def summarize_bootstrap(names: List[str], keys: List[str], point: np.ndarray, reps: np.ndarray, alpha: float = 0.05,
+                        ref: int = 0) -> Dict[str, Dict]:
+    """{scenario: {metric: {"value", "lo", "hi", "n_valid"}, "delta": {...}}} from point [S, K] and replicates [S, B, K]: percentile
+    intervals (np.nanpercentile, linear, at 100 alpha/2 and 100 (1 - alpha/2)) over the non-NaN replicates, and for every scenario but
+    `ref` the paired difference point[s] - point[ref] with the interval of reps[s, b] - reps[ref, b]."""
+    out = {}
+    for s, name in enumerate(names):
+        res = {k: _interval(point[s, j], reps[s, :, j], alpha) for j, k in enumerate(keys)}
+        if s != ref:
+            res["delta"] = {k: _interval(point[s, j] - point[ref, j], reps[s, :, j] - reps[ref, :, j], alpha) for j, k in enumerate(keys)}
+        out[name] = res
+    return out
+
+
+def bootstrap_model(model, df_test, mask_test, prep_info, config, n_boot: int = 1000, alpha: float = 0.05, seed: int = 0,
+                    reference=None) -> Dict[str, Dict]:
+    """evaluate_model's metrics with Poisson-bootstrap confidence intervals, computed on the device (utils.metrics.bootstrap_metrics):
+    {scenario: {metric: {"value", "lo", "hi", "n_valid"}, "subject_<metric>": ... (with config["group_col"]),
+    "delta": {metric: {...}} (every scenario but the reference)}}.
+
+    The probabilities come from the sweep exactly as in evaluate_model (same masks under the same numpy seed; nothing else draws from
+    numpy's RNG), so each "value" is evaluate_model's metric.  "lo"/"hi" are the alpha/2 and 1 - alpha/2 percentiles of the n_boot
+    replicates whose metric is defined ("n_valid" of them).  "delta" is the paired difference to the reference scenario (`reference`,
+    a scenario name; default the first): the same replicate b in both, so it carries no between-scenario resampling noise.  With
+    group_col the resampling unit is the group (rows without a group resample alone), and the subject_* metrics are computed on
+    _with_groups' group rows under the same replicates."""
+    if not 0 < alpha < 1:
+        raise ValueError("alpha must lie in (0, 1)")
+    scenarios = config.get("scenarios", [{"name": "baseline", "drop_modalities": []}])
+    names = [sc["name"] for sc in scenarios]
+    if reference is not None and reference not in names:
+        raise ValueError(f"reference scenario {reference!r} is not one of {names}")
+    ref = 0 if reference is None else names.index(reference)
+    group_col = config.get("group_col")
+    y_true = df_test[TARGET_COL].values
+    probs, _ = _sweep_probs(model, df_test, mask_test, prep_info, scenarios)
+    probs = [np.asarray(probs[s]) for s in range(len(scenarios))]
+    keys = list(METRIC_NAMES)
+    grouped = bool(group_col) and group_col in df_test.columns
+    units = _group_units(df_test[group_col].values)[0] if grouped else None
+    point, reps = bootstrap_metrics(y_true, np.stack([p.astype(np.float64) for p in probs]), n_boot, seed, units)
+    if grouped:
+        gy, gp = None, []
+        for p in probs:        # _with_groups' group rows, from the same dtype it sees
+            t = pd.DataFrame({"group": df_test[group_col].values, "y_true": y_true, "y_prob": p})
+            gy = t.groupby("group")["y_true"].first().values
+            gp.append(t.groupby("group")["y_prob"].mean().values.astype(np.float64))
+        gpoint, greps = bootstrap_metrics(gy, np.stack(gp), n_boot, seed, np.arange(len(gy)))
+        point, reps = np.concatenate([point, gpoint], axis=1), np.concatenate([reps, greps], axis=2)
+        keys += [f"subject_{k}" for k in METRIC_NAMES]
+    return summarize_bootstrap(names, keys, point, reps, alpha, ref)
 
 
 def explain_model(model, df_test, mask_test, prep_info, config, steps: int = 32) -> Dict[str, Dict]:
