@@ -525,6 +525,39 @@ int pdf_bootstrap_metrics(int n_scenarios, int n, int n_boot, uint64_t seed, con
                           const uint8_t* d_label /* [N], != 0 positive */, const int32_t* d_unit /* [N] or NULL = row index */,
                           void* d_workspace, double* d_out /* [S, 1+B, 6] */, pdf_stream_t stream);
 
+/* Monte-Carlo (MC) dropout uncertainty of the ModDrop and MIL heads (csrc/uncertainty.cu), for every scenario in one call: T = n_samples
+ * stochastic forward passes with the heads' nn.Dropout layers active (and nothing else: the scenario masks play the part of the
+ * training-time modality dropout).  Dropout probability p = p_drop in [0, 1) (a float, widened to double): unit j of row n, sample t
+ * is dropped iff
+ *   philox4x32_10(key = seed, counter = (n, t, (l << 16) | i, 0x80000000 | (j >> 2))).word[j & 3] < floor(p 2^32)   (float64),
+ * and a kept unit is multiplied by the float (float)(1 / (1 - p)).  ModDrop: n = subject row of d_x, l = hidden-layer index (0: the
+ * first hidden layer's output), i = 0.  MIL: n = bag index, l = 0, i = instance index within the bag.  The top bit of counter word 3
+ * keeps these streams apart from pdf_bootstrap_metrics' counters (u, b, 0, 0).  The masks are stateless: sample t of row n has the
+ * same masks under every scenario, and nothing depends on S, N, T or the launch shape.
+ *   d_stats [S,N,5] float64, per (scenario, subject) over the T sample probabilities p_t, in ascending t:
+ *     0 mean = mean_t p_t;  1 std = sqrt(mean_t (p_t - mean)^2) (population);  2 entropy = H(mean),
+ *     H(q) = -q ln q - (1-q) ln(1-q) with 0 ln 0 = 0 (nats);  3 expected_entropy = mean_t H(p_t);
+ *     4 mutual_info = max(0, entropy - expected_entropy).  T equal samples give exactly mean = p_t, std = mutual_info = 0.
+ *   d_samples [S,N,T] float32 sample probabilities, or NULL.
+ * ModDrop: d_x [N,F] and d_masks [S,N,M] as pdf_moddrop_sweep.  Layer 1 comes from the sweep's per-modality partials, layers 2.. run
+ *   on the shared-memory tile of pdf_moddrop_explain (a net too wide for it is refused the same way); with p = 0 every sample is the
+ *   sweep's probability up to float32 rounding.
+ * MIL: d_bags, d_len, d_live [S,n_bags] (NULL: live everywhere) as pdf_mil_sweep, FP32 arithmetic whatever the sweep's precision;
+ *   live[s, b] && len[b] > 0 selects the bag's samples (which do not depend on s), anything else is missing_prob for every sample.
+ *   Lmax <= 65536.
+ * Bad arguments (p outside [0, 1), T outside 1..4096, S < 1, N < 1, NULL inputs, workspace or d_stats, d_stats not 8-byte, the float
+ * and int arrays not 4-byte or d_workspace not 256-byte aligned, a net the tile does not fit) return PDF_ERR_ARG before any device
+ * work.  No atomics: two calls are bit-identical.  Workspace: pdf_moddrop_mc_workspace_bytes / pdf_mil_mc_workspace_bytes (0 for bad
+ * sizes). */
+size_t pdf_moddrop_mc_workspace_bytes(const pdf_mlp* net, int n_subjects, int n_scenarios, int n_samples);
+int pdf_moddrop_mc(const pdf_mlp* net, float p_drop, int n_subjects, int n_scenarios, const float* d_x, const uint8_t* d_masks,
+                   int n_samples, uint64_t seed, void* d_workspace, double* d_stats /* [S,N,5] */,
+                   float* d_samples /* [S,N,T] or NULL */, pdf_stream_t stream);
+size_t pdf_mil_mc_workspace_bytes(const pdf_mil_weights* w, int n_bags, int Lmax, int n_samples);
+int pdf_mil_mc(const pdf_mil_weights* w, float p_drop, int n_bags, int Lmax, const float* d_bags, const int32_t* d_len,
+               int n_scenarios, const uint8_t* d_live /* [S,n_bags] or NULL */, int n_samples, uint64_t seed,
+               void* d_workspace, double* d_stats /* [S,n_bags,5] */, float* d_samples /* [S,n_bags,T] or NULL */, pdf_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * Self-tests of the tensor-core building blocks (used by tests/ and smoke on the GPU box).
  * pdf_selftest_umma: C[M,N] = A[M,K] * B[N,K]^T through TMA(2D tiled) + tcgen05.mma, bf16 in / f32 out.

@@ -5,6 +5,9 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string.h>
+#ifdef __CUDACC__
+#include <curand_philox4x32_x.h>
+#endif
 
 #include "../../include/pdfusion_b200.h"
 
@@ -83,6 +86,11 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+// Philox4x32-10 (Salmon et al., SC'11; curand's constants and rounds): four 32-bit words, a pure function of (counter, key).  The
+// device's stateless random streams: the bootstrap weights (metrics.cu, counters (unit, b, 0, 0)) and the Monte-Carlo dropout masks
+// (uncertainty.cu, counters with the top bit of word 3 set), each from key = (seed low, seed high).
+__device__ __forceinline__ uint4 philox4x32_10(uint4 counter, uint2 key) { return curand_Philox4x32_10(counter, key); }
 #endif
 
 int num_sms();

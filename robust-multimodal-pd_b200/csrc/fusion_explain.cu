@@ -12,12 +12,12 @@
 #include <algorithm>
 
 #include "common.cuh"
+#include "mlp_tile.cuh"
 #include "ops.cuh"
 
 namespace pdf {
 
 constexpr int kMaxIgSteps = 256;
-constexpr size_t kIgSmemMax = 227 * 1024;
 
 static size_t fx_align(size_t n) { return (n + 63) & ~(size_t)63; }     // floats -> 256-byte aligned workspace regions
 
@@ -55,56 +55,6 @@ shapley_combine_kernel(const float* __restrict__ v, const uint8_t* __restrict__ 
       }
     }
     shap[i] = (float)phi;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------------
-// One linear layer on the rows of a tile: out(r, c) = sum_k in[r][k] W(k, c), k ascending, 64-column x 16-k weight chunks in shared
-// memory, a 16 x 16 thread grid with RT rows x 4 columns each (moddrop_tile_kernel's loop).  kBackward = false: W(k, c) = W[c * n_in + k]
-// (the forward x W^T, W [n_out, n_in]); true: W(k, c) = W[k * n_out + c] (delta W, W [n_in, n_out]).  epi(r, c, acc) takes every
-// valid output; it may overwrite any buffer but `in`.
-template <int RT, bool kBackward, typename Epi>
-__device__ __forceinline__ void tile_layer(const float* in, int in_stride, const float* __restrict__ W, int n_in, int n_out, float* Ws,
-                                           Epi epi) {
-  const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15;
-  for (int c0 = 0; c0 < n_out; c0 += 64) {
-    float acc[RT][4];
-#pragma unroll
-    for (int i = 0; i < RT; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[i][j] = 0.f;
-    for (int k0 = 0; k0 < n_in; k0 += 16) {
-      if (!kBackward) {
-        const int col = c0 + (tid >> 2), kk = (tid & 3) * 4;
-#pragma unroll
-        for (int e = 0; e < 4; ++e)
-          Ws[(kk + e) * 68 + (tid >> 2)] = (col < n_out && k0 + kk + e < n_in) ? __ldg(W + (size_t)col * n_in + k0 + kk + e) : 0.f;
-      } else {
-        const int kk = tid >> 4, cc = (tid & 15) * 4;
-#pragma unroll
-        for (int e = 0; e < 4; ++e)
-          Ws[kk * 68 + cc + e] = (c0 + cc + e < n_out && k0 + kk < n_in) ? __ldg(W + (size_t)(k0 + kk) * n_out + c0 + cc + e) : 0.f;
-      }
-      __syncthreads();
-      const int kmax = min(16, n_in - k0);
-      for (int kk = 0; kk < kmax; ++kk) {
-        float a[RT], b[4];
-#pragma unroll
-        for (int i = 0; i < RT; ++i) a[i] = in[(ty * RT + i) * in_stride + k0 + kk];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) b[j] = Ws[kk * 68 + tx * 4 + j];
-#pragma unroll
-        for (int i = 0; i < RT; ++i)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
-      }
-      __syncthreads();
-    }
-#pragma unroll
-    for (int i = 0; i < RT; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j)
-        if (c0 + tx * 4 + j < n_out) epi(ty * RT + i, c0 + tx * 4 + j, acc[i][j]);
   }
 }
 
@@ -254,23 +204,6 @@ moe_ig_finish_kernel(const float* __restrict__ x, int d, const uint8_t* __restri
 
 static int ew_grid(long long n) { return (int)std::max<long long>(1, std::min<long long>((n + 255) / 256, (long long)num_sms() * 16)); }
 
-// The widest IG tile (64, 32 or 16 rows) whose shared memory fits: weight chunk, seeds, and every hidden layer's activations.
-static int ig_tile(const pdf_mlp& net, int* tp, size_t* smem, const char* what) {
-  size_t widths = 0;
-  for (int l = 1; l <= std::max(net.n_layers - 1, 1); ++l) widths += (size_t)net.dims[l] + 1;
-  for (int t = 64; t >= 16; t /= 2) {
-    const size_t b = (16 * 68 + (size_t)t + (size_t)t * widths) * sizeof(float);
-    if (b <= kIgSmemMax) {
-      *tp = t;
-      *smem = b;
-      return PDF_OK;
-    }
-  }
-  set_error("%s: hidden layers too wide for the integrated-gradients tile (%zu activations per row; 16 rows need more than 227 KB)", what,
-            widths);
-  return PDF_ERR_ARG;
-}
-
 template <int TP, bool kSigmoidSeed>
 static int ig_launch_tp(const pdf_mlp& net, const float* partials, const uint8_t* masks, int M, int N, int S, int K, size_t smem,
                         float* dbar, cudaStream_t s) {
@@ -288,7 +221,7 @@ template <bool kSigmoidSeed>
 static int ig_launch(const pdf_mlp& net, const float* partials, const uint8_t* masks, int M, int N, int S, int K, float* dbar, cudaStream_t s) {
   int tp = 0;
   size_t smem = 0;
-  if (int rc = ig_tile(net, &tp, &smem, "mlp_ig_kernel")) return rc;
+  if (int rc = mlp_tile(net, &tp, &smem, "mlp_ig_kernel")) return rc;
   if (tp == 64) return ig_launch_tp<64, kSigmoidSeed>(net, partials, masks, M, N, S, K, smem, dbar, s);
   if (tp == 32) return ig_launch_tp<32, kSigmoidSeed>(net, partials, masks, M, N, S, K, smem, dbar, s);
   return ig_launch_tp<16, kSigmoidSeed>(net, partials, masks, M, N, S, K, smem, dbar, s);
@@ -329,7 +262,7 @@ extern "C" int pdf_moddrop_explain(const pdf_mlp* net, int n_subjects, int n_sce
   if (d_ig && L > 1) {
     int tp;
     size_t smem;
-    if (int rc = ig_tile(*net, &tp, &smem, what)) return rc;
+    if (int rc = mlp_tile(*net, &tp, &smem, what)) return rc;
   }
   cudaStream_t s = as_stream(stream);
   const size_t N = (size_t)n_subjects, S = (size_t)n_scenarios;
@@ -390,7 +323,7 @@ extern "C" int pdf_moe_explain(const pdf_moe* net, int n_subjects, int n_scenari
       PDF_REQUIRE(d_ig[e], "pdf_moe_explain: null d_ig[%d]", e);
       int tp;
       size_t smem;
-      if (int rc = ig_tile(net->expert[e], &tp, &smem, what)) return rc;
+      if (int rc = mlp_tile(net->expert[e], &tp, &smem, what)) return rc;
     }
   }
   cudaStream_t s = as_stream(stream);

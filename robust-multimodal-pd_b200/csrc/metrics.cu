@@ -21,7 +21,6 @@
 #include <algorithm>
 
 #include <cub/device/device_radix_sort.cuh>
-#include <curand_philox4x32_x.h>
 
 #include "common.cuh"
 
@@ -37,7 +36,7 @@ __device__ __forceinline__ uint32_t boot_weight(uint2 key, uint32_t unit, uint32
   // floor(2^32 P(X <= k)), X ~ Poisson(1), k = 0..12 (T_12 = 2^32 - 1)
   constexpr uint32_t kPoisson1[13] = {0x5e2d58d8u, 0xbc5ab1b1u, 0xeb715e1du, 0xfb239797u, 0xff1025f5u, 0xffd90f3bu, 0xfffa8b71u,
                                       0xffff540cu, 0xffffed1fu, 0xfffffe21u, 0xffffffd4u, 0xfffffffcu, 0xffffffffu};
-  const uint32_t u = curand_Philox4x32_10(make_uint4(unit, b, 0u, 0u), key).x;
+  const uint32_t u = philox4x32_10(make_uint4(unit, b, 0u, 0u), key).x;
   uint32_t w = 0;
 #pragma unroll
   for (int k = 0; k < 13; ++k) w += u >= kPoisson1[k];

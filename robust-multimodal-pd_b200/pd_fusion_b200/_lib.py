@@ -154,6 +154,10 @@ PROTOTYPES = {
     "pdf_moe_explain": (C.c_int, [C.POINTER(Moe), C.c_int, C.c_int, C.POINTER(_P), _P, C.c_int, _P, _P, _P, _P, C.POINTER(_P), _P]),
     "pdf_bootstrap_metrics_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int]),
     "pdf_bootstrap_metrics": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_uint64, _P, _P, _P, _P, _P, _P]),
+    "pdf_moddrop_mc_workspace_bytes": (C.c_size_t, [C.POINTER(Mlp), C.c_int, C.c_int, C.c_int]),
+    "pdf_moddrop_mc": (C.c_int, [C.POINTER(Mlp), C.c_float, C.c_int, C.c_int, _P, _P, C.c_int, C.c_uint64, _P, _P, _P, _P]),
+    "pdf_mil_mc_workspace_bytes": (C.c_size_t, [C.POINTER(MilWeights), C.c_int, C.c_int, C.c_int]),
+    "pdf_mil_mc": (C.c_int, [C.POINTER(MilWeights), C.c_float, C.c_int, C.c_int, _P, _P, C.c_int, _P, C.c_int, C.c_uint64, _P, _P, _P, _P]),
     "pdf_gemm_f32": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, C.c_long, C.c_long, _P, C.c_long, C.c_long, _P, C.c_long, _P, C.c_int, C.c_int, _P]),
     "pdf_conv_dgrad_f32": (C.c_int, [C.POINTER(Op), _P, _P, _P, C.c_int, _P]),
     "pdf_conv_wgrad_f32": (C.c_int, [C.POINTER(Op), _P, _P, _P, _P]),

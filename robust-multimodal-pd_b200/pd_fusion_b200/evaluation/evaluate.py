@@ -9,6 +9,7 @@ per-scenario `predict_proba` calls -- each of which still runs on the device.
 `explain_model` explains a fusion head's predictions under the same scenario masks.
 `bootstrap_model` adds bootstrap confidence intervals, and paired intervals of each scenario's difference to a reference scenario, to
 `evaluate_model`'s metrics; the replicates are computed on the device (utils.metrics.bootstrap_metrics).
+`uncertainty_model` estimates every subject's predictive uncertainty under every scenario by Monte-Carlo dropout on the device.
 """
 from __future__ import annotations
 
@@ -187,6 +188,45 @@ def explain_model(model, df_test, mask_test, prep_info, config, steps: int = 32)
     X, masks, _, order = _fusion_inputs(df_test, mask_test, prep_info, scenarios)
     ex = model.explain_sweep(X, masks, order, steps)
     return {sc["name"]: ex[s] for s, sc in enumerate(scenarios)}
+
+
+def _risk_coverage_by_entropy(y_true, mean, entropy) -> Dict:
+    """subjects ranked by entropy ascending (stable): risk at coverage k/N = error rate of the first k predictions (mean >= 0.5),
+    aurc = the mean risk"""
+    order = np.argsort(entropy, kind="stable")
+    err = ((np.asarray(mean) >= 0.5).astype(int) != np.asarray(y_true).astype(int)).astype(np.float64)[order]
+    k = np.arange(1, len(err) + 1)
+    risk = np.cumsum(err) / k
+    return {"coverage": k / len(err), "risk": risk, "aurc": float(np.mean(risk))}
+
+
+def uncertainty_model(model, df_test, mask_test, prep_info, config, n_samples: int = 32, seed: int = 0) -> Dict[str, Dict]:
+    """Monte-Carlo dropout uncertainty of every test subject under every scenario of `config`, in one device call for all of them:
+    {scenario: {"mean", "std", "entropy", "expected_entropy", "mutual_info": [N] float64, "risk_coverage": {"coverage", "risk",
+    "aurc"}}}.  The scenario masks are drawn as evaluate_model draws them (same helper, same numpy RNG order, nothing else drawn), and
+    the dropout masks come from a counter-based generator keyed by `seed`, so numpy's and torch's RNGs are left as evaluate_model
+    leaves them.  risk_coverage ranks the subjects by entropy (most certain first) and gives the error rate of the prediction
+    mean >= 0.5 among the first k, and its mean (aurc).  Needs a head with dropout: ModalityDropoutModel or MilAttentionModel."""
+    if not hasattr(model, "predict_uncertainty_sweep") or hasattr(model, "mask_dim") or _kind(prep_info) == "moe":
+        raise ValueError(f"{type(model).__name__} has no Monte-Carlo dropout uncertainty: uncertainty_model supports "
+                         "ModalityDropoutModel and MilAttentionModel (MoENet has no dropout layer)")
+    scenarios = config.get("scenarios", [{"name": "baseline", "drop_modalities": []}])
+    y_true = df_test[TARGET_COL].values
+    if _kind(prep_info) == "mil":
+        _, per = scenario_mask_tensor(df_test, scenarios, mask_test, list(mask_test.keys()))
+        bags = df_test[prep_info[1]].tolist()
+        n = len(bags)
+        mri = np.stack([np.asarray(cur["mri"]) if "mri" in cur else np.ones(n, dtype=int) for cur in per])
+        res = model.predict_uncertainty_sweep(bags, mri, n_samples, seed)
+    else:
+        X, masks, _, order = _fusion_inputs(df_test, mask_test, prep_info, scenarios)
+        res = model.predict_uncertainty_sweep(X, masks, order, n_samples, seed)
+    out = {}
+    for s, sc in enumerate(scenarios):
+        r = dict(res[s])
+        r["risk_coverage"] = _risk_coverage_by_entropy(y_true, r["mean"], r["entropy"])
+        out[sc["name"]] = r
+    return out
 
 
 def predict_proba_for_scenario(model, df_test, mask_test, prep_info, scenario):

@@ -1,6 +1,6 @@
 """Host side of K3/K4: thin wrappers that marshal state_dict tensors into the C structs of
-pdf_mil_forward / pdf_mil_explain / pdf_gradcam / pdf_moddrop_sweep / pdf_moe_sweep / pdf_moddrop_explain / pdf_moe_explain.
-No arithmetic happens here.
+pdf_mil_forward / pdf_mil_explain / pdf_gradcam / pdf_moddrop_sweep / pdf_moe_sweep / pdf_moddrop_explain / pdf_moe_explain /
+pdf_moddrop_mc / pdf_mil_mc.  No arithmetic happens here.
 """
 from __future__ import annotations
 
@@ -11,6 +11,23 @@ import numpy as np
 import torch
 
 from . import _lib
+
+
+MC_STATS = ("mean", "std", "entropy", "expected_entropy", "mutual_info")     # the last axis of pdf_moddrop_mc / pdf_mil_mc's stats
+
+
+def mc_dicts(stats: torch.Tensor, samples: Optional[torch.Tensor]) -> List[Dict[str, np.ndarray]]:
+    """stats [S, N, 5] (and samples [S, N, T] or None) of an `mc` call -> one dict per scenario: the five statistics as [N] float64
+    arrays (MC_STATS order), plus "samples" [N, T] float64 when samples were returned."""
+    st = stats.cpu().numpy()
+    sm = samples.cpu().numpy().astype(np.float64) if samples is not None else None
+    out = []
+    for s in range(st.shape[0]):
+        d = {k: st[s, :, j].copy() for j, k in enumerate(MC_STATS)}
+        if sm is not None:
+            d["samples"] = sm[s]
+        out.append(d)
+    return out
 
 
 def _dev_f32(t, device) -> torch.Tensor:
@@ -113,6 +130,30 @@ class MilHead:
                                             attn.data_ptr(), contrib.data_ptr(), _lib.ptr(dX), _lib.stream_ptr()), "pdf_mil_explain")
         return logit, attn, contrib, dX
 
+    def mc(self, bags: torch.Tensor, lens: torch.Tensor, live: Optional[torch.Tensor] = None, n_scenarios: int = 1, n_samples: int = 32,
+           seed: int = 0, p: float = 0.0, samples: bool = False):
+        """Monte-Carlo dropout of pdf_mil_mc: n_samples forward passes with the instance layer's dropout (probability p) active.
+        bags, lens and live as `sweep` -> device tensors (stats [S, n, 5] float64: mean, std, entropy, expected_entropy, mutual_info;
+        sample probabilities [S, n, T] f32 with `samples`, else None).  Bag b's masks are a function of (seed, b, sample) only.  Always
+        the FP32 head arithmetic, whatever `precision` says."""
+        if bags.dtype != torch.float32 or not bags.is_cuda or not bags.is_contiguous() or bags.shape[2] != self.D:
+            raise ValueError("bags must be a contiguous float32 CUDA tensor [n, Lmax, D]")
+        n, lmax = int(bags.shape[0]), int(bags.shape[1])
+        lens = lens.to(device=bags.device, dtype=torch.int32).contiguous()
+        if live is not None:
+            live = live.to(device=bags.device, dtype=torch.uint8).contiguous()
+            n_scenarios = int(live.shape[0])
+            if tuple(live.shape) != (n_scenarios, n):
+                raise ValueError("live must be [S, n]")
+        need = int(self.lib.pdf_mil_mc_workspace_bytes(C.byref(self.w), n, lmax, int(n_samples)))
+        ws = torch.empty(max(need, 1), dtype=torch.uint8, device=bags.device)
+        stats = torch.empty((n_scenarios, n, 5), dtype=torch.float64, device=bags.device)
+        smp = torch.empty((n_scenarios, n, int(n_samples)), dtype=torch.float32, device=bags.device) if samples else None
+        _lib.check(self.lib.pdf_mil_mc(C.byref(self.w), float(p), n, lmax, bags.data_ptr(), lens.data_ptr(), n_scenarios, _lib.ptr(live),
+                                       int(n_samples), int(seed) & (2 ** 64 - 1), ws.data_ptr(), stats.data_ptr(), _lib.ptr(smp),
+                                       _lib.stream_ptr()), "pdf_mil_mc")
+        return stats, smp
+
 
 def gradcam(fmap: torch.Tensor, g: torch.Tensor, out_hw, cam_small: bool = False):
     """Grad-CAM of pdf_gradcam: fmap [n, hw, hw, C] f32 cuda (the feature map whose spatial mean is the embedding), g [n, C] f32 =
@@ -196,6 +237,25 @@ class ModDropSweep:
                                                 value.data_ptr(), base.data_ptr(), shap.data_ptr(), _lib.ptr(ig), _lib.stream_ptr()),
                    "pdf_moddrop_explain")
         return value, base, shap, ig
+
+    def mc(self, X: torch.Tensor, masks: torch.Tensor, n_samples: int = 32, seed: int = 0, p: float = 0.0, samples: bool = False):
+        """Monte-Carlo dropout of pdf_moddrop_mc: n_samples forward passes with every hidden layer's dropout (probability p) active.
+        X [N,F] f32 cuda (unmasked); masks [S,N,M] u8 cuda in self.mods order -> device tensors (stats [S,N,5] float64: mean, std,
+        entropy, expected_entropy, mutual_info; sample probabilities [S,N,T] f32 with `samples`, else None).  Subject n's masks
+        are a function of (seed, n, sample) only, the same under every scenario."""
+        N, S = int(X.shape[0]), int(masks.shape[0])
+        X = X.to(dtype=torch.float32).contiguous()
+        masks = masks.to(dtype=torch.uint8).contiguous()
+        if tuple(masks.shape) != (S, N, len(self.mods)) or X.shape[1] != int(self.net.dims[0]):
+            raise ValueError("X must be [N, F] and masks [S, N, M]")
+        need = int(self.lib.pdf_moddrop_mc_workspace_bytes(C.byref(self.net), N, S, int(n_samples)))
+        ws = torch.empty(max(need, 1), dtype=torch.uint8, device=X.device)
+        stats = torch.empty((S, N, 5), dtype=torch.float64, device=X.device)
+        smp = torch.empty((S, N, int(n_samples)), dtype=torch.float32, device=X.device) if samples else None
+        _lib.check(self.lib.pdf_moddrop_mc(C.byref(self.net), float(p), N, S, X.data_ptr(), masks.data_ptr(), int(n_samples),
+                                           int(seed) & (2 ** 64 - 1), ws.data_ptr(), stats.data_ptr(), _lib.ptr(smp), _lib.stream_ptr()),
+                   "pdf_moddrop_mc")
+        return stats, smp
 
 
 class MoeSweep:

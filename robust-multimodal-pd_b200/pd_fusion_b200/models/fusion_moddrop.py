@@ -3,7 +3,8 @@
 `ModalityDropoutNet` keeps the reference's layout (feature blocks in sorted(modality) order, `net.{0,3,6,..}`
 keys).  `predict_proba` runs on the device through pdf_moddrop_sweep; `predict_proba_sweep` evaluates every
 scenario mask of a missingness sweep in ONE launch (layer-1 partials per modality computed once).  `explain`
-returns the modalities' exact Shapley values and integrated gradients of the logit (pdf_moddrop_explain).
+returns the modalities' exact Shapley values and integrated gradients of the logit (pdf_moddrop_explain).  `predict_uncertainty`
+estimates the predictive uncertainty by Monte-Carlo dropout (pdf_moddrop_mc).
 """
 from __future__ import annotations
 
@@ -13,7 +14,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from ..heads import ModDropSweep
+from ..heads import ModDropSweep, mc_dicts
 from ..utils.torch_utils import get_torch_device
 from .base import BaseModel
 
@@ -162,6 +163,33 @@ class ModalityDropoutModel(BaseModel):
         with `steps` midpoints (None for steps = 0; 0 on a missing modality's features)."""
         X = np.asarray(X)
         return self.explain_sweep(X, self._single_mask(X.shape[0], masks), self._get_sweep().mods, steps)[0]
+
+    def _dropout_p(self) -> float:
+        """the probability of the net's nn.Dropout layers (0 for a net without hidden layers)"""
+        ps = {float(m.p) for m in self.model.net if isinstance(m, nn.Dropout)}
+        if len(ps) > 1:
+            raise ValueError(f"Monte-Carlo dropout needs one dropout probability for every hidden layer, got {sorted(ps)}")
+        return ps.pop() if ps else 0.0
+
+    def predict_uncertainty_sweep(self, X: np.ndarray, masks_snm: np.ndarray, order: List[str], n_samples: int = 32, seed: int = 0,
+                                  return_samples: bool = False) -> List[Dict]:
+        """`predict_uncertainty` under every scenario mask of masks_snm (uint8 [S,N,len(order)], as predict_proba_sweep) in one
+        pdf_moddrop_mc call -> one dict per scenario.  Sample t of a subject drops the same units under every scenario."""
+        sw = self._get_sweep()
+        dev = sw.device
+        stats, smp = sw.mc(torch.as_tensor(np.asarray(X), dtype=torch.float32).to(dev), torch.from_numpy(self._sweep_masks(masks_snm, order)).to(dev),
+                           n_samples, seed, self._dropout_p(), return_samples)
+        return mc_dicts(stats, smp)
+
+    def predict_uncertainty(self, X, masks=None, n_samples: int = 32, seed: int = 0, return_samples: bool = False) -> Dict:
+        """Monte-Carlo dropout for the arguments of `predict_proba`: n_samples forward passes with the net's own nn.Dropout layers
+        active (their probability p; the training-time modality dropout stays off, the masks decide which modalities are present).
+        Returns [N] float64 arrays "mean" (of the sample probabilities), "std" (population), "entropy" (of the mean, nats),
+        "expected_entropy" (mean entropy of the samples) and "mutual_info" (max(0, entropy - expected_entropy): the model's own,
+        epistemic, part), and with return_samples "samples" [N, n_samples].  Stateless in (seed, subject row, sample)."""
+        X = np.asarray(X)
+        return self.predict_uncertainty_sweep(X, self._single_mask(X.shape[0], masks), self._get_sweep().mods, n_samples, seed,
+                                              return_samples)[0]
 
     def save(self, path):
         torch.save(self.model.state_dict(), path)

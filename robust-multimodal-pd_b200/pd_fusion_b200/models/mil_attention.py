@@ -3,7 +3,8 @@
 `MILAttentionNet` keeps the reference's parameter names so its `state_dict` is the weight-interchange format
 (SURVEY.md A.6).  Inference (`predict_proba`) runs ALL bags in one launch of pdf_mil_forward instead of the
 reference's per-bag B=1 loop with a `.cpu()` per bag (mil_attention.py:169-177).  Training (`train`) runs the native forward/backward/Adam
-kernels of csrc/train.cu through pd_fusion_b200/training.py (SURVEY.md 8f rank 2).
+kernels of csrc/train.cu through pd_fusion_b200/training.py (SURVEY.md 8f rank 2).  `predict_uncertainty` estimates the predictive
+uncertainty by Monte-Carlo dropout of the instance layer (pdf_mil_mc).
 """
 from __future__ import annotations
 
@@ -13,7 +14,7 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from ..heads import MilHead
+from ..heads import MilHead, mc_dicts
 from ..utils.torch_utils import get_torch_device
 from .base import BaseModel
 
@@ -211,6 +212,37 @@ class MilAttentionModel(BaseModel):
         live = None if mri_masks is None else torch.from_numpy(np.ascontiguousarray(np.asarray(mri_masks)[:, have] != 0).astype(np.uint8))
         out[:, have] = head.sweep(X, lens, live, S).cpu().numpy().astype(np.float64)
         return out
+
+    def predict_uncertainty_sweep(self, bags: List[Optional[np.ndarray]], mri_masks: Optional[np.ndarray], n_samples: int = 32,
+                                  seed: int = 0, return_samples: bool = False) -> List[dict]:
+        """`predict_uncertainty` under every scenario of mri_masks ([S, N] {0,1} as predict_proba_sweep; None = one scenario,
+        everything present) in one pdf_mil_mc call -> one dict per scenario.  Every bag position is uploaded (absent ones empty), so
+        bag i's masks depend on (seed, i, sample) only and a bag's samples are the same under every scenario where it is present."""
+        head = self._get_head()
+        n = len(bags)
+        S = 1 if mri_masks is None else int(np.asarray(mri_masks).shape[0])
+        lmax = max([1] + [np.asarray(b).shape[0] for b in bags if b is not None])
+        X = np.zeros((n, lmax, head.D), dtype=np.float32)
+        lens = np.zeros(n, dtype=np.int32)
+        for i, b in enumerate(bags):
+            if b is not None:
+                b = np.asarray(b, dtype=np.float32)
+                X[i, : b.shape[0]] = b
+                lens[i] = b.shape[0]
+        live = None if mri_masks is None else torch.from_numpy(np.ascontiguousarray(np.asarray(mri_masks) != 0).astype(np.uint8))
+        stats, smp = head.mc(torch.from_numpy(X).to(head.device), torch.from_numpy(lens).to(head.device), live, S, n_samples, seed,
+                             float(self.model.instance[2].p), return_samples)
+        return mc_dicts(stats, smp)
+
+    def predict_uncertainty(self, bags: List[Optional[np.ndarray]], masks=None, n_samples: int = 32, seed: int = 0,
+                            return_samples: bool = False) -> dict:
+        """Monte-Carlo dropout for the arguments of `predict_proba` (a bag that is None or whose masks["mri"] is 0 is missing):
+        n_samples forward passes with the instance layer's nn.Dropout active.  Returns [N] float64 arrays "mean", "std"
+        (population), "entropy" (of the mean, nats), "expected_entropy" and "mutual_info" (max(0, entropy - expected_entropy)), and
+        with return_samples "samples" [N, n_samples].  A missing bag gets mean = missing_prob, std = mutual_info = 0.  Always the
+        FP32 head arithmetic, whatever `precision` says."""
+        mri = masks["mri"] if isinstance(masks, dict) and "mri" in masks else None
+        return self.predict_uncertainty_sweep(bags, None if mri is None else np.asarray(mri)[None], n_samples, seed, return_samples)[0]
 
     def save(self, path):
         torch.save(self.model.state_dict(), path)
