@@ -443,6 +443,41 @@ int pdf_clip_scale(const float* d_sumsq, float max_norm, float* d_out2, pdf_stre
 int pdf_adam_step(float* d_param, const float* d_grad, float* d_m, float* d_v, size_t n, float lr, float beta1, float beta2, float eps,
                   float weight_decay, int step, const float* d_grad_scale, pdf_stream_t stream);
 
+/* Deep ensembles: the training kernels above for n_members (1..1024) heads of one architecture in one launch (the statistics:
+ * csrc/uncertainty.cu).
+ * Member e of an operand starts e * (its member stride, in elements) after member 0; stride 0 = shared by every member.  Per member
+ * the results are those of the single kernels: pdf_gemm_f32_batched bit for bit; the loss kernels' elementwise outputs (prob, dz, dr,
+ * dh, dvu) bit for bit, their losses and parameter gradients reduced in a fixed order (no atomics), so calls are bit-identical and a
+ * member's results do not depend on the other members.  Null or misaligned pointers and bad sizes return PDF_ERR_ARG before any
+ * device work.
+ * pdf_bce_sigmoid_train_batched: d_z, d_prob, d_dz [E, n], d_y member stride y_es; d_loss [E] WRITTEN (the member's mean BCE).
+ * pdf_moe_combine_train_batched: d_z, d_r, d_dz, d_dr [E, n, n_experts], d_out [E, n], d_y member stride y_es, d_loss [E] written.
+ * pdf_mil_pool_train_batched: w / t hold member 0's head weights and gradient accumulators, member e's are w_es / g_es floats further;
+ *   d_h [E, n_bags*Lmax, H], d_vu [E, n_bags*Lmax, NA], d_len, d_target, d_prob [E, n_bags]; gradients ACCUMULATED (each the sum over
+ *   bags in bag order), d_loss [E] written; workspace pdf_mil_pool_train_batched_workspace_bytes.
+ * pdf_clip_scale_batched: d_scale[e] = min(1, max_norm / (||row e of d_grad [E, n_params]|| + 1e-6)), clip_grad_norm_ per member.
+ * pdf_adam_step_batched: pdf_adam_step over [E, n_params] with member e's gradient scaled by d_grad_scale[e] (NULL = 1); a member
+ *   whose d_active[e] is 0 keeps its parameters and moments (d_active NULL = all active). */
+int pdf_gemm_f32_batched(int n_members, int M, int N, int K, const float* A, long a_rs, long a_cs, long a_es, const float* B, long b_rs,
+                         long b_cs, long b_es, float* C, long c_rs, long c_es, const float* bias, long bias_es, int act, int accumulate,
+                         pdf_stream_t stream);
+int pdf_bce_sigmoid_train_batched(int n_members, int n, const float* d_z, const float* d_y, long y_es, float* d_prob, float* d_loss,
+                                  float* d_dz, pdf_stream_t stream);
+int pdf_moe_combine_train_batched(int n_members, int n, int n_experts, const float* d_z, const float* d_r, const float* d_y, long y_es,
+                                  float* d_out, float* d_loss, float* d_dz, float* d_dr, pdf_stream_t stream);
+size_t pdf_mil_pool_train_batched_workspace_bytes(int n_members, const pdf_mil_weights* w, int n_bags);
+int pdf_mil_pool_train_batched(int n_members, const pdf_mil_weights* w, long w_es, const pdf_mil_train* t, long g_es, int n_bags, int Lmax,
+                               const float* d_h, const float* d_vu, const int32_t* d_len, const float* d_target, float* d_prob,
+                               float* d_loss, float* d_dh, float* d_dvu, void* d_workspace, pdf_stream_t stream);
+int pdf_clip_scale_batched(int n_members, const float* d_grad, long n_params, float max_norm, float* d_scale, pdf_stream_t stream);
+int pdf_adam_step_batched(int n_members, float* d_param, const float* d_grad, float* d_m, float* d_v, long n_params, float lr, float beta1,
+                          float beta2, float eps, float weight_decay, int step, const float* d_grad_scale, const uint8_t* d_active,
+                          pdf_stream_t stream);
+/* the ensemble statistics of every (scenario, subject) pair: d_probs [E, pairs] f32 -> d_stats [pairs, 5] float64 = mean, std
+ * (population), entropy of the mean, mean member entropy, mutual information; pdf_moddrop_mc's formulas with members in place of
+ * samples (ascending e), so equal members give exactly std = mutual information = 0 */
+int pdf_ensemble_stats(int n_members, long long pairs, const float* d_probs, double* d_stats, pdf_stream_t stream);
+
 /* ------------------------------------------------------------------------------------------
  * K4a -- Fusion-ModDrop under every scenario mask in one launch.  Replaces the per-scenario
  * apply_masks_to_matrix + ModalityDropoutModel.predict_proba (data/feature_utils.py:49-61,

@@ -26,9 +26,16 @@ constexpr int TBM = 64, TBN = 64, TBK = 16;
 
 // ------------------------------------------------------------------------------------------------------
 // C[M,N] (+)= act( sum_k A(i,k) B(k,j) + bias[j] ) ; A(i,k) = A[i*a_rs + k*a_cs], B(k,j) = B[k*b_rs + j*b_cs], C row stride c_rs
+// blockIdx.z = e runs member e of an ensemble: every operand moved by e times its member stride (*_es, 0 = shared)
 __global__ void __launch_bounds__(256)
 gemm_strided_kernel(const float* __restrict__ A, long a_rs, long a_cs, const float* __restrict__ B, long b_rs, long b_cs,
-                    float* __restrict__ C, long c_rs, const float* __restrict__ bias, int M, int N, int K, int act, int accumulate) {
+                    float* __restrict__ C, long c_rs, const float* __restrict__ bias, int M, int N, int K, int act, int accumulate,
+                    long a_es, long b_es, long c_es, long bias_es) {
+  const long e = blockIdx.z;
+  A += e * a_es;
+  B += e * b_es;
+  C += e * c_es;
+  if (bias) bias += e * bias_es;
   __shared__ float As[TBK][TBM + 4];
   __shared__ float Bs[TBK][TBN + 4];
   const int tid = threadIdx.x;
@@ -482,8 +489,10 @@ __device__ __forceinline__ float sigm(float x) { return 1.0f / (1.0f + expf(-x))
 //   vu [n_bags*Lmax, NA] = pre-activations of attn_v | attn_u (gated) or attn.0 (plain), bias included
 // forward : s_l = w_w . (tanh(v_l) (.) sigmoid(u_l)) + b_w ; a = softmax_l(s) over the bag's len ; pooled = sum_l a_l h_l ;
 //           p = sigmoid(w_c . pooled + b_c) ; per-bag loss (BCE, optionally pos-weighted or focal), mean over the batch
-// backward: d_h (the pooling path: a_l * d_pooled), d_vu, and the head's small parameter gradients (atomicAdd):
+// backward: d_h (the pooling path: a_l * d_pooled), d_vu, and the head's small parameter gradients, handed to the sink with the loss:
 //           d_w_cls [H], d_b_cls, d_w_w [A], d_b_w.   (models/mil_attention.py:40-51, mil_attention_finetune.py:211-224)
+// The single model accumulates them with atomicAdd (MilAtomicSink).  An ensemble runs member e on blockIdx.y (its weights w_es floats,
+// its bags one batch further) and stores each bag's terms in a row of its own (MilPartialSink), reduced in bag order afterwards.
 struct MilTrainArgs {
   int H, A, gated, Lmax, n_bags;
   int loss_type;          // 0 BCE (x sample weight), 1 focal
@@ -493,11 +502,37 @@ struct MilTrainArgs {
   float *d_w_w, *d_b_w, *d_w_cls, *d_b_cls;
 };
 
+struct MilAtomicSink {
+  float *loss_sum, *d_w_w, *d_b_w, *d_w_cls, *d_b_cls;
+  __device__ void loss(float v) { atomicAdd(loss_sum, v); }
+  __device__ void b_cls(float v) { atomicAdd(d_b_cls, v); }
+  __device__ void w_cls(int i, float v) { atomicAdd(d_w_cls + i, v); }
+  __device__ void b_w(float v) { atomicAdd(d_b_w, v); }
+  __device__ void w_w(int j, float v) { atomicAdd(d_w_w + j, v); }
+};
+// row (member, bag) of partial [E, n_bags, H + A + 3]: d w_cls [H] | d w_w [A] | d b_cls | d b_w | loss / n_bags (zeroed before the launch)
+struct MilPartialSink {
+  float* partial;
+  int H, A;
+  __device__ float* row() const { return partial + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * (H + A + 3); }
+  __device__ void w_cls(int i, float v) { row()[i] = v; }
+  __device__ void w_w(int j, float v) { row()[H + j] = v; }
+  __device__ void b_cls(float v) { row()[H + A] = v; }
+  __device__ void b_w(float v) { row()[H + A + 1] = v; }
+  __device__ void loss(float v) { row()[H + A + 2] = v; }
+};
+
+template <class Sink>
 __global__ void __launch_bounds__(256)
-mil_pool_train_kernel(MilTrainArgs a, const float* __restrict__ h, const float* __restrict__ vu, const int32_t* __restrict__ lens,
-                      const float* __restrict__ target, float* __restrict__ prob, float* __restrict__ loss_sum, float* __restrict__ dh,
-                      float* __restrict__ dvu) {
+mil_pool_train_kernel(MilTrainArgs a, long w_es, const float* __restrict__ h, const float* __restrict__ vu, const int32_t* __restrict__ lens,
+                      const float* __restrict__ target, float* __restrict__ prob, float* __restrict__ dh, float* __restrict__ dvu, Sink sink) {
   extern __shared__ float sm[];
+  const long member = blockIdx.y;
+  const size_t mrows = (size_t)a.n_bags * a.Lmax;
+  a.w_w += member * w_es; a.b_w += member * w_es; a.w_cls += member * w_es; a.b_cls += member * w_es;
+  h += member * mrows * a.H; dh += member * mrows * a.H;
+  vu += member * mrows * (a.gated ? 2 * a.A : a.A); dvu += member * mrows * (a.gated ? 2 * a.A : a.A);
+  lens += member * a.n_bags; target += member * a.n_bags; prob += member * a.n_bags;
   float* s_a = sm;                     // [Lmax] scores -> attention weights
   float* s_da = sm + a.Lmax;           // [Lmax] d loss / d a_l -> d s_l
   float* s_pool = sm + 2 * a.Lmax;     // [H]
@@ -570,9 +605,9 @@ mil_pool_train_kernel(MilTrainArgs a, const float* __restrict__ h, const float* 
   }
   const float inv_b = 1.f / (float)a.n_bags;                   // mean over the batch
   const float dz = dl_dp * p * (1.f - p) * inv_b;
-  if (tid == 0) { prob[bag] = p; atomicAdd(loss_sum, loss * inv_b); atomicAdd(a.d_b_cls, dz); }
+  if (tid == 0) { prob[bag] = p; sink.loss(loss * inv_b); sink.b_cls(dz); }
   // classifier grads, d pooled
-  for (int i = tid; i < H; i += 256) atomicAdd(a.d_w_cls + i, dz * s_pool[i]);
+  for (int i = tid; i < H; i += 256) sink.w_cls(i, dz * s_pool[i]);
   // d a_l = d pooled . h_l ;  d h_l = a_l * d pooled   (d pooled_i = dz * w_cls_i)
   for (int l = warp; l < len; l += 8) {
     float da = 0.f;
@@ -593,7 +628,7 @@ mil_pool_train_kernel(MilTrainArgs a, const float* __restrict__ h, const float* 
   float dbw = 0.f;
   for (int l = tid; l < len; l += 256) dbw += s_da[l];
   dbw = block_sum(dbw, red);
-  if (tid == 0) atomicAdd(a.d_b_w, dbw);
+  if (tid == 0) sink.b_w(dbw);
   // attention layer: d w_w, d v_pre, d u_pre
   for (int j = tid; j < A; j += 256) {
     const float ww = __ldg(a.w_w + j);
@@ -611,7 +646,7 @@ mil_pool_train_kernel(MilTrainArgs a, const float* __restrict__ h, const float* 
         dvb[(size_t)l * NA + j] = ds * ww * (1.f - tv * tv);
       }
     }
-    atomicAdd(a.d_w_w + j, dww);
+    sink.w_w(j, dww);
   }
 }
 
@@ -649,9 +684,14 @@ __global__ void clip_scale_kernel(const float* __restrict__ sumsq, float max_nor
   out2[1] = norm;
 }
 // torch.optim.Adam (no amsgrad), L2-style weight decay: g' = g*scale + wd*p; m, v EMAs; p -= lr * mhat / (sqrt(vhat) + eps)
+// blockIdx.y = e: member e of an ensemble's flat [E, n] buffers, its gradient scaled by scale[e]; skipped when active[e] == 0
 __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m, float* __restrict__ v, size_t n,
-                            float lr, float b1, float b2, float eps, float wd, float bc1, float bc2, const float* __restrict__ scale) {
-  const float sc = scale ? scale[0] : 1.f;
+                            float lr, float b1, float b2, float eps, float wd, float bc1, float bc2, const float* __restrict__ scale,
+                            const uint8_t* __restrict__ active) {
+  const size_t e = blockIdx.y;
+  if (active && !active[e]) return;
+  const float sc = scale ? scale[e] : 1.f;
+  p += e * n; g += e * n; m += e * n; v += e * n;
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
     float gr = g[i] * sc;
     if (wd != 0.f) gr = fmaf(wd, p[i], gr);
@@ -664,49 +704,54 @@ __global__ void adam_kernel(float* __restrict__ p, const float* __restrict__ g, 
 }
 
 // p = sigmoid(z); loss += mean_i BCE(p_i, y_i); dz_i = d loss / d z_i   (nn.BCELoss on a Sigmoid output, logs clamped at -100 as torch)
+// One element: writes p and dz, returns t log p + (1-t) log(1-p) (the caller subtracts it from its loss sum)
+__device__ __forceinline__ float bce_sigmoid_elem(float z, float t, float inv_n, float& p_out, float& dz) {
+  const float p = sigm(z);
+  const float lp = fmaxf(logf(p), -100.f), l1p = fmaxf(logf(1.f - p), -100.f);
+  const float dl_dp = -(t / fmaxf(p, 1e-44f)) * (lp > -100.f ? 1.f : 0.f) + ((1.f - t) / fmaxf(1.f - p, 1e-44f)) * (l1p > -100.f ? 1.f : 0.f);
+  p_out = p;
+  dz = dl_dp * p * (1.f - p) * inv_n;
+  return t * lp + (1.f - t) * l1p;
+}
 __global__ void bce_sigmoid_kernel(const float* __restrict__ z, const float* __restrict__ y, int n, float* __restrict__ p_out,
                                    float* __restrict__ loss_sum, float* __restrict__ dz) {
   __shared__ float red[8];
   float ls = 0.f;
   const float inv_n = 1.f / (float)n;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    const float p = sigm(z[i]), t = y[i];
-    const float lp = fmaxf(logf(p), -100.f), l1p = fmaxf(logf(1.f - p), -100.f);
-    ls -= t * lp + (1.f - t) * l1p;
-    const float dl_dp = -(t / fmaxf(p, 1e-44f)) * (lp > -100.f ? 1.f : 0.f) + ((1.f - t) / fmaxf(1.f - p, 1e-44f)) * (l1p > -100.f ? 1.f : 0.f);
-    p_out[i] = p;
-    dz[i] = dl_dp * p * (1.f - p) * inv_n;
-  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) ls -= bce_sigmoid_elem(z[i], y[i], inv_n, p_out[i], dz[i]);
   ls = block_sum(ls, red);
   if (threadIdx.x == 0) atomicAdd(loss_sum, ls * inv_n);
 }
 
 // MoE combine (models/moe.py:37-47) + BCE, forward and backward: out_i = sum_e sigmoid(z[i,e]) * softmax_e(r[i,:]);
-// loss = mean BCE(out, y); dz [n,E] (expert logits), dr [n,E] (router logits)
+// loss = mean BCE(out, y); dz [n,E] (expert logits), dr [n,E] (router logits).  One row (its E logits z, r): writes out, dz, dr and
+// returns t log o + (1-t) log(1-o)
+__device__ __forceinline__ float moe_combine_elem(const float* __restrict__ z, const float* __restrict__ r, float t, int E, float inv_n,
+                                                  float& out, float* __restrict__ dz, float* __restrict__ dr) {
+  float mx = -INFINITY;
+  for (int e = 0; e < E; ++e) mx = fmaxf(mx, r[e]);
+  float se = 0.f;
+  for (int e = 0; e < E; ++e) se += expf(r[e] - mx);
+  float o = 0.f;
+  for (int e = 0; e < E; ++e) o += sigm(z[e]) * (expf(r[e] - mx) / se);
+  const float lp = fmaxf(logf(o), -100.f), l1p = fmaxf(logf(1.f - o), -100.f);
+  const float dl_do = (-(t / fmaxf(o, 1e-44f)) * (lp > -100.f ? 1.f : 0.f) + ((1.f - t) / fmaxf(1.f - o, 1e-44f)) * (l1p > -100.f ? 1.f : 0.f)) * inv_n;
+  out = o;
+  for (int e = 0; e < E; ++e) {
+    const float pe = sigm(z[e]);
+    const float we = expf(r[e] - mx) / se;
+    dz[e] = dl_do * we * pe * (1.f - pe);
+    dr[e] = dl_do * we * (pe - o);               // softmax backward: w_e * (d_w_e - sum_j w_j d_w_j), d_w_e = dl_do * p_e
+  }
+  return t * lp + (1.f - t) * l1p;
+}
 __global__ void moe_combine_train_kernel(const float* __restrict__ z, const float* __restrict__ r, const float* __restrict__ y, int n, int E,
                                          float* __restrict__ out, float* __restrict__ loss_sum, float* __restrict__ dz, float* __restrict__ dr) {
   __shared__ float red[8];
   float ls = 0.f;
   const float inv_n = 1.f / (float)n;
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-    float mx = -INFINITY;
-    for (int e = 0; e < E; ++e) mx = fmaxf(mx, r[(size_t)i * E + e]);
-    float se = 0.f;
-    for (int e = 0; e < E; ++e) se += expf(r[(size_t)i * E + e] - mx);
-    float o = 0.f;
-    for (int e = 0; e < E; ++e) o += sigm(z[(size_t)i * E + e]) * (expf(r[(size_t)i * E + e] - mx) / se);
-    const float t = y[i];
-    const float lp = fmaxf(logf(o), -100.f), l1p = fmaxf(logf(1.f - o), -100.f);
-    ls -= t * lp + (1.f - t) * l1p;
-    const float dl_do = (-(t / fmaxf(o, 1e-44f)) * (lp > -100.f ? 1.f : 0.f) + ((1.f - t) / fmaxf(1.f - o, 1e-44f)) * (l1p > -100.f ? 1.f : 0.f)) * inv_n;
-    out[i] = o;
-    for (int e = 0; e < E; ++e) {
-      const float pe = sigm(z[(size_t)i * E + e]);
-      const float we = expf(r[(size_t)i * E + e] - mx) / se;
-      dz[(size_t)i * E + e] = dl_do * we * pe * (1.f - pe);
-      dr[(size_t)i * E + e] = dl_do * we * (pe - o);               // softmax backward: w_e * (d_w_e - sum_j w_j d_w_j), d_w_e = dl_do * p_e
-    }
-  }
+  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+    ls -= moe_combine_elem(z + (size_t)i * E, r + (size_t)i * E, y[i], E, inv_n, out[i], dz + (size_t)i * E, dr + (size_t)i * E);
   ls = block_sum(ls, red);
   if (threadIdx.x == 0) atomicAdd(loss_sum, ls * inv_n);
 }
@@ -739,6 +784,65 @@ __global__ void dilate_bf16_kernel(const float* __restrict__ dy, __nv_bfloat16* 
   }
 }
 
+// ------------------------------------------------------------------------------------------------------
+// Deep ensembles: E members of one head trained in lockstep, every launch covering all members (flat [E, P] parameter and gradient
+// buffers, member e's operands e times their member stride further, stride 0 = shared).  Per member the arithmetic is the single
+// kernels' (the GEMM tile, bce_sigmoid_elem, moe_combine_elem, the MIL bag, Adam's element); losses, MIL's parameter gradients and the
+// clip norms are reduced in a fixed order without atomics, so results repeat bit for bit and do not depend on the other members.
+// One block per member: loss[e] = the member's mean BCE (or MoE BCE); y member stride y_es
+__global__ void __launch_bounds__(256)
+bce_sigmoid_batched_kernel(const float* __restrict__ z, const float* __restrict__ y, long y_es, int n, float* __restrict__ p_out,
+                           float* __restrict__ loss, float* __restrict__ dz) {
+  __shared__ float red[8];
+  const long e = blockIdx.x, off = e * n;
+  const float inv_n = 1.f / (float)n;
+  float ls = 0.f;
+  for (int i = threadIdx.x; i < n; i += 256) ls -= bce_sigmoid_elem(z[off + i], y[e * y_es + i], inv_n, p_out[off + i], dz[off + i]);
+  ls = block_sum(ls, red);
+  if (threadIdx.x == 0) loss[e] = ls * inv_n;
+}
+__global__ void __launch_bounds__(256)
+moe_combine_batched_kernel(const float* __restrict__ z, const float* __restrict__ r, const float* __restrict__ y, long y_es, int n, int M,
+                           float* __restrict__ out, float* __restrict__ loss, float* __restrict__ dz, float* __restrict__ dr) {
+  __shared__ float red[8];
+  const size_t e = blockIdx.x, off = e * n * M;
+  z += off; r += off; dz += off; dr += off; out += e * n; y += e * y_es;
+  const float inv_n = 1.f / (float)n;
+  float ls = 0.f;
+  for (int i = threadIdx.x; i < n; i += 256)
+    ls -= moe_combine_elem(z + (size_t)i * M, r + (size_t)i * M, y[i], M, inv_n, out[i], dz + (size_t)i * M, dr + (size_t)i * M);
+  ls = block_sum(ls, red);
+  if (threadIdx.x == 0) loss[e] = ls * inv_n;
+}
+// MIL: column c of member e's MilPartialSink rows summed over the bags in ascending order, added to the member's gradient (loss: written)
+__global__ void __launch_bounds__(256)
+mil_partial_reduce_kernel(const float* __restrict__ partial, int E, int B, int H, int A, float* __restrict__ d_w_cls, float* __restrict__ d_w_w,
+                          float* __restrict__ d_b_cls, float* __restrict__ d_b_w, long g_es, float* __restrict__ loss) {
+  const int W = H + A + 3;
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < (long)E * W; i += (long)gridDim.x * blockDim.x) {
+    const long e = i / W;
+    const int c = (int)(i - e * W);
+    const float* p = partial + (size_t)e * B * W + c;
+    float s = 0.f;
+    for (int b = 0; b < B; ++b) s += p[(size_t)b * W];
+    if (c < H) d_w_cls[e * g_es + c] += s;
+    else if (c < H + A) d_w_w[e * g_es + c - H] += s;
+    else if (c == H + A) d_b_cls[e * g_es] += s;
+    else if (c == H + A + 1) d_b_w[e * g_es] += s;
+    else loss[e] = s;
+  }
+}
+// clip_grad_norm_ per member: one block per row of g [E, P]; scale[e] = min(1, max_norm / (norm + 1e-6))
+__global__ void __launch_bounds__(256)
+clip_scale_batched_kernel(const float* __restrict__ g, long P, float max_norm, float* __restrict__ scale) {
+  __shared__ float red[8];
+  const float* x = g + (long)blockIdx.x * P;
+  float s = 0.f;
+  for (long i = threadIdx.x; i < P; i += 256) s = fmaf(x[i], x[i], s);
+  s = block_sum(s, red);
+  if (threadIdx.x == 0) scale[blockIdx.x] = max_norm > 0.f ? fminf(1.f, max_norm / (sqrtf(s) + 1e-6f)) : 1.f;
+}
+
 static inline int ew_blocks(size_t n) { return (int)std::max<size_t>(1, std::min<size_t>((n + 255) / 256, (size_t)num_sms() * 16)); }
 
 }  // namespace pdf
@@ -749,7 +853,7 @@ extern "C" int pdf_gemm_f32(int M, int N, int K, const float* A, long a_rs, long
                             long c_rs, const float* bias, int act, int accumulate, pdf_stream_t stream) {
   PDF_REQUIRE(M > 0 && N > 0 && K > 0 && A && B && C, "pdf_gemm_f32: bad arguments");
   dim3 grid(ceil_div(M, TBM), ceil_div(N, TBN));
-  gemm_strided_kernel<<<grid, 256, 0, as_stream(stream)>>>(A, a_rs, a_cs, B, b_rs, b_cs, C, c_rs, bias, M, N, K, act, accumulate);
+  gemm_strided_kernel<<<grid, 256, 0, as_stream(stream)>>>(A, a_rs, a_cs, B, b_rs, b_cs, C, c_rs, bias, M, N, K, act, accumulate, 0, 0, 0, 0);
   PDF_CHECK_LAUNCH();
   return PDF_OK;
 }
@@ -868,8 +972,10 @@ extern "C" int pdf_mil_pool_train(const pdf_mil_weights* w, const pdf_mil_train*
   a.d_w_w = t->d_w_w; a.d_b_w = t->d_b_w; a.d_w_cls = t->d_w_cls; a.d_b_cls = t->d_b_cls;
   const size_t smem = ((size_t)2 * Lmax + w->H) * sizeof(float);
   PDF_REQUIRE(smem <= 200 * 1024, "pdf_mil_pool_train: bag too large for shared memory");
-  if (smem > 48 * 1024) PDF_CHECK_CUDA(cudaFuncSetAttribute(mil_pool_train_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  mil_pool_train_kernel<<<n_bags, 256, smem, as_stream(stream)>>>(a, d_h, d_vu, d_len, d_target, d_prob, d_loss, d_dh, d_dvu);
+  if (smem > 48 * 1024)
+    PDF_CHECK_CUDA(cudaFuncSetAttribute(mil_pool_train_kernel<MilAtomicSink>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const MilAtomicSink sink{d_loss, a.d_w_w, a.d_b_w, a.d_w_cls, a.d_b_cls};
+  mil_pool_train_kernel<<<n_bags, 256, smem, as_stream(stream)>>>(a, 0L, d_h, d_vu, d_len, d_target, d_prob, d_dh, d_dvu, sink);
   PDF_CHECK_LAUNCH();
   return PDF_OK;
 }
@@ -915,7 +1021,8 @@ extern "C" int pdf_adam_step(float* d_param, const float* d_grad, float* d_m, fl
                              float eps, float weight_decay, int step, const float* d_grad_scale, pdf_stream_t stream) {
   PDF_REQUIRE(d_param && d_grad && d_m && d_v && n > 0 && step >= 1, "pdf_adam_step: bad arguments");
   const float bc1 = 1.f - powf(beta1, (float)step), bc2 = 1.f - powf(beta2, (float)step);
-  adam_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(d_param, d_grad, d_m, d_v, n, lr, beta1, beta2, eps, weight_decay, bc1, bc2, d_grad_scale);
+  adam_kernel<<<ew_blocks(n), 256, 0, as_stream(stream)>>>(d_param, d_grad, d_m, d_v, n, lr, beta1, beta2, eps, weight_decay, bc1, bc2, d_grad_scale,
+                                                                  nullptr);
   PDF_CHECK_LAUNCH();
   return PDF_OK;
 }
@@ -956,6 +1063,102 @@ extern "C" int pdf_dilate_bf16(int n, int ho, int wo, int k, int hd, int wd, int
               offset >= 0 && d_dy && d_out, "pdf_dilate_bf16: bad arguments");
   dilate_bf16_kernel<<<ew_blocks((size_t)n * hd * wd * k), 256, 0, as_stream(stream)>>>(d_dy, reinterpret_cast<__nv_bfloat16*>(d_out), n, ho, wo, k,
                                                                                         hd, wd, stride, offset);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------ deep ensembles
+static constexpr int kMaxMembers = 1024;
+static bool ens_ok(const void* p) { return p && (reinterpret_cast<uintptr_t>(p) & 3) == 0; }      // non-null, 4-byte aligned
+static bool ens_members_ok(int E) { return E >= 1 && E <= kMaxMembers; }
+
+extern "C" int pdf_gemm_f32_batched(int n_members, int M, int N, int K, const float* A, long a_rs, long a_cs, long a_es, const float* B, long b_rs,
+                                    long b_cs, long b_es, float* C, long c_rs, long c_es, const float* bias, long bias_es, int act, int accumulate,
+                                    pdf_stream_t stream) {
+  PDF_REQUIRE(ens_members_ok(n_members) && M > 0 && N > 0 && K > 0, "pdf_gemm_f32_batched: bad sizes (1 <= members <= %d)", kMaxMembers);
+  PDF_REQUIRE(ens_ok(A) && ens_ok(B) && ens_ok(C) && (!bias || ens_ok(bias)), "pdf_gemm_f32_batched: null or misaligned pointer");
+  PDF_REQUIRE(a_es >= 0 && b_es >= 0 && c_es >= 0 && bias_es >= 0, "pdf_gemm_f32_batched: negative member stride");
+  PDF_REQUIRE(n_members == 1 || c_es > 0, "pdf_gemm_f32_batched: members may not share the output");
+  dim3 grid(ceil_div(M, TBM), ceil_div(N, TBN), n_members);
+  gemm_strided_kernel<<<grid, 256, 0, as_stream(stream)>>>(A, a_rs, a_cs, B, b_rs, b_cs, C, c_rs, bias, M, N, K, act, accumulate, a_es, b_es, c_es,
+                                                           bias_es);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+extern "C" int pdf_bce_sigmoid_train_batched(int n_members, int n, const float* d_z, const float* d_y, long y_es, float* d_prob, float* d_loss,
+                                             float* d_dz, pdf_stream_t stream) {
+  PDF_REQUIRE(ens_members_ok(n_members) && n > 0 && y_es >= 0, "pdf_bce_sigmoid_train_batched: bad sizes");
+  PDF_REQUIRE(ens_ok(d_z) && ens_ok(d_y) && ens_ok(d_prob) && ens_ok(d_loss) && ens_ok(d_dz), "pdf_bce_sigmoid_train_batched: null or misaligned pointer");
+  bce_sigmoid_batched_kernel<<<n_members, 256, 0, as_stream(stream)>>>(d_z, d_y, y_es, n, d_prob, d_loss, d_dz);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+extern "C" int pdf_moe_combine_train_batched(int n_members, int n, int n_experts, const float* d_z, const float* d_r, const float* d_y, long y_es,
+                                             float* d_out, float* d_loss, float* d_dz, float* d_dr, pdf_stream_t stream) {
+  PDF_REQUIRE(ens_members_ok(n_members) && n > 0 && n_experts > 0 && n_experts <= PDF_MAX_MODS && y_es >= 0,
+              "pdf_moe_combine_train_batched: bad sizes");
+  PDF_REQUIRE(ens_ok(d_z) && ens_ok(d_r) && ens_ok(d_y) && ens_ok(d_out) && ens_ok(d_loss) && ens_ok(d_dz) && ens_ok(d_dr),
+              "pdf_moe_combine_train_batched: null or misaligned pointer");
+  moe_combine_batched_kernel<<<n_members, 256, 0, as_stream(stream)>>>(d_z, d_r, d_y, y_es, n, n_experts, d_out, d_loss, d_dz, d_dr);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+extern "C" size_t pdf_mil_pool_train_batched_workspace_bytes(int n_members, const pdf_mil_weights* w, int n_bags) {
+  if (!ens_members_ok(n_members) || !w || n_bags <= 0 || w->H <= 0 || w->A <= 0) return 0;
+  return (size_t)n_members * n_bags * (w->H + w->A + 3) * sizeof(float);
+}
+
+extern "C" int pdf_mil_pool_train_batched(int n_members, const pdf_mil_weights* w, long w_es, const pdf_mil_train* t, long g_es, int n_bags,
+                                          int Lmax, const float* d_h, const float* d_vu, const int32_t* d_len, const float* d_target,
+                                          float* d_prob, float* d_loss, float* d_dh, float* d_dvu, void* d_workspace, pdf_stream_t stream) {
+  PDF_REQUIRE(ens_members_ok(n_members) && w && t && n_bags > 0 && Lmax > 0 && w_es >= 0 && g_es >= 0 && w->H > 0 && w->A > 0,
+              "pdf_mil_pool_train_batched: bad arguments");
+  PDF_REQUIRE(ens_ok(w->w_w) && ens_ok(w->b_w) && ens_ok(w->w_cls) && ens_ok(w->b_cls) && ens_ok(t->d_w_w) && ens_ok(t->d_b_w) &&
+              ens_ok(t->d_w_cls) && ens_ok(t->d_b_cls), "pdf_mil_pool_train_batched: null or misaligned parameter pointer");
+  PDF_REQUIRE(ens_ok(d_h) && ens_ok(d_vu) && ens_ok(d_len) && ens_ok(d_target) && ens_ok(d_prob) && ens_ok(d_loss) && ens_ok(d_dh) &&
+              ens_ok(d_dvu) && ens_ok(d_workspace), "pdf_mil_pool_train_batched: null or misaligned pointer");
+  const size_t smem = ((size_t)2 * Lmax + w->H) * sizeof(float);
+  PDF_REQUIRE(smem <= 200 * 1024, "pdf_mil_pool_train_batched: bag too large for shared memory");
+  MilTrainArgs a;
+  a.H = w->H; a.A = w->A; a.gated = w->gated; a.Lmax = Lmax; a.n_bags = n_bags;
+  a.loss_type = t->loss_type; a.pos_weight = t->pos_weight; a.focal_gamma = t->focal_gamma; a.focal_alpha = t->focal_alpha;
+  a.w_w = w->w_w; a.b_w = w->b_w; a.w_cls = w->w_cls; a.b_cls = w->b_cls;
+  a.d_w_w = t->d_w_w; a.d_b_w = t->d_b_w; a.d_w_cls = t->d_w_cls; a.d_b_cls = t->d_b_cls;
+  cudaStream_t s = as_stream(stream);
+  float* partial = static_cast<float*>(d_workspace);
+  PDF_CHECK_CUDA(cudaMemsetAsync(partial, 0, pdf_mil_pool_train_batched_workspace_bytes(n_members, w, n_bags), s));    // empty bags add 0
+  if (smem > 48 * 1024)
+    PDF_CHECK_CUDA(cudaFuncSetAttribute(mil_pool_train_kernel<MilPartialSink>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const MilPartialSink sink{partial, w->H, w->A};
+  mil_pool_train_kernel<<<dim3(n_bags, n_members), 256, smem, s>>>(a, w_es, d_h, d_vu, d_len, d_target, d_prob, d_dh, d_dvu, sink);
+  PDF_CHECK_LAUNCH();
+  mil_partial_reduce_kernel<<<ew_blocks((size_t)n_members * (w->H + w->A + 3)), 256, 0, s>>>(partial, n_members, n_bags, w->H, w->A, t->d_w_cls,
+                                                                                            t->d_w_w, t->d_b_cls, t->d_b_w, g_es, d_loss);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+extern "C" int pdf_clip_scale_batched(int n_members, const float* d_grad, long n_params, float max_norm, float* d_scale, pdf_stream_t stream) {
+  PDF_REQUIRE(ens_members_ok(n_members) && n_params > 0, "pdf_clip_scale_batched: bad sizes");
+  PDF_REQUIRE(ens_ok(d_grad) && ens_ok(d_scale), "pdf_clip_scale_batched: null or misaligned pointer");
+  clip_scale_batched_kernel<<<n_members, 256, 0, as_stream(stream)>>>(d_grad, n_params, max_norm, d_scale);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+extern "C" int pdf_adam_step_batched(int n_members, float* d_param, const float* d_grad, float* d_m, float* d_v, long n_params, float lr,
+                                     float beta1, float beta2, float eps, float weight_decay, int step, const float* d_grad_scale,
+                                     const uint8_t* d_active, pdf_stream_t stream) {
+  PDF_REQUIRE(ens_members_ok(n_members) && n_params > 0 && step >= 1, "pdf_adam_step_batched: bad arguments");
+  PDF_REQUIRE(ens_ok(d_param) && ens_ok(d_grad) && ens_ok(d_m) && ens_ok(d_v) && (!d_grad_scale || ens_ok(d_grad_scale)),
+              "pdf_adam_step_batched: null or misaligned pointer");
+  const float bc1 = 1.f - powf(beta1, (float)step), bc2 = 1.f - powf(beta2, (float)step);
+  const int per = std::max(1, ew_blocks((size_t)n_params * n_members) / n_members);
+  adam_kernel<<<dim3(per, n_members), 256, 0, as_stream(stream)>>>(d_param, d_grad, d_m, d_v, (size_t)n_params, lr, beta1, beta2, eps, weight_decay,
+                                                                   bc1, bc2, d_grad_scale, d_active);
   PDF_CHECK_LAUNCH();
   return PDF_OK;
 }

@@ -58,20 +58,20 @@ __device__ __forceinline__ double mc_entropy(double q) {
   return -(q > 0.0 ? q * log(q) : 0.0) - (q < 1.0 ? (1.0 - q) * log(1.0 - q) : 0.0);
 }
 
-// o[5] = mean, std (population), entropy of the mean, mean entropy, mutual information of T sample probabilities, float64, ascending
-// t.  The sums run over differences to the first sample, so T equal samples give exactly mean = p, std = 0 and mutual_info = 0.
-__device__ void mc_stats(const float* __restrict__ p, int T, double* __restrict__ o) {
+// o[5] = mean, std (population), entropy of the mean, mean entropy, mutual information of T sample probabilities p[t * stride], float64,
+// ascending t (the samples of MC dropout, stride 1, or the members of a deep ensemble).  The sums run over differences to the first sample, so T equal samples give exactly mean = p, std = 0 and mutual_info = 0.
+__device__ void mc_stats(const float* __restrict__ p, int T, long long stride, double* __restrict__ o) {
   const double p0 = p[0], h0 = mc_entropy(p0);
   double sd = 0.0, sh = 0.0;
   for (int t = 0; t < T; ++t) {
-    const double q = p[t];
+    const double q = p[t * stride];
     sd += q - p0;
     sh += mc_entropy(q) - h0;
   }
   const double mean = p0 + sd / T;
   double v = 0.0;
   for (int t = 0; t < T; ++t) {
-    const double d = (double)p[t] - mean;
+    const double d = (double)p[t * stride] - mean;
     v += d * d;
   }
   const double ent = mc_entropy(mean), eent = h0 + sh / T;
@@ -171,7 +171,14 @@ moddrop_mc_kernel(pdf_mlp net, const float* __restrict__ partials, const uint8_t
 __global__ void __launch_bounds__(256)
 mc_stats_kernel(const float* __restrict__ samples, long long pairs, int T, double* __restrict__ stats) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < pairs; i += (long long)gridDim.x * blockDim.x)
-    mc_stats(samples + i * T, T, stats + i * kMcStats);
+    mc_stats(samples + i * T, T, 1, stats + i * kMcStats);
+}
+
+// deep ensembles: probs [E, pairs] -> stats [pairs, 5], mc_stats over the members in ascending order
+__global__ void __launch_bounds__(256)
+ensemble_stats_kernel(const float* __restrict__ probs, int E, long long pairs, double* __restrict__ stats) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < pairs; i += (long long)gridDim.x * blockDim.x)
+    mc_stats(probs + i, E, pairs, stats + i * kMcStats);
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -311,7 +318,7 @@ mil_mc_stats_kernel(const float* __restrict__ bagprob, const int32_t* __restrict
     const bool on = min(lens[b], Lmax) > 0 && (!live || live[i]);
     double* o = stats + i * kMcStats;
     if (on) {
-      mc_stats(bagprob + (size_t)b * T, T, o);
+      mc_stats(bagprob + (size_t)b * T, T, 1, o);
     } else {
       const double h = mc_entropy((double)missing_prob);
       o[0] = missing_prob;
@@ -466,6 +473,14 @@ extern "C" int pdf_mil_mc(const pdf_mil_weights* w, float p_drop, int n_bags, in
   if (rc) return rc;
   mil_mc_stats_kernel<<<mc_grid((long long)n_scenarios * n_bags), 256, 0, s>>>(bagprob, d_len, Lmax, d_live, n_bags, n_scenarios, T,
                                                                                  w->missing_prob, d_stats, d_samples);
+  PDF_CHECK_LAUNCH();
+  return PDF_OK;
+}
+
+extern "C" int pdf_ensemble_stats(int n_members, long long pairs, const float* d_probs, double* d_stats, pdf_stream_t stream) {
+  PDF_REQUIRE(n_members >= 1 && n_members <= 1024 && pairs > 0, "pdf_ensemble_stats: bad sizes (1 <= members <= 1024)");
+  PDF_REQUIRE(d_probs && mc_aligned(d_probs, 4) && d_stats && mc_aligned(d_stats, 8), "pdf_ensemble_stats: null or misaligned pointer");
+  ensemble_stats_kernel<<<mc_grid(pairs), 256, 0, as_stream(stream)>>>(d_probs, n_members, pairs, d_stats);
   PDF_CHECK_LAUNCH();
   return PDF_OK;
 }

@@ -203,6 +203,17 @@ PROTOTYPES = {
     "pdf_sumsq_f32": (C.c_int, [_P, C.c_size_t, _P, _P]),
     "pdf_clip_scale": (C.c_int, [_P, C.c_float, _P, _P]),
     "pdf_adam_step": (C.c_int, [_P, _P, _P, _P, C.c_size_t, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int, _P, _P]),
+    "pdf_gemm_f32_batched": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_long, C.c_long, C.c_long, _P, C.c_long, C.c_long, C.c_long,
+                                       _P, C.c_long, C.c_long, _P, C.c_long, C.c_int, C.c_int, _P]),
+    "pdf_bce_sigmoid_train_batched": (C.c_int, [C.c_int, C.c_int, _P, _P, C.c_long, _P, _P, _P, _P]),
+    "pdf_moe_combine_train_batched": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, _P, _P, C.c_long, _P, _P, _P, _P, _P]),
+    "pdf_mil_pool_train_batched_workspace_bytes": (C.c_size_t, [C.c_int, C.POINTER(MilWeights), C.c_int]),
+    "pdf_mil_pool_train_batched": (C.c_int, [C.c_int, C.POINTER(MilWeights), C.c_long, C.POINTER(MilTrain), C.c_long, C.c_int, C.c_int, _P, _P,
+                                             _P, _P, _P, _P, _P, _P, _P, _P]),
+    "pdf_clip_scale_batched": (C.c_int, [C.c_int, _P, C.c_long, C.c_float, _P, _P]),
+    "pdf_adam_step_batched": (C.c_int, [C.c_int, _P, _P, _P, _P, C.c_long, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_int, _P,
+                                        _P, _P]),
+    "pdf_ensemble_stats": (C.c_int, [C.c_int, C.c_longlong, _P, _P, _P]),
     "pdf_selftest_umma": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "pdf_selftest_umma_shift": (C.c_int, [C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "pdf_selftest_umma_rate": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),

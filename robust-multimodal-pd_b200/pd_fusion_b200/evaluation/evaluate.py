@@ -10,6 +10,8 @@ per-scenario `predict_proba` calls -- each of which still runs on the device.
 `bootstrap_model` adds bootstrap confidence intervals, and paired intervals of each scenario's difference to a reference scenario, to
 `evaluate_model`'s metrics; the replicates are computed on the device (utils.metrics.bootstrap_metrics).
 `uncertainty_model` estimates every subject's predictive uncertainty under every scenario by Monte-Carlo dropout on the device.
+`ensemble_model` evaluates a deep ensemble (models.ensemble.HeadEnsemble): the mean's metrics, every member's, their spread across seeds
+and the members' disagreement per subject.
 """
 from __future__ import annotations
 
@@ -224,6 +226,44 @@ def uncertainty_model(model, df_test, mask_test, prep_info, config, n_samples: i
     out = {}
     for s, sc in enumerate(scenarios):
         r = dict(res[s])
+        r["risk_coverage"] = _risk_coverage_by_entropy(y_true, r["mean"], r["entropy"])
+        out[sc["name"]] = r
+    return out
+
+
+def ensemble_model(ens, df_test, mask_test, prep_info, config) -> Dict[str, Dict]:
+    """A deep ensemble (models.ensemble.HeadEnsemble) under every scenario of `config`: {scenario: {"metrics": evaluate_model's
+    metrics of the ensemble mean, "members": [each member's metrics], "member_mean" / "member_std": {metric: mean / population std
+    over the members} (the spread across training seeds), "mean", "std", "entropy", "expected_entropy", "mutual_info": [N] float64
+    ensemble statistics per subject, "risk_coverage": {"coverage", "risk", "aurc"} ranked by the entropy of the ensemble mean}}.
+    With config["group_col"] the metrics include _with_groups' subject_* metrics.  The scenario masks are drawn as evaluate_model
+    draws them (same helpers, same numpy RNG order, nothing else drawn), so each member's metrics are evaluate_model's of that member
+    under the same seed."""
+    if not hasattr(ens, "predict_ensemble_sweep"):
+        raise ValueError(f"{type(ens).__name__} is not an ensemble: ensemble_model needs a HeadEnsemble")
+    scenarios = config.get("scenarios", [{"name": "baseline", "drop_modalities": []}])
+    group_col = config.get("group_col")
+    y_true = df_test[TARGET_COL].values
+    if _kind(prep_info) == "mil":
+        _, per = scenario_mask_tensor(df_test, scenarios, mask_test, list(mask_test.keys()))
+        bags = df_test[prep_info[1]].tolist()
+        n = len(bags)
+        mri = np.stack([np.asarray(cur["mri"]) if "mri" in cur else np.ones(n, dtype=int) for cur in per])
+        members, stats = ens.predict_ensemble_sweep(bags, mri)
+    else:
+        X, masks, _, order = _fusion_inputs(df_test, mask_test, prep_info, scenarios)
+        members, stats = ens.predict_ensemble_sweep(X, masks, order)
+    mean = ens._mean(members)
+    out = {}
+    for s, sc in enumerate(scenarios):
+        per_member = [_with_groups(compute_metrics(y_true, members[e, s]), df_test, y_true, members[e, s], group_col)
+                      for e in range(members.shape[0])]
+        keys = list(per_member[0])
+        r = {"metrics": _with_groups(compute_metrics(y_true, mean[s]), df_test, y_true, mean[s], group_col),
+             "members": per_member,
+             "member_mean": {k: float(np.mean([m[k] for m in per_member])) for k in keys},
+             "member_std": {k: float(np.std([m[k] for m in per_member])) for k in keys}}
+        r.update(stats[s])
         r["risk_coverage"] = _risk_coverage_by_entropy(y_true, r["mean"], r["entropy"])
         out[sc["name"]] = r
     return out

@@ -207,13 +207,14 @@ class ModDropSweep:
             raise ValueError("modality_dims do not add up to the network input width")
         self.net = m
 
-    def forward(self, X: torch.Tensor, masks: torch.Tensor) -> torch.Tensor:
-        """X [N,F] f32 cuda; masks [S,N,M] u8 cuda in self.mods order -> prob [S,N] f32."""
+    def forward(self, X: torch.Tensor, masks: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """X [N,F] f32 cuda; masks [S,N,M] u8 cuda in self.mods order -> prob [S,N] f32 (written into `out`, a contiguous
+        [S,N] f32 cuda tensor, when given)."""
         N, S = int(X.shape[0]), int(masks.shape[0])
         X = X.to(dtype=torch.float32).contiguous()
         masks = masks.to(dtype=torch.uint8).contiguous()
         ws = torch.empty(self.lib.pdf_moddrop_workspace_bytes(C.byref(self.net), N), dtype=torch.uint8, device=X.device)
-        prob = torch.empty((S, N), dtype=torch.float32, device=X.device)
+        prob = out if out is not None else torch.empty((S, N), dtype=torch.float32, device=X.device)
         _lib.check(self.lib.pdf_moddrop_sweep(C.byref(self.net), N, S, X.data_ptr(), masks.data_ptr(), ws.data_ptr(),
                                               prob.data_ptr(), _lib.stream_ptr()), "pdf_moddrop_sweep")
         return prob
@@ -283,13 +284,14 @@ class MoeSweep:
         net.w_r0, net.b_r0, net.w_r1, net.b_r1 = (t.data_ptr() for t in r)
         self.net = net
 
-    def forward(self, X: Dict[str, torch.Tensor], masks: torch.Tensor) -> torch.Tensor:
-        """X {mod: [N,d] f32 cuda, UNMASKED}; masks [S,N,M] u8 in self.mods order -> prob [S,N] f32."""
+    def forward(self, X: Dict[str, torch.Tensor], masks: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """X {mod: [N,d] f32 cuda, UNMASKED}; masks [S,N,M] u8 in self.mods order -> prob [S,N] f32 (written into `out`, a
+        contiguous [S,N] f32 cuda tensor, when given)."""
         xs = [X[m].to(dtype=torch.float32).contiguous() for m in self.mods]
         N, S = int(xs[0].shape[0]), int(masks.shape[0])
         masks = masks.to(dtype=torch.uint8).contiguous()
         ptrs = (C.c_void_p * len(xs))(*[x.data_ptr() for x in xs])
-        prob = torch.empty((S, N), dtype=torch.float32, device=xs[0].device)
+        prob = out if out is not None else torch.empty((S, N), dtype=torch.float32, device=xs[0].device)
         _lib.check(self.lib.pdf_moe_sweep(C.byref(self.net), N, S, ptrs, masks.data_ptr(), prob.data_ptr(), _lib.stream_ptr()),
                    "pdf_moe_sweep")
         return prob

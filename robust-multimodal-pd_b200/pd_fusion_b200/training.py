@@ -684,3 +684,210 @@ class ResNetTrainer:
             dop.d_residual = x.grad.data_ptr()                       # accumulate: out = conv + the gradient already there
         self._run_op(dop)
         x.grad = dst
+
+
+# -- deep ensembles: E members of one architecture trained in lockstep (csrc/train.cu) ----------------------------------------
+def flatten_members(member_params: Sequence[Dict[str, torch.Tensor]]) -> Tuple[torch.Tensor, Dict[str, int]]:
+    """Moves the parameters of E members of one architecture into ONE flat f32 buffer [E, P] (row e = member e, each row in
+    `_flat_like`'s layout) and re-points every member's `param.data` at its view.  Returns (buffer, offset of each parameter in a
+    row).  The members' nn.Modules keep working unchanged; every launch of a training step covers all rows."""
+    first = member_params[0]
+    offs, P = {}, 0
+    for k, v in first.items():
+        offs[k] = P
+        P += (v.numel() + 7) // 8 * 8
+    flat = torch.zeros((len(member_params), P), dtype=torch.float32, device=first[next(iter(first))].device)
+    for e, params in enumerate(member_params):
+        if list(params) != list(first) or any(params[k].shape != first[k].shape for k in first):
+            raise ValueError("ensemble members must have the same parameters")
+        for k, v in params.items():
+            view = flat[e, offs[k]:offs[k] + v.numel()].view(v.shape)
+            view.copy_(v.data)
+            v.data = view
+    return flat, offs
+
+
+def _dropout_mask(shape, gens: Sequence[torch.Generator], keep: float, dev) -> torch.Tensor:
+    """[E, *shape] inverted-dropout masks, member e's drawn from its own CUDA generator exactly as the single trainers draw theirs"""
+    return torch.stack([torch.rand(shape, device=dev, generator=g) < keep for g in gens]).to(torch.float32) / keep
+
+
+class BatchedGemm:
+    """pdf_gemm_f32_batched over the members of a flat [E, P] parameter / gradient buffer pair"""
+
+    def __init__(self, flat_param: torch.Tensor, flat_grad: torch.Tensor, offs: Dict[str, int]):
+        self.lib = _lib.load()
+        self.E, self.P = int(flat_param.shape[0]), int(flat_param.shape[1])
+        self.flat_param, self.flat_grad, self.offs = flat_param, flat_grad, offs
+        self.dev = flat_param.device
+        self._ones_buf = None
+
+    def param(self, name: str) -> int:
+        return self.flat_param.data_ptr() + 4 * self.offs[name]
+
+    def grad(self, name: str) -> int:
+        return self.flat_grad.data_ptr() + 4 * self.offs[name]
+
+    def gemm(self, M, N, K, A, a_rs, a_cs, a_es, B, b_rs, b_cs, b_es, Cm, c_rs, c_es, bias=None, bias_es=0, act=0, acc=0):
+        ptr = lambda t: t.data_ptr() if isinstance(t, torch.Tensor) else t
+        _lib.check(self.lib.pdf_gemm_f32_batched(self.E, M, N, K, ptr(A), a_rs, a_cs, a_es, ptr(B), b_rs, b_cs, b_es, ptr(Cm), c_rs, c_es,
+                                                 bias, bias_es, act, acc, _lib.stream_ptr()), "pdf_gemm_f32_batched")
+
+    def colsum(self, rows: int, n: int, d, d_es: int, out_name: str, d_rs: Optional[int] = None):
+        """gradient[out_name] (+)= the column sums of every member's d [rows, n] (row stride d_rs): a GEMM with a shared row of ones,
+        whose k-ascending accumulation adds the rows in pdf_colsum_f32's order"""
+        self.gemm(1, n, rows, self.ones(rows), 0, 1, 0, d, n if d_rs is None else d_rs, 1, d_es, self.grad(out_name), n, self.P, acc=1)
+
+    def ones(self, n: int) -> torch.Tensor:
+        if self._ones_buf is None or self._ones_buf.numel() < n:
+            self._ones_buf = torch.ones(n, dtype=torch.float32, device=self.dev)
+        return self._ones_buf
+
+
+class BatchedMlpTrainer:
+    """MlpTrainer for the same `nn.Sequential` of E members at once: activations [E, rows, width], member e's weights in row e of
+    the shared flat buffers.  The input of `forward` is [E, rows, F] or one [rows, F] matrix every member reads (MoE's full batch)."""
+
+    def __init__(self, seq: nn.Sequential, prefix: str, bg: BatchedGemm):
+        self.bg, self.lib = bg, bg.lib
+        self.layers: List[Tuple[str, int, int, bool, float]] = []      # (name, n_out, n_in, relu after, dropout p after)
+        mods = list(seq)
+        for i, m in enumerate(mods):
+            if isinstance(m, nn.Linear):
+                relu = i + 1 < len(mods) and isinstance(mods[i + 1], nn.ReLU)
+                drop = float(mods[i + 2].p) if relu and i + 2 < len(mods) and isinstance(mods[i + 2], nn.Dropout) else 0.0
+                self.layers.append((f"{prefix}{i}", int(m.weight.shape[0]), int(m.weight.shape[1]), relu, drop))
+
+    def forward(self, X: torch.Tensor, gens: Optional[Sequence[torch.Generator]] = None) -> torch.Tensor:
+        """-> logits [E, rows, n_out]; gens: the members' CUDA generators for the dropout masks (None = no dropout, eval)"""
+        bg, E, s = self.bg, self.bg.E, _lib.stream_ptr()
+        a = X.contiguous()
+        rows = int(a.shape[-2])
+        a_es = 0 if a.dim() == 2 else rows * int(a.shape[-1])
+        self.saved = []
+        for name, n_out, n_in, relu, drop in self.layers:
+            out = torch.empty((E, rows, n_out), dtype=torch.float32, device=bg.dev)
+            bg.gemm(rows, n_out, n_in, a, n_in, 1, a_es, bg.param(name + ".weight"), 1, n_in, bg.P, out, n_out, rows * n_out,
+                    bg.param(name + ".bias"), bg.P, 1 if relu else 0)
+            mask = None
+            if gens is not None and relu and drop > 0:
+                mask = _dropout_mask((rows, n_out), gens, 1.0 - drop, bg.dev)
+                _lib.check(self.lib.pdf_mul_f32(out.data_ptr(), mask.data_ptr(), out.numel(), s), "pdf_mul_f32")
+            self.saved.append((a, a_es, out, mask))
+            a, a_es = out, rows * n_out
+        return a
+
+    def backward(self, dlogits: torch.Tensor) -> None:
+        bg, E, s = self.bg, self.bg.E, _lib.stream_ptr()
+        d = dlogits.contiguous()
+        for (name, n_out, n_in, relu, drop), (a_in, a_es, out, mask) in zip(reversed(self.layers), reversed(self.saved)):
+            rows = int(out.shape[1])
+            if relu:
+                _lib.check(self.lib.pdf_relu_mask_backward(d.data_ptr(), out.data_ptr(), _p(mask), d.numel(), s), "pdf_relu_mask_backward")
+            bg.gemm(n_out, n_in, rows, d, 1, n_out, rows * n_out, a_in, n_in, 1, a_es, bg.grad(name + ".weight"), n_in, bg.P, acc=1)
+            bg.colsum(rows, n_out, d, rows * n_out, name + ".bias")
+            if name != self.layers[0][0]:
+                dn = torch.empty((E, rows, n_in), dtype=torch.float32, device=bg.dev)
+                bg.gemm(rows, n_in, n_out, d, n_out, 1, rows * n_out, bg.param(name + ".weight"), n_in, 1, bg.P, dn, n_in, rows * n_in)
+                d = dn
+        self.saved = []
+
+
+class BatchedMilHeadTrainer:
+    """MilHeadTrainer.forward_backward for E members of one MILAttentionNet architecture at once (BCE loss): bags [E, B, Lmax, D]
+    (each member its own minibatch), member e's parameters and gradients in row e of the flat buffers."""
+
+    def __init__(self, net: nn.Module, gated: bool, bg: BatchedGemm):
+        self.bg, self.lib, self.gated = bg, bg.lib, bool(gated)
+        self.H, self.D = (int(v) for v in net.instance[0].weight.shape)
+        self.A = int((net.attn_v[0] if self.gated else net.attn[0]).weight.shape[0])
+        self.NA = 2 * self.A if self.gated else self.A
+        self.dropout = float(net.instance[2].p) if len(net.instance) > 2 else 0.0
+
+    def forward_backward(self, X: torch.Tensor, lens: torch.Tensor, y: torch.Tensor, pos_weight: Optional[float],
+                         gens: Sequence[torch.Generator]) -> Tuple[torch.Tensor, torch.Tensor]:
+        """X [E, B, Lmax, D], lens [E, B] i32, y [E, B] f32 -> (loss [E], prob [E, B]); gradients ACCUMULATED into the flat buffer"""
+        bg, E, s = self.bg, self.bg.E, _lib.stream_ptr()
+        B, Lmax, D = (int(v) for v in X.shape[1:])
+        rows, H, A, NA, P = B * Lmax, self.H, self.A, self.NA, bg.P
+        X = X.contiguous()
+        h = torch.empty((E, rows, H), dtype=torch.float32, device=bg.dev)
+        bg.gemm(rows, H, D, X, D, 1, rows * D, bg.param("instance.0.weight"), 1, D, P, h, H, rows * H, bg.param("instance.0.bias"), P, act=1)
+        mask = None
+        if self.dropout > 0:
+            mask = _dropout_mask((rows, H), gens, 1.0 - self.dropout, bg.dev)
+            _lib.check(self.lib.pdf_mul_f32(h.data_ptr(), mask.data_ptr(), h.numel(), s), "pdf_mul_f32")
+        vu = torch.empty((E, rows, NA), dtype=torch.float32, device=bg.dev)
+        names = [("attn_v.0", 0), ("attn_u.0", A)] if self.gated else [("attn.0", 0)]
+        for name, off in names:
+            bg.gemm(rows, A, H, h, H, 1, rows * H, bg.param(name + ".weight"), 1, H, P, vu.data_ptr() + 4 * off, NA, rows * NA,
+                    bg.param(name + ".bias"), P)
+        ww, bw = ("attn_w.weight", "attn_w.bias") if self.gated else ("attn.2.weight", "attn.2.bias")
+        w = _lib.MilWeights()
+        w.D, w.H, w.A, w.gated = D, H, A, 1 if self.gated else 0
+        w.w_w, w.b_w, w.w_cls, w.b_cls = bg.param(ww), bg.param(bw), bg.param("classifier.0.weight"), bg.param("classifier.0.bias")
+        t = _lib.MilTrain()
+        t.loss_type, t.pos_weight, t.focal_gamma, t.focal_alpha = 0, 1.0 if pos_weight is None else float(pos_weight), 2.0, -1.0
+        t.d_w_w, t.d_b_w = bg.grad(ww), bg.grad(bw)
+        t.d_w_cls, t.d_b_cls = bg.grad("classifier.0.weight"), bg.grad("classifier.0.bias")
+        prob = torch.empty((E, B), dtype=torch.float32, device=bg.dev)
+        loss = torch.empty(E, dtype=torch.float32, device=bg.dev)
+        dh = torch.empty((E, rows, H), dtype=torch.float32, device=bg.dev)
+        dvu = torch.empty((E, rows, NA), dtype=torch.float32, device=bg.dev)
+        ws = torch.empty(int(self.lib.pdf_mil_pool_train_batched_workspace_bytes(E, C.byref(w), B)), dtype=torch.uint8, device=bg.dev)
+        lens = lens.to(device=bg.dev, dtype=torch.int32).contiguous()
+        y = y.to(device=bg.dev, dtype=torch.float32).contiguous()
+        _lib.check(self.lib.pdf_mil_pool_train_batched(E, C.byref(w), P, C.byref(t), P, B, Lmax, h.data_ptr(), vu.data_ptr(), lens.data_ptr(),
+                                                       y.data_ptr(), prob.data_ptr(), loss.data_ptr(), dh.data_ptr(), dvu.data_ptr(),
+                                                       ws.data_ptr(), s), "pdf_mil_pool_train_batched")
+        # attention layers: dW = dvu^T h, db = colsum(dvu), dh += dvu W
+        for name, off in names:
+            dv = dvu.data_ptr() + 4 * off
+            bg.gemm(A, H, rows, dv, 1, NA, rows * NA, h, H, 1, rows * H, bg.grad(name + ".weight"), H, P, acc=1)
+            bg.colsum(rows, A, dv, rows * NA, name + ".bias", d_rs=NA)
+            bg.gemm(rows, H, A, dv, NA, 1, rows * NA, bg.param(name + ".weight"), H, 1, P, dh, H, rows * H, acc=1)
+        # instance layer: ReLU (+ dropout) backward, dW_i = dh^T X, db_i
+        _lib.check(self.lib.pdf_relu_mask_backward(dh.data_ptr(), h.data_ptr(), _p(mask), dh.numel(), s), "pdf_relu_mask_backward")
+        bg.gemm(H, D, rows, dh, 1, H, rows * H, X, D, 1, rows * D, bg.grad("instance.0.weight"), D, P, acc=1)
+        bg.colsum(rows, H, dh, rows * H, "instance.0.bias")
+        return loss, prob
+
+
+class BatchedAdam:
+    """NativeAdam (+ clip_grad_norm_) per member over flat [E, P] parameters: one pdf_clip_scale_batched and one pdf_adam_step_batched
+    per step.  Each member keeps its own step count; a member that is not active (stopped early) keeps its weights and moments."""
+
+    def __init__(self, flat_param: torch.Tensor, lr: float, weight_decay: float = 0.0, betas=(0.9, 0.999), eps: float = 1e-8):
+        self.lib = _lib.load()
+        self.p = flat_param
+        self.E, self.P = int(flat_param.shape[0]), int(flat_param.shape[1])
+        self.lr, self.wd, self.b1, self.b2, self.eps = float(lr), float(weight_decay), float(betas[0]), float(betas[1]), float(eps)
+        self.m, self.v = torch.zeros_like(flat_param), torch.zeros_like(flat_param)
+        self.steps = [0] * self.E
+        self._scale = torch.ones(self.E, dtype=torch.float32, device=flat_param.device)
+        self._flags: Dict[Tuple[bool, ...], torch.Tensor] = {}
+
+    def clip(self, flat_grad: torch.Tensor, max_norm: float) -> torch.Tensor:
+        _lib.check(self.lib.pdf_clip_scale_batched(self.E, flat_grad.data_ptr(), self.P, float(max_norm), self._scale.data_ptr(),
+                                                   _lib.stream_ptr()), "pdf_clip_scale_batched")
+        return self._scale
+
+    def _active_ptr(self, flags: Tuple[bool, ...]):
+        if all(flags):
+            return None
+        if flags not in self._flags:
+            self._flags[flags] = torch.tensor(flags, dtype=torch.uint8, device=self.p.device)
+        return self._flags[flags].data_ptr()
+
+    def step(self, flat_grad: torch.Tensor, scale: Optional[torch.Tensor] = None, active: Optional[Sequence[bool]] = None):
+        """one Adam step of every active member; members whose step counts differ (after an earlier early stop) step in one launch
+        per distinct count"""
+        act = [True] * self.E if active is None else [bool(a) for a in active]
+        for cnt in sorted({self.steps[e] for e in range(self.E) if act[e]}):
+            flags = tuple(act[e] and self.steps[e] == cnt for e in range(self.E))
+            _lib.check(self.lib.pdf_adam_step_batched(self.E, self.p.data_ptr(), flat_grad.data_ptr(), self.m.data_ptr(), self.v.data_ptr(),
+                                                      self.P, self.lr, self.b1, self.b2, self.eps, self.wd, cnt + 1, _p(scale),
+                                                      self._active_ptr(flags), _lib.stream_ptr()), "pdf_adam_step_batched")
+            for e in range(self.E):
+                if flags[e]:
+                    self.steps[e] += 1
